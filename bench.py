@@ -7,6 +7,7 @@ solves (41 levels / 40 lines), drawn as SURVEY.md 8(d) config 2, each carried to
 own stop rule (pyradex: sum|dx| < 1e-16 after > 10 iterations, cap 200) unless --stop radex.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--log2n 20] [--stop pyradex|radex]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value`: inputs resident in HBM, kernel timed with CUDA events on
 its launch stream, L2 flushed between timed steps.  `e2e`: same workload through the C ABI's
@@ -47,6 +48,8 @@ F_ITER = 72368.0
 F_PRO = 1.3e4
 F_EPI = 4.0e3
 MOLFILE = os.path.join(ROOT, "radex_emcee_b200", "data", "co.dat")
+DUMP_BYTES = 48 << 20           # --dump-outputs: larger batches are sampled down to this many bytes of models
+DUMP_SEED = 20240601
 
 
 def draw(n, seed):
@@ -280,6 +283,33 @@ def sampler_small_records(ctx, dev, stop_rule):
     return out
 
 
+def dump_outputs(out_dir, arrays):
+    """Write the per-model device arrays `arrays` (name -> tensor with one row per model) as out_dir/<name>.npy in
+    float64.  Where all of them together exceed DUMP_BYTES, the same seeded sample of models is kept in every array.
+    Every file holds finite numbers only: the solver returns an infinite or NaN brightness where the reference does
+    (status bit RB_ST_NONFINITE), so each floating-point output is written with 0 in place of a non-finite entry, and
+    <name>_nonfinite.npy (float32, same shape) says what stood there: 0 finite, 1 NaN, 2 +inf, 3 -inf."""
+    import torch
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum((12 if a.is_floating_point() else 8) * (a[0].numel() if a.dim() > 1 else 1) for a in arrays.values())
+    keep = DUMP_BYTES // row_bytes
+    idx = None
+    if n > keep:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, keep, replace=False))
+        idx = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = (a if idx is None else a[idx]).to(torch.float64)
+        if arrays[name].is_floating_point():
+            code = torch.zeros(a.shape, dtype=torch.float32, device=a.device)
+            code[torch.isnan(a)] = 1
+            code[torch.isposinf(a)] = 2
+            code[torch.isneginf(a)] = 3
+            np.save(os.path.join(out_dir, name + "_nonfinite.npy"), code.cpu().numpy())
+            a = torch.where(code == 0, a, torch.zeros_like(a))
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def emit(line):
     """The ONE JSON line of the contract goes to the process's real stdout; everything else that libraries write to fd 1
     while the bench runs (NCCL prints its version there) is sent to stderr by main()."""
@@ -313,7 +343,16 @@ def main():
     ap.add_argument("--keep", default="", help="debug: small | big | k57 | k8 -- keep only the models whose lead block (from a first pass) has <= 16 | > 16 | 20..28 | > 28 levels, tiled to n")
     ap.add_argument("--park-max", type=int, default=0, help="rb_opts.park_max (profiling aid: 7 gives the 20/24/28-level engines their own launches on small batches)")
     ap.add_argument("--kernel", type=int, default=0, help="rb_opts.kernel: 0 default, 1 v1 LU, 2 v2 without caching, 3 single launch, 4 without the half-warp engine")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed launch returned (xpop, tex, tau, surf, niter, "
+                         "status) as DIR/<name>.npy in float64, rank 0 only, non-finite entries as 0 with their kind "
+                         "in DIR/<name>_nonfinite.npy; batches of more than %d MiB are sampled to that size, the same "
+                         "models on every run (fixed seed)" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times a sample whose size depends on its speed")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
@@ -427,6 +466,9 @@ def main():
     npar = min(args.parity_n, n)      # the arrays the parity record checks are the timed launch's own
     par_arrays = {"xpop": d_x[:npar].cpu().numpy(), "tex": d_tex[:npar].cpu().numpy(), "tau": d_tau[:npar].cpu().numpy(),
                   "surf": d_surf[:npar].cpu().numpy(), "niter": niter_host[:npar].copy(), "status": status_host[:npar].copy()}
+    if args.dump_outputs and rank == 0:         # before the extra records: their launches write into d_tex and d_tau
+        dump_outputs(args.dump_outputs, {"xpop": d_x, "tex": d_tex, "tau": d_tau, "surf": d_surf, "niter": d_it,
+                                         "status": d_st})
 
     # ---- e2e: host buffers through the C ABI (pinned), H2D + D2H inside the timed region --------------
     def pinned(shape, dtype):

@@ -218,6 +218,49 @@ int rb_stretch_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split,
                        int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
                        int64_t *counters, int32_t thin, double *chain, double *lnp_chain);
 
+/* ---- posterior statistics of the device-resident chain: replaces np.percentile over the flattened chain
+ * (er1:511-531) and emcee's get_autocorr_time / integrated_time, without moving the chain.  DEVICE pointers,
+ * asynchronous on the ctx stream.  Argument errors give RB_ERR_ARG, a machine without a CUDA device RB_ERR_CUDA.
+ *   view   : the chain as this rank stores it: chunk[c] is [steps[c]][nlocal][ndim] (one chunk per run_mcmc call),
+ *            read in place.  Selected steps over the concatenated step index are emcee's
+ *            discard + thin - 1, discard + 2 thin - 1, ... (get_chain(discard=, thin=)).  Local walker w belongs to
+ *            source (gid_base + w) / walkers_per_source, as in rb_split.
+ *   hist   : one digit pass of a radix select over keys k(x) = bits(x) ^ (x < 0 ? ~0 : 1 << 63) (order-preserving; NaN is
+ *            counted in nan_counts on pass 0 and in no histogram).  Column c is x[col_i[c]], or x[col_i[c]] + x[col_j[c]]
+ *            (one IEEE add) when col_j[c] >= 0; col_i, col_j are HOST arrays.  Pass p counts digit p (bits 63-8p..56-8p)
+ *            of the values whose higher digits equal prefix[src][c][t] (right-aligned; pass 0: nprefix = 1, prefix
+ *            ignored; UINT64_MAX = unused slot):  counts[src][c][t][digit] += ..., nan_counts[src][c] += ... (pass 0,
+ *            may be NULL).  ncol * nprefix <= RB_CHAIN_MAX_HIST.
+ *   moments: mean[nlocal][ndim] and c0 = sum_t (x_t - mean)^2 over the selected steps.
+ *   acf    : rho_sum[nsrc][k1 - k0][ndim] = sum over the walkers of each source of c_k / c_0, c_k = sum_t (x_t - mean)
+ *            (x_{t+k} - mean), for lags k0 <= k < k1 <= selected steps; sources not on this rank get 0.  Fixed summation
+ *            order: the same call on the same rank layout gives the same bits.  A walker with c_0 = 0 gives NaN.
+ * The caller sums hist / acf outputs over ranks and finishes on the host; for a percentile q (numpy's default
+ * 'linear' method) of n values:  v = (n - 1) (q / 100); i = floor(v), j = i + 1, or i = j = n - 1 when v >= n - 1
+ * (then gamma = v + 1, else gamma = v - i); d = x_(j) - x_(i); result = gamma >= 0.5 ? x_(j) - d (1 - gamma)
+ * : x_(i) + d gamma; NaN if the column holds a NaN.                                                               */
+#define RB_MAX_CHUNKS 64
+#define RB_CHAIN_MAX_DIM 16
+#define RB_CHAIN_MAX_COLS 32
+#define RB_CHAIN_MAX_HIST 128
+typedef struct rb_chain_view {
+  const double *chunk[RB_MAX_CHUNKS];
+  int64_t steps[RB_MAX_CHUNKS];
+  int32_t nchunks;
+  int32_t ndim;
+  int64_t nlocal;
+  int64_t gid_base;
+  int64_t walkers_per_source;
+  int64_t discard;
+  int64_t thin;
+} rb_chain_view;
+int rb_chain_hist_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, int32_t ncol, const int32_t *col_i,
+                      const int32_t *col_j, int32_t pass, int32_t nprefix, const uint64_t *prefix, uint64_t *counts,
+                      uint64_t *nan_counts);
+int rb_chain_moments_dev(rb_ctx *ctx, const rb_chain_view *view, double *mean, double *c0);
+int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *mean, const double *c0,
+                     int64_t k0, int64_t k1, double *rho_sum);
+
 /* counters of the last solve/lnprob call on this ctx (device-measured, read back on request):
  * total matrix iterations summed over models, and kernels launched since ctx creation.        */
 int rb_ctx_counters(rb_ctx *ctx, int64_t *total_iters_last, int64_t *launches_total);

@@ -11,6 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libradex_b200.so")
 
 RB_MAX_OBS = 16
+RB_MAX_CHUNKS, RB_CHAIN_MAX_DIM, RB_CHAIN_MAX_COLS, RB_CHAIN_MAX_HIST = 64, 16, 32, 128
 STOP_PYRADEX, STOP_RADEX = 0, 1
 GEOM = {"sphere": 1, "lvg": 2, "slab": 3}
 ST_T_RANGE, ST_N_RANGE, ST_MAXITER, ST_NONFINITE = 1, 2, 4, 8
@@ -39,6 +40,12 @@ class rb_source(C.Structure):
 class rb_split(C.Structure):
     _fields_ = [("nwalkers", C.c_int64), ("walkers_per_source", C.c_int64), ("block", C.c_int64),
                 ("randomize", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64)]
+
+
+class rb_chain_view(C.Structure):
+    _fields_ = [("chunk", C.c_void_p * RB_MAX_CHUNKS), ("steps", C.c_int64 * RB_MAX_CHUNKS), ("nchunks", C.c_int32),
+                ("ndim", C.c_int32), ("nlocal", C.c_int64), ("gid_base", C.c_int64), ("walkers_per_source", C.c_int64),
+                ("discard", C.c_int64), ("thin", C.c_int64)]
 
 
 _dp = C.POINTER(C.c_double)
@@ -90,6 +97,10 @@ SIGNATURES = {
     "rb_ctx_counters": (C.c_int, [_vp, _lp, _lp]),
     "rb_ctx_cache_stats": (C.c_int, [_vp, _lp]),
     "rb_fp64_peak": (C.c_int, [_vp, _dp]),
+    "rb_chain_hist_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, C.c_int32, _ip, _ip, C.c_int32, C.c_int32,
+                                    _vp, _vp, _vp]),
+    "rb_chain_moments_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), _vp, _vp]),
+    "rb_chain_acf_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, _vp, _vp, C.c_int64, C.c_int64, _vp]),
 }
 
 _lib = None

@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libradex_b200.so")
 SOURCES = ["radex_b200.cu", "moldata.cpp"]
 HEADERS = [os.path.join(CSRC, "internal.h"), os.path.join(CSRC, "lvg_v2.cuh"), os.path.join(CSRC, "lvg_small.cuh"),
-           os.path.join(ROOT, "include", "radex_b200.h")]
+           os.path.join(CSRC, "stretch.cuh"), os.path.join(CSRC, "chain_stats.cuh"), os.path.join(ROOT, "include", "radex_b200.h")]
 
 
 def nvcc_path() -> str:

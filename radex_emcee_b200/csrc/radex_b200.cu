@@ -104,6 +104,8 @@ struct rb_ctx {
   cudaEvent_t ev_samp = nullptr;
   cudaGraphExec_t samp_graph = nullptr;   // one stretch-move step, captured for the arguments in samp_key
   std::vector<unsigned char> samp_key;
+  void *cs_buf = nullptr;                 // rb_chain_acf_dev: per-block partial sums (grow-only)
+  size_t cs_bytes = 0;
   long long launches = 0;
   long long last_total_iters = 0;
 };
@@ -1360,6 +1362,7 @@ __global__ void k_stretch_accept(long long ns, int ndim, double *S, double *lnp_
 
 
 #include "stretch.cuh"
+#include "chain_stats.cuh"
 
 // ------------------------------------------------------------------------------------------------
 // FP64 FMA peak probe: the roofline denominator for the solve kernels is the vector FP64 pipe,
@@ -1645,6 +1648,7 @@ void rb_ctx_destroy(rb_ctx *ctx) {
   if (ctx->ln_buf) cudaFree(ctx->ln_buf);
   if (ctx->src_one) cudaFree(ctx->src_one);
   if (ctx->samp_buf) cudaFree(ctx->samp_buf);
+  if (ctx->cs_buf) cudaFree(ctx->cs_buf);
   if (ctx->samp_graph) cudaGraphExecDestroy(ctx->samp_graph);
   if (ctx->ev_samp) cudaEventDestroy(ctx->ev_samp);
   for (cudaEvent_t ev : ctx->chunk_done) cudaEventDestroy(ev);
@@ -2591,6 +2595,182 @@ int rb_fp64_peak(rb_ctx *ctx, double *tflops) {
   cudaFree(d);
   const double flops = 2.0 * 8 * 16 * (double)iters * (double)blocks * tpb;
   *tflops = flops / (best * 1e-3) * 1e-12;
+  return RB_OK;
+}
+
+// ---- chain statistics (chain_stats.cuh) --------------------------------------------------------------------------
+// Argument checks first (RB_ERR_ARG), then the device (RB_ERR_CUDA), then the context.
+static int chain_view(const char *who, const rb_chain_view *in, int32_t nsrc, cs::View *v) {
+  std::string e;
+  if (!in) e = "null view";
+  else if (in->nchunks < 0 || in->nchunks > RB_MAX_CHUNKS) e = "nchunks must be in 0..RB_MAX_CHUNKS";
+  else if (in->ndim < 1 || in->ndim > RB_CHAIN_MAX_DIM) e = "ndim must be in 1..RB_CHAIN_MAX_DIM";
+  else if (in->thin < 1) e = "thin must be positive";
+  else if (in->discard < 0 || in->nlocal < 0 || in->gid_base < 0 || in->walkers_per_source < 1) e = "bad walker layout";
+  if (e.empty()) {
+    long long t = 0;
+    for (int c = 0; c < in->nchunks && e.empty(); ++c) {
+      if (in->steps[c] < 0 || (in->steps[c] > 0 && in->nlocal > 0 && !in->chunk[c])) e = "bad chunk";
+      t += in->steps[c];
+    }
+    v->nchunks = in->nchunks;
+    v->ndim = in->ndim;
+    v->nlocal = in->nlocal;
+    v->gid_base = in->gid_base;
+    v->W = in->walkers_per_source;
+    v->first = in->discard + in->thin - 1;
+    v->thin = in->thin;
+    v->nsel = t > v->first ? (t - v->first + v->thin - 1) / v->thin : 0;
+    v->src0 = in->gid_base / in->walkers_per_source;
+    long long acc = 0;
+    for (int c = 0; c < RB_MAX_CHUNKS; ++c) {
+      v->chunk[c] = c < in->nchunks ? in->chunk[c] : nullptr;
+      v->start[c] = acc;
+      if (c < in->nchunks) acc += in->steps[c];
+    }
+    v->start[RB_MAX_CHUNKS] = acc;
+    if (e.empty() && in->nlocal > 0 && (in->gid_base + in->nlocal - 1) / in->walkers_per_source >= nsrc)
+      e = "nsrc does not cover the rank's walkers";
+  }
+  if (!e.empty()) {
+    rb_set_error(std::string(who) + ": " + e);
+    return RB_ERR_ARG;
+  }
+  return RB_OK;
+}
+
+static int chain_device(const char *who, rb_ctx *ctx) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+    cudaGetLastError();
+    rb_set_error(std::string(who) + ": no CUDA device");
+    return RB_ERR_CUDA;
+  }
+  if (!ctx) {
+    rb_set_error(std::string(who) + ": null context");
+    return RB_ERR_ARG;
+  }
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  return RB_OK;
+}
+
+static long long local_sources(const cs::View &v) {
+  return v.nlocal ? (v.gid_base + v.nlocal - 1) / v.W - v.src0 + 1 : 0;
+}
+
+int rb_chain_hist_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, int32_t ncol, const int32_t *col_i,
+                      const int32_t *col_j, int32_t pass, int32_t nprefix, const uint64_t *prefix, uint64_t *counts,
+                      uint64_t *nan_counts) {
+  static const char *who = "rb_chain_hist_dev";
+  cs::View v;
+  int rc = chain_view(who, view, nsrc, &v);
+  if (rc != RB_OK) return rc;
+  cs::Cols cols;
+  std::string e;
+  if (ncol < 1 || ncol > RB_CHAIN_MAX_COLS || !col_i || !col_j) e = "ncol must be in 1..RB_CHAIN_MAX_COLS";
+  else if (pass < 0 || pass > 7) e = "pass must be in 0..7";
+  else if (nprefix < 1 || ncol * nprefix > RB_CHAIN_MAX_HIST || (pass == 0 && nprefix != 1)) e = "bad nprefix";
+  else if (!prefix || !counts) e = "null output";
+  for (int c = 0; e.empty() && c < ncol; ++c) {
+    if (col_i[c] < 0 || col_i[c] >= v.ndim || col_j[c] < -1 || col_j[c] >= v.ndim) e = "column outside [0, ndim)";
+    cols.i[c] = col_i[c];
+    cols.j[c] = col_j[c];
+  }
+  cols.n = ncol;
+  if (!e.empty()) {
+    rb_set_error(std::string(who) + ": " + e);
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long nls = local_sources(v);
+  if (nls == 0 || v.nsel == 0) return RB_OK;
+  const int nh = ncol * nprefix;
+  const size_t smem = (size_t)nh * 8 + (size_t)cs::HIST_THREADS * (v.ndim | 1) * 8 + ((size_t)nh * 256 + ncol) * 4;
+  CUDA_TRY(cudaFuncSetAttribute(cs::k_hist, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // enough blocks to fill the GPU; at most 2^31 items per block so that the 32-bit shared counters cannot wrap
+  const long long items = std::min<long long>(v.W, v.nlocal) * v.nsel;
+  long long bx = std::max<long long>(1, (long long)ctx->sm_count * 4 / nls);
+  bx = std::min<long long>(bx, (items + cs::HIST_THREADS - 1) / cs::HIST_THREADS);
+  bx = std::max<long long>(bx, (items >> 31) + 1);
+  if (nls > 65535 || bx > 0x7fffffffLL) {
+    rb_set_error(std::string(who) + ": too many sources on this rank");
+    return RB_ERR_ARG;
+  }
+  cs::k_hist<<<dim3((unsigned)bx, (unsigned)nls), cs::HIST_THREADS, smem, ctx->stream>>>(
+      v, cols, pass, nprefix, reinterpret_cast<const unsigned long long *>(prefix),
+      reinterpret_cast<unsigned long long *>(counts), reinterpret_cast<unsigned long long *>(nan_counts));
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches += 1;
+  return RB_OK;
+}
+
+int rb_chain_moments_dev(rb_ctx *ctx, const rb_chain_view *view, double *mean, double *c0) {
+  static const char *who = "rb_chain_moments_dev";
+  cs::View v;
+  int rc = chain_view(who, view, INT32_MAX, &v);
+  if (rc != RB_OK) return rc;
+  if (!mean || !c0) {
+    rb_set_error(std::string(who) + ": null output");
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long n = v.nlocal * v.ndim;
+  if (n == 0) return RB_OK;
+  cs::k_moments<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(v, mean, c0);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches += 1;
+  return RB_OK;
+}
+
+int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *mean, const double *c0,
+                     int64_t k0, int64_t k1, double *rho_sum) {
+  static const char *who = "rb_chain_acf_dev";
+  cs::View v;
+  int rc = chain_view(who, view, nsrc, &v);
+  if (rc != RB_OK) return rc;
+  if (!mean || !c0 || !rho_sum || nsrc < 1 || k0 < 0 || k1 <= k0 || k1 > v.nsel) {
+    rb_set_error(std::string(who) + ": bad argument (need 0 <= k0 < k1 <= selected steps)");
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long nl_all = k1 - k0;
+  CUDA_TRY(cudaMemsetAsync(rho_sum, 0, (size_t)nsrc * nl_all * v.ndim * sizeof(double), ctx->stream));
+  const long long nls = local_sources(v);
+  if (nls == 0) return RB_OK;
+  long long lo, hi;
+  cs::local_range(v, 0, lo, hi);
+  const long long ng0 = (hi - lo + cs::ACF_GROUP - 1) / cs::ACF_GROUP;
+  const long long ngW = (v.W + cs::ACF_GROUP - 1) / cs::ACF_GROUP;
+  // blocks: ng0 groups of the first local source, ngW of every later one but the last, which may hold fewer walkers
+  long long nb = ng0;
+  if (nls > 1) {
+    long long l2, h2;
+    cs::local_range(v, nls - 1, l2, h2);
+    nb += (nls - 2) * ngW + (h2 - l2 + cs::ACF_GROUP - 1) / cs::ACF_GROUP;
+  }
+  const size_t need = (size_t)nb * std::min<long long>(nl_all, cs::ACF_LAGS) * v.ndim * sizeof(double);
+  if (need > ctx->cs_bytes) {
+    if (ctx->cs_buf) cudaFree(ctx->cs_buf);
+    ctx->cs_buf = nullptr;
+    ctx->cs_bytes = 0;
+    CUDA_TRY(cudaMalloc(&ctx->cs_buf, need));
+    ctx->cs_bytes = need;
+  }
+  double *partial = static_cast<double *>(ctx->cs_buf);
+  const size_t smem = (size_t)v.ndim * (2 * cs::ACF_TT + cs::ACF_LAGS + 2 * cs::ACF_R) * sizeof(double);
+  CUDA_TRY(cudaFuncSetAttribute(cs::k_acf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  for (long long kb = k0; kb < k1; kb += cs::ACF_LAGS) {
+    const int nl = (int)std::min<long long>(cs::ACF_LAGS, k1 - kb);
+    cs::k_acf<<<(unsigned)nb, v.ndim * (cs::ACF_LAGS / cs::ACF_R), smem, ctx->stream>>>(v, mean, c0, kb, nl, ng0, ngW,
+                                                                                         partial);
+    CUDA_TRY(cudaGetLastError());
+    // rho_sum is [nsrc][k1 - k0][ndim]; this launch fills lags [kb, kb + nl) through a temporary view of its rows
+    const long long per = (long long)nl * v.ndim, nout = nls * per;
+    cs::k_acf_reduce<<<(unsigned)((nout + 255) / 256), 256, 0, ctx->stream>>>(v, nl, ng0, ngW, nls, partial,
+                                                                             rho_sum, nl_all, kb - k0);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches += 2;
+  }
   return RB_OK;
 }
 

@@ -16,6 +16,13 @@ What differs from the reference, on purpose:
   * fluxes in the pickle are plain float arrays in Jy km/s, not astropy Quantities.
 With ``torchrun`` every rank takes the sources ``rank::world_size`` on its own GPU: replicas, no
 communication (BASELINE.json configs[3]).
+
+The 16/50/84 percentiles (``summary``) and ``theta_med`` are computed on the device from the stored chain
+(``StretchSampler.get_quantiles``: the same values ``np.percentile`` gives on the host chain), and the result gains
+``autocorr_time`` (emcee's integrated autocorrelation time per parameter).  With ``chain_to_host=False``
+(CLI ``--summaries-only``) the chain is never gathered or copied to the host: ``chain`` and ``lnprobability`` of the
+result are ``None``, and so is the pickle's ``(chain, lnprobability)`` slot.  That is the only way to run ensembles whose
+chain does not fit in host memory (``--walkers 1048576``).
 """
 from __future__ import annotations
 
@@ -96,6 +103,28 @@ def posterior_summary(flatchain, ncomp):
     return out
 
 
+def summary_columns(ncomp):
+    """get_quantiles columns of the drivers' summaries: the 4 ncomp parameters, then log P = log n + log T per
+    component."""
+    return list(range(4 * ncomp)) + [(4 * c, 4 * c + 1) for c in range(ncomp)]
+
+
+def summaries_from_quantiles(Q, ncomp):
+    """(summary, theta_med) from get_quantiles([16, 50, 84], columns=summary_columns(ncomp)) of one source ([3, ncol]):
+    the same values and types posterior_summary and np.percentile(flatchain, 50, axis=0) give on the host chain."""
+    ndim = 4 * ncomp
+    out = []
+    for c in range(ncomp):
+        sel = [4 * c, 4 * c + 1, 4 * c + 2, ndim + c]
+        lo, med, hi = Q[0, sel], Q[1, sel], Q[2, sel]
+        out.append(dict(zip(("n_H2", "T_kin", "N_CO/dv", "P"), [(m, h - m, m - l) for l, m, h in zip(lo, med, hi)])))
+    return out, np.array(Q[1, :ndim])
+
+
+def log_autocorr(source, tau):
+    logger.info("%s: integrated autocorrelation time (steps) %s", source, np.array2string(np.asarray(tau), precision=1))
+
+
 def nearest_sample_to_vector(samples, target, metric="mahalanobis", eps=1e-9):
     """Sample closest to ``target``: (sample, index, squared distance); metrics as in
     emcee_radex.py:242-266 ('mahalanobis' with a regularised covariance, 'z' = per-axis standardised,
@@ -170,9 +199,11 @@ def prefit(ncomp, R, Jup, flux, eflux, bounds, p0, T_d=None, opts=None):
 
 
 def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
-               device=0, datapath=None, opts=None, outdir=None, store_chain=True, allow_synthetic=False):
+               device=0, datapath=None, opts=None, outdir=None, store_chain=True, allow_synthetic=False,
+               chain_to_host=True):
     """One pass of the reference's per-source loop.  Returns a dict with every item of the pickle plus
-    the percentile summaries and the sampler's acceptance fraction."""
+    the percentile summaries, the sampler's acceptance fraction and the integrated autocorrelation time.
+    ``chain_to_host=False``: the chain stays on the device (``chain`` and ``lnprobability`` are None)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -209,13 +240,15 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
     sampler.reset()
     logger.info("walking")
     sampler.run_mcmc(None, n_iter_walk, store=store_chain)
-    chain = sampler.get_chain()
-    lnprobability = sampler.get_log_prob()
-    flatchain = chain.reshape(-1, ndim)
-    theta_med = np.percentile(flatchain, 50, axis=0)
+    summary, theta_med = summaries_from_quantiles(
+        sampler.get_quantiles([16, 50, 84], columns=summary_columns(ncomp))[0], ncomp)
+    tau = sampler.get_autocorr_time(quiet=True)[0]
+    log_autocorr(source, tau)
+    chain = sampler.get_chain() if chain_to_host else None
+    lnprobability = sampler.get_log_prob() if chain_to_host else None
     result = dict(source=source, z=z, bounds=bounds, T_d=T_d, data=(Jup, flux, eflux), popt=popt, pcov=pcov,
                   pmin=pmin, theta_med=theta_med, chain=chain, lnprobability=lnprobability,
-                  summary=posterior_summary(flatchain, ncomp),
+                  summary=summary, autocorr_time=tau,
                   acceptance_fraction=float(np.mean(sampler.acceptance_fraction)),
                   acceptance_fraction_per_walker=sampler.acceptance_fraction,
                   prefit_info=info, solves=int(eng.total_solves.item()) + sampler.total_solves,
@@ -235,13 +268,13 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
 
 
 def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
-                             device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False):
+                             device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False, chain_to_host=True):
     """BASELINE.json configs[3]: every source of the table in ONE ensemble.  The reference fits the sources one after the
     other (emcee_radex.py:389); here the pre-fits run per source (they are a few dozen batched launches each) and the
     walkers of all sources -- each with its own background temperature, bounds, line set and, with two components, dust
     temperature -- step together: ``nwalkers`` per source, partners drawn inside the source's own sub-ensemble, one fused
     lnprob launch per half-step for all of them.  Under torchrun the ensemble is sharded over the ranks (whole sources per
-    rank).  Returns one result dict per source, the same items ``fit_source`` returns."""
+    rank).  Returns one result dict per source, the same items ``fit_source`` returns (``chain_to_host`` as there)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -280,14 +313,19 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
     sampler.reset()
     logger.info("walking")
     sampler.run_mcmc(None, n_iter_walk)
-    chain, lnp, acc = sampler.get_chain(), sampler.get_log_prob(), sampler.acceptance_fraction
+    Q = sampler.get_quantiles([16, 50, 84], columns=summary_columns(ncomp))
+    taus = sampler.get_autocorr_time(quiet=True)
+    acc = sampler.acceptance_fraction
+    chain, lnp = (sampler.get_chain(), sampler.get_log_prob()) if chain_to_host else (None, None)
     results = []
     for k, st in enumerate(setups):
         sl = slice(k * nwalkers, (k + 1) * nwalkers)
-        c, l = np.ascontiguousarray(chain[:, sl]), np.ascontiguousarray(lnp[:, sl])
-        flat = c.reshape(-1, ndim)
-        res = dict(st, theta_med=np.percentile(flat, 50, axis=0), chain=c, lnprobability=l,
-                   summary=posterior_summary(flat, ncomp), acceptance_fraction=float(np.mean(acc[sl])),
+        c, l = (np.ascontiguousarray(chain[:, sl]), np.ascontiguousarray(lnp[:, sl])) if chain_to_host else (None, None)
+        summary, theta_med = summaries_from_quantiles(Q[k], ncomp)
+        if sampler.rank == 0:
+            log_autocorr(st["source"], taus[k])
+        res = dict(st, theta_med=theta_med, chain=c, lnprobability=l, summary=summary, autocorr_time=taus[k],
+                   acceptance_fraction=float(np.mean(acc[sl])),
                    acceptance_fraction_per_walker=acc[sl], molfile=R.molpath, molfile_synthetic=R.molfile_is_synthetic)
         if outdir is not None and sampler.rank == 0:
             os.makedirs(outdir, exist_ok=True)
@@ -338,6 +376,10 @@ def main(argv=None):
                     help="all sources in one ensemble (BASELINE configs[3]); with torchrun the ensemble is sharded over the ranks")
     ap.add_argument("--allow-synthetic", action="store_true",
                     help="fit with the synthetic test table shipped in the package (NOT physical)")
+    ap.add_argument("--summaries-only", action="store_true",
+                    help="keep the chain on the GPU: percentiles and autocorrelation times are computed there, the "
+                         "pickles hold None for (chain, lnprobability); needed for ensembles whose chain does not fit "
+                         "in host memory")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -355,7 +397,8 @@ def main(argv=None):
             dist.init_process_group("nccl", device_id=torch.device("cuda", device))
         for res in fit_sources_concurrently(sources, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                                             n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir,
-                                            datapath=args.datapath, allow_synthetic=args.allow_synthetic):
+                                            datapath=args.datapath, allow_synthetic=args.allow_synthetic,
+                                            chain_to_host=not args.summaries_only):
             if rank == 0:
                 print_summary(res, args.ncomp)
         if world > 1:
@@ -365,7 +408,7 @@ def main(argv=None):
         logger.info("Processing %s on GPU %d", source, device)
         res = fit_source(source, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                          n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir, datapath=args.datapath,
-                         allow_synthetic=args.allow_synthetic)
+                         allow_synthetic=args.allow_synthetic, chain_to_host=not args.summaries_only)
         print_summary(res, args.ncomp)
 
 

@@ -25,6 +25,11 @@ Sharding
   independent of G.  On one GPU the whole loop runs inside the library (``rb_stretch_run_dev``; small
   ensembles replay a CUDA graph of one step) -- same kernels, same chain.
 
+Posterior statistics where the chain lives
+  ``get_quantiles`` (exact ``np.percentile`` of every source's flattened chain) and ``get_autocorr_time``
+  (emcee's integrated autocorrelation time) read the stored chain in place on every rank (csrc/chain_stats.cuh):
+  only 256-bin digit histograms and per-lag sums cross ranks (``all_reduce``) and PCIe, never the chain.
+
 The arithmetic is behind an ``engine`` object so that the host logic (sharding, gather order,
 bookkeeping) can be exercised on CPU by the test-suite's engine (tests/ref_engine.py); the
 package itself only ships the CUDA engine -- there is no CPU fallback in the product path.
@@ -32,11 +37,75 @@ package itself only ships the CUDA engine -- there is no CPU fallback in the pro
 from __future__ import annotations
 
 import ctypes as C
+import logging
 
 import numpy as np
 import torch
 
 from . import _lib
+
+logger = logging.getLogger("radex_emcee_b200.sampler")
+
+ACF_LAG_BLOCK = 128            # lags per rb_chain_acf_dev call; get_autocorr_time stops once every window is found
+NO_PREFIX = np.uint64(0xFFFFFFFFFFFFFFFF)
+
+
+class AutocorrError(Exception):
+    """emcee's ``AutocorrError``: the chain is shorter than ``tol`` integrated autocorrelation times.  ``tau`` holds
+    the estimate (in thinned steps, as emcee's ``integrated_time`` returns it)."""
+
+    def __init__(self, tau, *args, **kwargs):
+        self.tau = tau
+        super().__init__(*args, **kwargs)
+
+
+class ChainView:
+    """One rank's stored chain as the chain-statistics kernels read it (rb_chain_view): chunks [steps_i, nlocal, ndim]
+    in place, and emcee's ``discard`` / ``thin`` over the concatenated step index (steps discard + thin - 1,
+    discard + 2 thin - 1, ...)."""
+
+    def __init__(self, chunks, nlocal, ndim, gid_base, walkers_per_source, discard, thin):
+        self.chunks = list(chunks)
+        self.nlocal, self.ndim, self.gid_base = int(nlocal), int(ndim), int(gid_base)
+        self.walkers_per_source, self.discard, self.thin = int(walkers_per_source), int(discard), int(thin)
+        if self.discard < 0 or self.thin < 1:
+            raise ValueError("discard must be >= 0 and thin >= 1")
+        self.nsteps = sum(int(c.shape[0]) for c in self.chunks)
+        self.nsel = len(range(self.discard + self.thin - 1, self.nsteps, self.thin))
+
+    def c_struct(self):
+        if len(self.chunks) > _lib.RB_MAX_CHUNKS:
+            raise ValueError("at most %d chunks" % _lib.RB_MAX_CHUNKS)
+        v = _lib.rb_chain_view()
+        for k, c in enumerate(self.chunks):
+            if not c.is_contiguous() or tuple(c.shape[1:]) != (self.nlocal, self.ndim) or c.dtype != torch.float64:
+                raise ValueError("chain chunks must be contiguous float64 [steps, nlocal, ndim]")
+            v.chunk[k] = c.data_ptr()
+            v.steps[k] = int(c.shape[0])
+        v.nchunks, v.ndim, v.nlocal, v.gid_base = len(self.chunks), self.ndim, self.nlocal, self.gid_base
+        v.walkers_per_source, v.discard, v.thin = self.walkers_per_source, self.discard, self.thin
+        return v
+
+
+def _distinct_prefixes(pre):
+    """pre [..., m] uint64 -> (table [..., P] of the distinct prefixes, padded with NO_PREFIX; slot [..., m] of each)."""
+    order = np.argsort(pre, axis=-1, kind="stable")
+    srt = np.take_along_axis(pre, order, axis=-1)
+    new = np.ones(srt.shape, dtype=bool)
+    new[..., 1:] = srt[..., 1:] != srt[..., :-1]
+    rank = np.cumsum(new, axis=-1) - 1
+    table = np.full(pre.shape[:-1] + (int(rank.max()) + 1,), NO_PREFIX, dtype=np.uint64)
+    np.put_along_axis(table, rank, srt, axis=-1)
+    slot = np.empty_like(rank)
+    np.put_along_axis(slot, order, rank, axis=-1)
+    return table, slot
+
+
+def _key_to_double(key):
+    """Inverse of the kernels' order-preserving key (csrc/chain_stats.cuh order_key)."""
+    key = np.asarray(key, dtype=np.uint64)
+    neg = (key >> np.uint64(63)) == 0
+    return np.where(neg, ~key, key ^ np.uint64(1 << 63)).view(np.float64)
 
 
 class SLEDModel:
@@ -172,6 +241,42 @@ class CudaEngine:
                                                  logfac.data_ptr(), naccept.data_ptr(), counters.data_ptr()))
         self.launches += 1
 
+    # ---- chain statistics (csrc/chain_stats.cuh) -------------------------------------------------------
+    def chain_hist(self, view, nsrc, cols, pass_, prefix):
+        """One digit pass: counts [nsrc, ncol, nprefix, 256] (int64) for the prefixes [nsrc, ncol, nprefix] (uint64)
+        and, on pass 0, NaN counts [nsrc, ncol]."""
+        self._bind_stream()
+        ncol, P = len(cols), prefix.shape[2]
+        ci = (C.c_int32 * ncol)(*[i for i, _ in cols])
+        cj = (C.c_int32 * ncol)(*[j for _, j in cols])
+        pre = torch.from_numpy(np.ascontiguousarray(prefix, dtype=np.uint64).view(np.int64)).to(self.device)
+        counts = torch.zeros((nsrc, ncol, P, 256), dtype=torch.int64, device=self.device)
+        nans = torch.zeros((nsrc, ncol), dtype=torch.int64, device=self.device) if pass_ == 0 else None
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_hist_dev(self.ctx.handle, C.byref(vs), nsrc, ncol, ci, cj, pass_, P, pre.data_ptr(),
+                                            counts.data_ptr(), nans.data_ptr() if nans is not None else None))
+        self.launches += 1
+        return counts, nans
+
+    def chain_moments(self, view):
+        self._bind_stream()
+        mean = torch.empty((view.nlocal, view.ndim), dtype=torch.float64, device=self.device)
+        c0 = torch.empty_like(mean)
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_moments_dev(self.ctx.handle, C.byref(vs), mean.data_ptr(), c0.data_ptr()))
+        self.launches += 1
+        return mean, c0
+
+    def chain_acf(self, view, nsrc, mean, c0, k0, k1):
+        """[nsrc, k1 - k0, ndim]: sum over each source's local walkers of c_k / c_0."""
+        self._bind_stream()
+        out = torch.empty((nsrc, k1 - k0, view.ndim), dtype=torch.float64, device=self.device)
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_acf_dev(self.ctx.handle, C.byref(vs), nsrc, mean.data_ptr(), c0.data_ptr(), k0, k1,
+                                           out.data_ptr()))
+        self.launches += 1
+        return out
+
     def run_native(self, split, a, step0, nsteps, X, lnp, naccept, counters, thin, chain, lnp_chain):
         """nsteps steps of the whole (single-rank) ensemble inside the library."""
         self._bind_stream()
@@ -202,7 +307,8 @@ def walkers_independent(coords):
 
 class StretchSampler:
     """``EnsembleSampler``-like driver: ``run_mcmc``, ``get_chain``, ``get_log_prob``, ``reset``,
-    ``acceptance_fraction`` (per walker, like emcee)."""
+    ``acceptance_fraction`` (per walker, like emcee), ``get_autocorr_time``, and ``get_quantiles`` (exact
+    percentiles of the stored chain without moving it)."""
 
     def __init__(self, nwalkers, ndim, engine, a=2.0, seed=0, group=None, randomize_split=True, nsources=1,
                  split_block=None, native=True, time_gather=False):
@@ -321,14 +427,25 @@ class StretchSampler:
                     self._lnp_chain.append(lchain)
                 self._check_nan()
                 return None
-        for _ in range(nsteps):
-            self._half_step(0)
-            self._half_step(1)
-            self.step += 1
-            self.nsteps_done += 1
-            if store and (self.nsteps_done % thin == 0):
-                self._chain.append(self.X.clone()[None])
-                self._lnp_chain.append(self.lnp.clone()[None])
+        # one chunk per call, as in the native loop: the chain-statistics kernels take at most RB_MAX_CHUNKS chunks
+        nstore = (self.nsteps_done + nsteps) // thin - self.nsteps_done // thin if store else 0
+        chain = torch.empty((nstore, self.nlocal, self.ndim), dtype=torch.float64, device=self.device)
+        lchain = torch.empty((nstore, self.nlocal), dtype=torch.float64, device=self.device)
+        k = 0
+        try:
+            for _ in range(nsteps):
+                self._half_step(0)
+                self._half_step(1)
+                self.step += 1
+                self.nsteps_done += 1
+                if store and (self.nsteps_done % thin == 0):
+                    chain[k].copy_(self.X)
+                    lchain[k].copy_(self.lnp)
+                    k += 1
+        finally:
+            if k:
+                self._chain.append(chain[:k])
+                self._lnp_chain.append(lchain[:k])
         self._check_nan()
         return None
 
@@ -341,22 +458,152 @@ class StretchSampler:
         """(positions (nwalkers, ndim), lnprob (nwalkers,)) gathered over ranks, as numpy."""
         return self._gather(self.X).cpu().numpy(), self._gather(self.lnp).cpu().numpy()
 
-    def _stacked(self, parts, tail):
+    def _stacked(self, parts, tail, discard, thin):
+        discard, thin = int(discard), int(thin)
+        if discard < 0 or thin < 1:
+            raise ValueError("discard must be >= 0 and thin >= 1")
         if not parts:
             return np.empty((0, self.nwalkers) + tail)
-        loc = torch.cat(parts)                               # steps, nlocal, ...
+        loc = torch.cat(parts)[discard + thin - 1::thin]     # steps, nlocal, ...  (emcee's selection)
         if self.world > 1:
             loc = self._gather(loc.transpose(0, 1).contiguous()).transpose(0, 1)
         return loc.cpu().numpy()
 
-    def get_chain(self, flat=False):
-        """(steps, nwalkers, ndim) like emcee v3's ``get_chain``."""
-        c = self._stacked(self._chain, (self.ndim,))
+    def get_chain(self, flat=False, discard=0, thin=1):
+        """(steps, nwalkers, ndim) like emcee v3's ``get_chain``: steps discard + thin - 1, discard + 2 thin - 1, ...
+        Gathers the whole selection onto every rank and copies it to the host; for summaries of a large chain use
+        ``get_quantiles`` / ``get_autocorr_time``, which leave it on the device."""
+        c = self._stacked(self._chain, (self.ndim,), discard, thin)
         return c.reshape(-1, self.ndim) if flat else c
 
-    def get_log_prob(self, flat=False):
-        c = self._stacked(self._lnp_chain, ())
+    def get_log_prob(self, flat=False, discard=0, thin=1):
+        c = self._stacked(self._lnp_chain, (), discard, thin)
         return c.reshape(-1) if flat else c
+
+    # ---- posterior statistics on the device -----------------------------------------------------------
+    def _chain_view(self, discard, thin):
+        if len(self._chain) > _lib.RB_MAX_CHUNKS:         # more run_mcmc calls than the kernels take chunks
+            self._chain = [torch.cat(self._chain)]
+        return ChainView(self._chain, self.nlocal, self.ndim, self.gid_base, self.split.walkers_per_source, discard, thin)
+
+    def _allreduce(self, t):
+        if self.world > 1:
+            self.dist.all_reduce(t, op=self.dist.ReduceOp.SUM, group=self.group)
+        return t
+
+    def _columns(self, columns):
+        cols = []
+        for c in (range(self.ndim) if columns is None else columns):
+            i, j = (c, -1) if isinstance(c, (int, np.integer)) else tuple(c)
+            i, j = int(i), int(j)
+            if not (0 <= i < self.ndim and -1 <= j < self.ndim) or (j == -1 and not isinstance(c, (int, np.integer))):
+                raise ValueError("a column is a parameter index or a pair of them, in [0, %d)" % self.ndim)
+            cols.append((i, j))
+        if not 1 <= len(cols) <= _lib.RB_CHAIN_MAX_COLS:
+            raise ValueError("between 1 and %d columns" % _lib.RB_CHAIN_MAX_COLS)
+        return cols
+
+    def _order_statistics(self, view, cols, ranks):
+        """Values of the given 0-based ranks (ascending) of every (source, column): [nsources, len(ranks), ncol], and
+        which (source, column) holds a NaN.  Radix select, 8 digit passes over the chain per group of ranks."""
+        S, ncol = self.nsources, len(cols)
+        out = np.empty((S, len(ranks), ncol))
+        has_nan = None
+        per = max(1, _lib.RB_CHAIN_MAX_HIST // ncol)
+        for g0 in range(0, len(ranks), per):
+            m = len(ranks[g0:g0 + per])
+            rem = np.broadcast_to(np.asarray(ranks[g0:g0 + per], dtype=np.int64), (S, ncol, m)).copy()
+            pre = np.zeros((S, ncol, m), dtype=np.uint64)
+            for p in range(8):
+                if p == 0:
+                    table, slot = np.zeros((S, ncol, 1), dtype=np.uint64), np.zeros((S, ncol, m), dtype=np.int64)
+                else:
+                    table, slot = _distinct_prefixes(pre)
+                counts, nans = self.engine.chain_hist(view, S, cols, p, table)
+                counts = self._allreduce(counts).cpu().numpy()
+                if p == 0 and has_nan is None:
+                    has_nan = self._allreduce(nans).cpu().numpy() > 0
+                h = np.take_along_axis(counts, slot[..., None], axis=2)             # [S, ncol, m, 256]
+                cum = np.cumsum(h, axis=-1)
+                digit = np.minimum((cum <= rem[..., None]).sum(axis=-1), 255)      # (a NaN column holds fewer values)
+                rem -= np.take_along_axis(cum - h, digit[..., None], axis=-1)[..., 0]
+                pre = (pre << np.uint64(8)) | digit.astype(np.uint64)
+            out[:, g0:g0 + m] = _key_to_double(pre).transpose(0, 2, 1)
+        return out, has_nan
+
+    def get_quantiles(self, q, discard=0, thin=1, columns=None):
+        """Percentiles of the stored chain per source: [nsources, len(q), ncol], every value equal to
+        ``np.percentile(get_chain(flat=True, discard=discard, thin=thin)[rows of the source], q, axis=0)`` (numpy's
+        default 'linear' method; NaN where a column holds a NaN).  A column is a parameter index ``i`` or a pair
+        ``(i, j)`` for x[i] + x[j]; the default is the ``ndim`` parameters.  The chain is read in place; only digit
+        histograms cross ranks and PCIe.  The two order statistics around each percentile are exact (radix select on
+        the device), and the interpolation between them is numpy's own arithmetic (numpy/lib/_function_base_impl.py:
+        _quantile, _get_indexes, _get_gamma, _lerp)."""
+        view = self._chain_view(discard, thin)
+        cols = self._columns(columns)
+        qq = np.true_divide(np.asarray(q, dtype=np.float64).reshape(-1), np.float64(100))
+        if not (np.all(qq >= 0) and np.all(qq <= 1)):
+            raise ValueError("Percentiles must be in the range [0, 100]")
+        n = view.nsel * self.split.walkers_per_source
+        if n == 0:
+            raise ValueError("no stored samples are selected")
+        v = (n - 1) * qq
+        prev = np.floor(v)
+        nxt = prev + 1
+        above = v >= n - 1
+        prev[above] = -1
+        nxt[above] = -1
+        gamma = np.asanyarray(v - prev, dtype=v.dtype)
+        ip, inx = prev.astype(np.intp) % n, nxt.astype(np.intp) % n
+        ranks = np.unique(np.concatenate([ip, inx]))
+        xs, has_nan = self._order_statistics(view, cols, ranks)
+        a, b = xs[:, np.searchsorted(ranks, ip)], xs[:, np.searchsorted(ranks, inx)]
+        t = gamma[None, :, None]
+        with np.errstate(invalid="ignore"):
+            diff = np.subtract(b, a)
+            out = np.asanyarray(np.add(a, diff * t))
+            np.subtract(b, diff * (1 - t), out=out, where=t >= 0.5)
+        out[np.broadcast_to(has_nan[:, None, :], out.shape)] = np.nan
+        return out
+
+    def _integrated_time(self, discard, thin, c):
+        """emcee's integrated_time per (source, parameter) with the device acf: (tau in thinned steps, window, n_t)."""
+        view = self._chain_view(discard, thin)
+        n_t = view.nsel
+        if n_t == 0:
+            raise ValueError("no stored samples are selected")
+        mean, c0 = self.engine.chain_moments(view)
+        blocks, k1 = [], 0
+        while True:
+            k0, k1 = k1, min(n_t, k1 + ACF_LAG_BLOCK)
+            rho = self._allreduce(self.engine.chain_acf(view, self.nsources, mean, c0, k0, k1))
+            blocks.append(rho.cpu().numpy() / self.split.walkers_per_source)         # f: mean of rho over the walkers
+            taus = 2.0 * np.cumsum(np.concatenate(blocks, axis=1), axis=1) - 1.0
+            m = np.arange(k1)[None, :, None] < c * taus
+            # emcee's auto_window is settled once m turns False after a True; a NaN series is False throughout
+            settled = (m[:, 0] & (~m).any(axis=1)) | np.isnan(taus[:, 0])
+            if k1 == n_t or settled.all():
+                break
+        window = np.where(m.any(axis=1), m.argmin(axis=1), n_t - 1)
+        tau = np.take_along_axis(taus, np.minimum(window, k1 - 1)[:, None], axis=1)[:, 0]
+        return np.where(window < k1, tau, np.nan), window, n_t
+
+    def get_autocorr_time(self, discard=0, thin=1, c=5, tol=50, quiet=False):
+        """Integrated autocorrelation time per (source, parameter), [nsources, ndim], in steps: emcee's
+        ``get_autocorr_time`` / ``integrated_time`` (f = mean over the source's walkers of the normalised
+        autocovariance, taus = 2 cumsum(f) - 1, emcee's auto_window with constant ``c``) with the autocovariance summed
+        directly on the device.  Raises ``AutocorrError`` when tol * tau exceeds the number of selected steps (a
+        warning only, with ``quiet``).  A walker whose chain is constant makes its source's tau NaN."""
+        tau, _, n_t = self._integrated_time(discard, thin, c)
+        flag = tol * tau > n_t
+        if np.any(flag):
+            msg = ("The chain is shorter than {0} times the integrated autocorrelation time for {1} parameter(s). Use this "
+                   "estimate with caution and run a longer chain!\nN/{0} = {2:.0f};\ntau: {3}").format(
+                       tol, int(np.sum(flag)), n_t / tol, tau)
+            if not quiet:
+                raise AutocorrError(tau, msg)
+            logger.warning(msg)
+        return thin * tau
 
     @property
     def acceptance_fraction(self):

@@ -1277,6 +1277,9 @@ __global__ void k_lnprob_combine(LnprobIO io, LnprobPipe pp) {
     bool value_error = false;
 #pragma unroll
     for (int c = 0; c < NCOMP; ++c) {
+      // the reference stops at the first ValueError: a later component was solved here but is not counted, as in
+      // k_lnprob_v2
+      if (value_error) break;
       const long long m = idx * NCOMP + c;
       if (pp.status[m] & (RB_ST_T_RANGE | RB_ST_N_RANGE)) {
         value_error = true;

@@ -23,7 +23,7 @@ def ctx():
     return _lib.Context(_lib.MolData(MOLFILE), 0)
 
 
-def gpu_solve(ctx, T, nh2, N, tbg, method=2, **optkw):
+def gpu_solve(ctx, T, nh2, N, tbg, method=2, deltav_kms=1.0, **optkw):
     T, nh2, N = (np.ascontiguousarray(np.atleast_1d(a), dtype=np.float64) for a in (T, nh2, N))
     n = T.size
     mol = ctx.mol
@@ -33,8 +33,8 @@ def gpu_solve(ctx, T, nh2, N, tbg, method=2, **optkw):
     out = dict(xpop=np.empty((n, mol.nlev)), tex=np.empty((n, mol.nline)), tau=np.empty((n, mol.nline)),
                surf=np.empty((n, mol.nline)), niter=np.empty(n, np.int32), status=np.empty(n, np.int32))
     opts = _lib.default_opts(**optkw)
-    _lib.check(_lib.load().rb_solve_batch(ctx.handle, n, _lib.ptr(T), _lib.ptr(dens), _lib.ptr(N), 1.0, float(tbg),
-                                          method, C.byref(opts), _lib.ptr(out["xpop"]), _lib.ptr(out["tex"]),
+    _lib.check(_lib.load().rb_solve_batch(ctx.handle, n, _lib.ptr(T), _lib.ptr(dens), _lib.ptr(N), float(deltav_kms),
+                                          float(tbg), method, C.byref(opts), _lib.ptr(out["xpop"]), _lib.ptr(out["tex"]),
                                           _lib.ptr(out["tau"]), _lib.ptr(out["surf"]), _lib.ptr(out["niter"]),
                                           _lib.ptr(out["status"])))
     return out

@@ -6,9 +6,9 @@
 // k_lvg_solve_v2 they pay for the full engine they do not use (an 18.8 KB slab, 168 registers: 12 warps per SM), and
 // for n <= 16 -- three quarters of the sweep, nearly all of a converged ensemble -- half of the warp idles.  Here
 // every lead size has its own instantiation and launch: the pivot loops are straight-line code with constant
-// addresses, the slab holds just lead block + response matrix + pivot buffers + per-model line state (6.8 .. 15 KB),
+// addresses, the slab holds just lead block + response matrix + pivot buffers + per-model line state (6.4 .. 15 KB),
 // and for n <= 16 two models share a warp (lanes 0-15 / 16-31, each half with its own slab, iteration state and
-// queue ticket): 32 / 26 / 20 / 17 / 15 models per SM for 12 / 16 / 20 / 24 / 28 lead levels.
+// queue ticket): 36 / 28 / 20 / 16 / 14 models per SM for 12 / 16 / 20 / 24 / 28 lead levels.
 // There is NO full elimination in these kernels: launch A (v2::solve, sched = 1) captures the frozen top of a model
 // and parks lead block, response matrix and line bases (v2::ext_size(n) doubles); a model whose frozen lines turn thick is
 // parked again and finished by launch C (v2::solve, sched = 4).
@@ -47,37 +47,64 @@ using v2::st2;
 using v2::KP_SMALL_MAX;               // largest lead block (in panels) with an engine here
 using v2::EXT_LEAD;
 // ---- per-model shared-memory slab (doubles), for a lead block of N = 4 KP levels -------------------------
-// KP = 3: 870 doubles (6960 B, 32 models = 16 warps per SM); KP = 4: 1100 doubles (8800 B, 26 models = 13 warps)
+// KP = 3: 796 doubles (6368 B, 36 models = 18 warps per SM); KP = 4: 1026 doubles (8208 B, 28 models = 14 warps)
 template <int KP>
 struct Lay {
   static constexpr int N = 4 * KP;
   static constexpr int G = (KP <= 4 || V2S_TWO_ROWS) ? 16 : 32;   // lanes per model: a half-warp (two rows per lane above 16 lead levels), or a warp
   static constexpr int MPW = 32 / G;                  // models per warp
   static constexpr int NT = (v2::MAXLINE + G - 1) / G;   // trips over the lines
+  // lines that may be lead lines (both levels below N): the first 16 (KP <= 4) or 32.  A CO-like table has its N - 1
+  // lead lines there; the engines only run tables that do (lead_lines_fit), so the per-line slots that only lead
+  // lines read (S_BETA, S_DNB, S_UPB) exist for these lines only, and the trips LEAD_TRIPS are the only ones patched
+  static constexpr int NLEAD = (KP <= 4) ? 16 : 32;
+  static constexpr unsigned LEAD_TRIPS = (1u << (NLEAD / G)) - 1u;
   static constexpr int S_LEAD = 0;                    // lead block, row pitch N + 2
   static constexpr int S_M = N * (N + 2);             // M[i][f]: frozen populations from the lead ones, pitch 42 - N
   static constexpr int PBW = (N > 16) ? 32 : 16;      // a pivot row has up to N - 1 entries + 1/s_k in slot K
   static constexpr int S_PB = S_M + N * (MP - N);     // pivot-row broadcast buffers, 2 x PBW (1/s_k rides in slot K)
   static constexpr int S_VT = S_PB + 2 * PBW;         // raw pivot columns, triangular
   static constexpr int S_X = S_VT + N * (N - 1) / 2;  // relaxed populations
-  static constexpr int S_XNEW = S_X + 42;             // un-relaxed populations of this call
-  static constexpr int S_BETA = S_XNEW + 42;          // per line: escape probability of the call about to be made
-  static constexpr int S_DNB = S_BETA + 40;           //           non-radiative part of q[m][n] (collisions + Schur term)
-  static constexpr int S_UPB = S_DNB + 40;            //           non-radiative part of q[n][m]
-  static constexpr int S_TEX = S_UPB + 40;            //           excitation temperature
+  static constexpr int S_XNEW = S_X + NL;             // un-relaxed populations of this call
+  static constexpr int S_BETA = S_XNEW + NL;          // per line < NLEAD: escape probability of the call about to be made
+  static constexpr int S_DNB = S_BETA + NLEAD;        //                   non-radiative part of q[m][n] (collisions + Schur term)
+  static constexpr int S_UPB = S_DNB + NLEAD;         //                   non-radiative part of q[n][m]
+  static constexpr int S_TEX = S_UPB + NLEAD;         // per line: excitation temperature
   static constexpr int SSLAB = S_TEX + 40;
   // warps per CTA: bounded by the 227 KB of shared memory and by 65536 registers / (32 x registers per thread)
-  static constexpr int WARPS = (KP == 3) ? 16 : (KP == 4) ? 13 : (KP == 5) ? V2S_WARPS5 : (KP == 6) ? V2S_WARPS6 : V2S_WARPS7;
-  static_assert(SSLAB % 2 == 0 && S_M % 2 == 0 && S_PB % 2 == 0 && S_X % 2 == 0, "16 B alignment of the slab parts");
+  static constexpr int WARPS = (KP == 3) ? 18 : (KP == 4) ? 14 : (KP == 5) ? V2S_WARPS5 : (KP == 6) ? V2S_WARPS6 : V2S_WARPS7;
+  static_assert(SSLAB % 2 == 0 && S_M % 2 == 0 && S_PB % 2 == 0 && S_X % 2 == 0 && S_DNB % 2 == 0 && S_UPB % 2 == 0,
+                "16 B alignment of the slab parts");
 };
 // ---- per-CTA constants (the same for every model of a call) --------------------------------------------
-constexpr int C_LA = 0, C_LGR = 40, C_LTDEN = 80, C_LECOEF = 120, C_LFKXNU = 160, C_LMN = 200, CSLAB = 220;
+constexpr int C_LA = 0, C_LGR = 40, C_LTDEN = 80, C_LECOEF = 120, C_LFKXNU = 160, C_LMN = 200, C_XNU = 220, C_BACKI = 260,
+              CSLAB = 300;
 // parked capture (global, per model; v2::ext_size(n) doubles at io.ext + io.ext_off[model]): DNB[40] UPB[40] lead[n(n+2)] M[n(42-n)]
 template <int KP>
 constexpr size_t smem_bytes() { return (size_t)(CSLAB + Lay<KP>::MPW * Lay<KP>::WARPS * Lay<KP>::SSLAB) * sizeof(double); }
 static_assert(smem_bytes<3>() <= 232448 && smem_bytes<4>() <= 232448 && smem_bytes<5>() <= 232448 &&
                   smem_bytes<6>() <= 232448 && smem_bytes<7>() <= 232448,
               "slabs exceed the 227 KB of shared memory per CTA");
+
+// Do the lead lines of every engine lie in its first NLEAD lines?  Decided once per molecule table; a table that fails
+// runs its cached iterations in launch B instead (SolveCfg::small off), with the same arithmetic.
+template <int KP>
+inline bool lead_lines_fit_kp(const int *iupp, const int *ilow, int nline) {
+  for (int l = Lay<KP>::NLEAD; l < nline; ++l)
+    if (std::max(iupp[l], ilow[l]) < Lay<KP>::N) return false;
+  return true;
+}
+inline bool lead_lines_fit(const int *iupp, const int *ilow, int nline) {
+  return lead_lines_fit_kp<3>(iupp, ilow, nline) && lead_lines_fit_kp<4>(iupp, ilow, nline) &&
+         lead_lines_fit_kp<5>(iupp, ilow, nline) && lead_lines_fit_kp<6>(iupp, ilow, nline) &&
+         lead_lines_fit_kp<7>(iupp, ilow, nline);
+}
+
+// ---- hand-over of a model: 16-byte asynchronous copies global -> shared (SASS: LDGSTS), all in flight at once ----
+__device__ __forceinline__ void cp_async16(double *dst_smem, const double *src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(v2::smem_u32(dst_smem)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 template <int G>
 __device__ __forceinline__ double group_sum(double v) {   // butterfly over the G lanes of a model

@@ -99,6 +99,7 @@ struct rb_ctx {
   rb_source src_one_host{};               // ... and what it holds (no transfer while the caller keeps passing the same source)
   bool src_one_valid = false;
   bool ln_partners_ok = false;            // lnprob: the file has H2, or p-H2 / o-H2, as a collision partner
+  bool engines_fit = false;               // v2: the lead lines of every cached engine lie in its lead trips (v2s::lead_lines_fit)
   void *samp_buf = nullptr;               // rb_stretch_run_dev: complementary half, proposals, their lnprob, step counter (grow-only)
   size_t samp_bytes = 0;
   cudaEvent_t ev_samp = nullptr;
@@ -823,7 +824,7 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
   using L = Lay<KP>;
   static_assert(v2::IT_DECIDE >= 1, "the engines never run a model's first call (it == 0 has its own arithmetic in v2::solve)");
   constexpr int G = L::G, NT = L::NT;
-  constexpr int SSLAB = L::SSLAB, S_LEAD = L::S_LEAD, S_M = L::S_M, S_X = L::S_X, S_XNEW = L::S_XNEW, S_BETA = L::S_BETA,
+  constexpr int SSLAB = L::SSLAB, S_LEAD = L::S_LEAD, S_X = L::S_X, S_XNEW = L::S_XNEW, S_BETA = L::S_BETA,
                 S_DNB = L::S_DNB, S_UPB = L::S_UPB, S_TEX = L::S_TEX;
   extern __shared__ double smem[];
   double *cs = smem;   // per-line constants of this call, shared by the CTA
@@ -845,24 +846,48 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
     cs[C_LTDEN + l] = 1.0 / (RB_FGAUS * xt / a);
     cs[C_LECOEF + l] = bi / (RB_THC * xt);
     cs[C_LFKXNU + l] = RB_FK * xnu;
+    cs[C_XNU + l] = xnu;   // the epilogue's line constants: its backi is bi
+    cs[C_BACKI + l] = bi;
   }
   // a slab that never receives a model still runs the arithmetic of its warp: give it finite numbers
   for (int e = hl; e < SSLAB; e += G) sm[e] = 1.0;
   __syncthreads();
-  // trips over the lines (tt: lines G tt .. G tt + G - 1) that hold a lead line, i.e. a line whose escape probability can
-  // differ from 1 while the model stays in this engine.  A CO-like table (line l: l + 1 -> l) has its 4 KP - 1 lead lines
-  // in the first trip (KP <= 4) or the first two: the loop then evaluates escprob for those trips only (LEAD_FAST).
-  unsigned lead_trips = 0;
-  for (int l = 0; l < nn; ++l)
-    if (max(lmn[l] & 0xff, (lmn[l] >> 8) & 0xff) < 4 * KP) lead_trips |= 1u << (l / G);
-  constexpr unsigned LEAD_FAST = (G == 16 && KP > 4) ? 3u : 1u, LEAD_ALL = (1u << NT) - 1u;
-  const bool lead_fast = (lead_trips & ~LEAD_FAST) == 0;
+  // trips over the lines (tt: lines G tt .. G tt + G - 1) that can hold a lead line, i.e. a line whose escape probability
+  // can differ from 1 while the model stays in this engine: the first trip (KP <= 4) or the first two (the host runs the
+  // engines only for tables where this holds, lead_lines_fit).  Only these trips are patched and evaluate escprob.
+  constexpr unsigned LEAD_TRIPS = L::LEAD_TRIPS;
   // queue: the positions of key KP in the sorted order (heaviest key first; key 3 is the last block)
   const unsigned long long p_begin = io.sched_small[16 + KP], p_end = io.sched_small[(KP == 3) ? 48 : 16 + KP - 1];
   const double qnan = __longlong_as_double(0x7ff8000000000000LL);
 
+  // Hand-over.  Each half holds the queue ticket of its NEXT model while the current one iterates, and walks the chain
+  // ticket -> order[] -> ext_off[] one link per call (pf: 1 ticket taken, 2 model index loaded, 3 capture offset loaded
+  // and ready, 5 queue ended).  A model that ends before the chain does finishes it at once.  (An L2 prefetch of the next
+  // model's state and capture as a further link measured 0.3 % slower on the sweep.)  A ticket is always used by the half that took it, so no model is lost at the queue's end.
+  int pf = 0;
+  unsigned long long tk = 0;
+  long long nidx = 0, noff = 0;
+  auto advance = [&]() {
+    if (pf == 1) {
+      const unsigned long long pos = p_begin + __shfl_sync(hmask, tk, 0, G);
+      if (pos >= p_end) {
+        pf = 5;
+      } else {
+        nidx = io.order[pos];
+        pf = 2;
+      }
+    } else if (pf == 2) {
+      noff = io.ext_off[nidx];
+      pf = 3;
+    }
+  };
+  auto take_ticket = [&]() {
+    if (hl == 0) tk = atomicAdd(&io.counters[io.queue], 1ULL);
+    pf = 1;
+  };
+
   bool active = false, exhausted = false, need_load = false;
-  long long idx = 0;
+  long long idx = 0, off = 0;
   constexpr int Kp = KP, n = 4 * KP, pitch = n + 2;
   int it = 0, nthick = 0, topthick = -1;
   unsigned flags = 0;   // bit t: line hl + 16 t had tau > 0.01f after the last call (RADEX's own stop rule)
@@ -877,15 +902,15 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
     TM(tm0);
     // ---- a free half takes the next model of the queue -------------------------------------------------------------
     if (!active && !exhausted) {
-      unsigned long long t = 0;
-      if (hl == 0) t = atomicAdd(&io.counters[io.queue], 1ULL);
-      t = __shfl_sync(hmask, t, 0, G);
-      const unsigned long long pos = p_begin + t;
-      if (pos >= p_end) {
+      if (pf == 0) take_ticket();
+      while (pf < 3) advance();
+      if (pf == 5) {
         exhausted = true;
       } else {
-        idx = io.order[pos];
+        idx = nidx;
+        off = noff;
         active = need_load = true;
+        take_ticket();   // the next model's; its chain advances during this model's calls
       }
     }
     __syncwarp();
@@ -893,34 +918,51 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
     if (need_load) {
       need_load = false;
       const double *st = io.state + idx * v2::STATE_STRIDE;
-      const double *ex = io.ext + io.ext_off[idx];
-      for (int i = hl; i < NL; i += G) sm[S_X + i] = st[i];
+      const double *ex = io.ext + off;
+      // lead block + M (contiguous in ext and in the slab) and the lead lines' bases, as 16-byte asynchronous copies;
+      // the state loads below are issued while they are in flight
+      for (int c = hl; c < 22 * n; c += G) cp_async16(sm + S_LEAD + 2 * c, ex + EXT_LEAD + 2 * c);
+      for (int c = hl; c < L::NLEAD; c += G) {
+        const int o = (c < L::NLEAD / 2) ? 2 * c : v2::MAXLINE - L::NLEAD + 2 * c;   // DNB pairs, then UPB pairs
+        cp_async16(sm + S_DNB + 2 * c, ex + o);
+      }
       const unsigned long long bits = reinterpret_cast<const unsigned long long *>(st)[121];
       const long long packed = reinterpret_cast<const long long *>(st)[122];
+      const double cdm = io.cdmol[idx];
+      double xs[(NL + G - 1) / G], tex[NT], beta[NT];
+#pragma unroll
+      for (int t = 0; t < (NL + G - 1) / G; ++t) xs[t] = (hl + G * t < NL) ? st[hl + G * t] : 0.0;
+#pragma unroll
+      for (int t = 0; t < NT; ++t) {
+        const int l = hl + G * t;
+        tex[t] = (l < nn) ? st[41 + l] : 0.0;
+        beta[t] = (l < nn) ? st[81 + l] : 0.0;
+      }
+#pragma unroll
+      for (int t = 0; t < (NL + G - 1) / G; ++t)
+        if (hl + G * t < NL) sm[S_X + hl + G * t] = xs[t];
       flags = 0;
       beta_nan = false;
 #pragma unroll
       for (int t = 0; t < NT; ++t) {
         const int l = hl + G * t;
         if (l < nn) {
-          sm[S_TEX + l] = st[41 + l];
-          sm[S_BETA + l] = st[81 + l];
-          if (st[81 + l] != st[81 + l]) beta_nan = true;
-          sm[S_DNB + l] = ex[l];
-          sm[S_UPB + l] = ex[v2::MAXLINE + l];
+          sm[S_TEX + l] = tex[t];
+          if (l < L::NLEAD) sm[S_BETA + l] = beta[t];
+          if (beta[t] != beta[t]) beta_nan = true;
           flags |= (unsigned)((bits >> l) & 1ULL) << t;
         }
       }
       beta_nan = __any_sync(hmask, beta_nan);
       nthick = (int)(packed & 0xffffffffLL);
       topthick = (int)(packed >> 32);
-      const int nlead = n * (n + 2), nm = n * (MP - n);
-      for (int e = hl; e < nlead; e += G) sm[S_LEAD + e] = ex[EXT_LEAD + e];
-      for (int e = hl; e < nm; e += G) sm[S_M + e] = ex[EXT_LEAD + nlead + e];
       it = v2::IT_DECIDE;
-      cdmol = io.cdmol[idx];
+      cdmol = cdm;
       cddv = cdmol / cfg.deltav_cms;
       ++n_models;
+      cp_async_wait_all();
+    } else if (active && pf < 3) {
+      advance();
     }
     __syncwarp();
     TM(tm1);
@@ -929,7 +971,7 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
     // every model of the warp is about to make a call whose solution is NaN (v2::solve: beta_nan): no elimination
     const bool skip_solve = __all_sync(0xffffffffu, !active || beta_nan);
 #pragma unroll
-    for (int t = 0; t < NT; ++t) {
+    for (int t = 0; t < L::NLEAD / G; ++t) {
       const int l = hl + G * t;
       if (l < nn && !skip_solve) {
         const int m = lmn[l] & 0xff, nlo = (lmn[l] >> 8) & 0xff;
@@ -981,8 +1023,8 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
     unsigned nflags = 0;
     double diff = 0.0, tsA = 0.0, tsB = 0.0;
     bool nan_next = false;
-    auto lines = [&](auto em) {
-      constexpr unsigned EM = decltype(em)::value;   // trips whose lines get their escape probability evaluated
+    {
+      constexpr unsigned EM = LEAD_TRIPS;   // trips whose lines get their escape probability evaluated
       int ll[NT], lm[NT], ln[NT];
       bool lvalid[NT], lfloored[NT];
       double ltold[NT], larg[NT], ltaur[NT], ltex[NT], lmid[NT];
@@ -1048,8 +1090,7 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
           }
         }
       }
-    };
-    if (lead_fast) lines(std::integral_constant<unsigned, LEAD_FAST>()); else lines(std::integral_constant<unsigned, LEAD_ALL>());
+    }
     flags = nflags;
     beta_nan = __any_sync(hmask, nan_next);
     topthick = group_max_int(hmask, topthick);
@@ -1123,10 +1164,9 @@ __global__ void __launch_bounds__(v2s::Lay<KP>::WARPS * 32, 1) k_lvg_small(MolDe
 #pragma unroll 1
     for (int l = l_first; l < nn; l += l_step) {
       const int m = lmn[l] & 0xff, nlo = (lmn[l] >> 8) & 0xff;
-      const double xnu = mol.xnu[l];
+      const double xnu = cs[C_XNU + l];
       const double xt = xnu * xnu * xnu;
-      const double hnu = RB_FK * xnu / cfg.tbg;
-      const double backi = (hnu >= 160.0) ? 1.0e-30 : RB_THC * xt / (exp(hnu) - 1.0);
+      const double backi = cs[C_BACKI + l];
       const double tex = sm[S_TEX + l];
       const double tau = (cdmol / cfg.deltav_cms) * (sm[S_XNEW + nlo] * cs[C_LGR + l] - sm[S_XNEW + m]) * cs[C_LTDEN + l];
       const double ftau = exp(-tau);
@@ -1417,7 +1457,7 @@ SolveCfg make_cfg(const rb_ctx *ctx, const rb_opts *o, double deltav_kms, double
   c.thc_epi = d.thc_epi;
   c.cache = (d.kernel != 2);
   c.sched = (d.kernel == 0 || d.kernel == 4);
-  c.small = (d.kernel == 0);
+  c.small = (d.kernel == 0) && ctx->engines_fit;
   c.park_max = (d.park_max >= v2::KP_CACHE_MIN && d.park_max <= v2::KP_SMALL_MAX) ? d.park_max : 0;
   c.lnprob_pipe_min = (d.lnprob_pipe_min > 0) ? d.lnprob_pipe_min : RB_LNPROB_PIPE_MIN;
   c.stats = ctx->counters + 3;
@@ -1553,6 +1593,7 @@ int rb_ctx_create(int device, const rb_mol *mol, rb_ctx **out) {
   m.nline = mol->nline;
   m.npart = mol->npart;
   m.sorted_levels = 1;
+  ctx->engines_fit = v2s::lead_lines_fit(mol->iupp.data(), mol->ilow.data(), mol->nline);
   for (int i = 0; i + 1 < mol->nlev; ++i)
     if (!(mol->eterm[i + 1] > mol->eterm[i])) m.sorted_levels = 0;
   int rc = RB_OK;

@@ -261,6 +261,26 @@ int rb_chain_moments_dev(rb_ctx *ctx, const rb_chain_view *view, double *mean, d
 int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *mean, const double *c0,
                      int64_t k0, int64_t k1, double *rho_sum);
 
+/* ---- posterior-predictive SLEDs of the device-resident chain: replaces the host replot's model_lvg over the pickled
+ * chain (er1:120-130, er2:122-147), one Radex call per sample, without moving the chain.  DEVICE pointers except jup,
+ * asynchronous on the ctx stream; rb_ctx_counters / rb_ctx_cache_stats report the call like any solve call.
+ *   view   : the selected steps of the chain as in rb_chain_hist_dev; ndim = 4 x set->ncomp.  Local walker w belongs to
+ *            source (gid_base + w) / walkers_per_source, whose row of `set` gives tbg.
+ *   jup    : HOST int32[nlines], 1 <= nlines <= RB_MAX_OBS one-based line indices 1 <= J <= nline, in any order, repeats
+ *            allowed.
+ *   model  : per sample theta and component c: T = 10^theta[4c+1], N = 10^theta[4c+2], partner densities split from
+ *            10^theta[4c] as rb_lnprob1/2 do (opr = 3), LVG, deltav = 1 km/s, opts as given;
+ *            flux_c[J] = surf_c[J-1] * 10^theta[4c+3] * 1e23 (Jy km/s, er1:129).  No prior is applied.  A component out
+ *            of pyradex's range (RB_ST_T_RANGE / RB_ST_N_RANGE, where model_lvg raises ValueError) gives NaN.
+ *   flux   : [nplanes][nsel][nlocal][nlines], nsel = the view's selected steps.  One component: nplanes = 1, the flux.
+ *            Two: nplanes = 3, the total flux_0 + flux_1 (er2:147, NaN if either is), then component 1 (theta[0:4]) and
+ *            component 2 (theta[4:8]).  A plane is a chain chunk of ndim = nlines: rb_chain_hist_dev reads it as is.
+ *   counters_dev : NULL, or int64[2]: [0] += components solved, [1] += components out of range.
+ * Argument errors give RB_ERR_ARG (bad nlines or J, null pointers, a bad view, a set of another ctx, of another ncomp
+ * or without the view's sources), a machine without a CUDA device RB_ERR_CUDA.                                        */
+int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *view, int32_t nlines, const int32_t *jup,
+                        const rb_opts *opts, double *flux, int64_t *counters_dev);
+
 /* counters of the last solve/lnprob call on this ctx (device-measured, read back on request):
  * total matrix iterations summed over models, and kernels launched since ctx creation.        */
 int rb_ctx_counters(rb_ctx *ctx, int64_t *total_iters_last, int64_t *launches_total);

@@ -101,6 +101,8 @@ SIGNATURES = {
                                     _vp, _vp, _vp]),
     "rb_chain_moments_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), _vp, _vp]),
     "rb_chain_acf_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, _vp, _vp, C.c_int64, C.c_int64, _vp]),
+    "rb_predict_sled_dev": (C.c_int, [_vp, _vp, C.POINTER(rb_chain_view), C.c_int32, _ip, C.POINTER(rb_opts), _vp,
+                                      _vp]),
 }
 
 _lib = None

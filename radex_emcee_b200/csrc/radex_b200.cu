@@ -1406,6 +1406,7 @@ __global__ void k_stretch_accept(long long ns, int ndim, double *S, double *lnp_
 
 #include "stretch.cuh"
 #include "chain_stats.cuh"
+#include "predict_sled.cuh"
 
 // ------------------------------------------------------------------------------------------------
 // FP64 FMA peak probe: the roofline denominator for the solve kernels is the vector FP64 pipe,
@@ -2814,6 +2815,122 @@ int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const
                                                                              rho_sum, nl_all, kb - k0);
     CUDA_TRY(cudaGetLastError());
     ctx->launches += 2;
+  }
+  return RB_OK;
+}
+
+// ---- posterior-predictive SLEDs (predict_sled.cuh) ---------------------------------------------------------------
+#define RB_PREDICT_MAX (2 * RB_PIPE_MAX)   // models per pipeline call: bounds ctx->ln_buf however long the chain is
+
+int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *view, int32_t nlines, const int32_t *jup,
+                        const rb_opts *opts, double *flux, int64_t *counters_dev) {
+  static const char *who = "rb_predict_sled_dev";
+  std::string e;
+  if (!set || !jup || !flux) e = "null argument";
+  else if (nlines < 1 || nlines > RB_MAX_OBS) e = "nlines must be in 1..RB_MAX_OBS";
+  for (int k = 0; e.empty() && k < nlines; ++k)
+    if (jup[k] < 1) e = "J must be in 1..nline";
+  if (!e.empty()) {
+    rb_set_error(std::string(who) + ": " + e);
+    return RB_ERR_ARG;
+  }
+  cs::View v;
+  int rc = chain_view(who, view, INT32_MAX, &v);
+  if (rc != RB_OK) return rc;
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  if (set->ctx != ctx) e = "the source set belongs to another context";
+  else if (view->ndim != 4 * set->ncomp) e = "ndim is not 4 x the source set's ncomp";
+  else if (v.nlocal > 0 && (v.gid_base + v.nlocal - 1) / v.W >= set->nsrc) e = "the source set does not cover the rank's walkers";
+  else if (!ctx->ln_partners_ok) e = "the molecular file has no H2 / p-H2 / o-H2 collision partner";
+  for (int k = 0; e.empty() && k < nlines; ++k)
+    if (jup[k] > ctx->mol.nline) e = "J must be in 1..nline";
+  if (!e.empty()) {
+    rb_set_error(std::string(who) + ": " + e);
+    return RB_ERR_ARG;
+  }
+  CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, 8 * sizeof(unsigned long long), ctx->stream));
+  const long long nls = local_sources(v);
+  if (nls == 0 || v.nsel == 0) return RB_OK;
+  const int ncomp = set->ncomp, np = ctx->mol.npart, nn = ctx->mol.nline;
+  const bool v2 = use_v2(ctx, opts);
+  // v2: observed-line mode, line k of model m at obs_surf[m][k]; v1: every line, at surf[m][J - 1]
+  const int stride = v2 ? RB_MAX_OBS : nn;
+  long long total = 0;
+  for (long long s = 0; s < nls; ++s) {
+    long long lo, hi;
+    cs::local_range(v, s, lo, hi);
+    total = std::max(total, (hi - lo) * v.nsel);
+  }
+  const long long per_call = std::max<long long>(1, RB_PREDICT_MAX / ncomp);
+  const long long mmax = std::min(total, per_call) * ncomp;
+  const size_t b_d = align256((size_t)mmax * sizeof(double)), b_dn = align256((size_t)mmax * np * sizeof(double));
+  const size_t b_o = align256((size_t)mmax * stride * sizeof(double)), b_s = align256((size_t)mmax * sizeof(int));
+  const size_t b_all = 2 * b_d + b_dn + b_o + b_s;
+  if (b_all > ctx->ln_bytes) {
+    if (ctx->ln_buf) cudaFree(ctx->ln_buf);
+    ctx->ln_buf = nullptr;
+    ctx->ln_bytes = 0;
+    CUDA_TRY(cudaMalloc(&ctx->ln_buf, b_all));
+    ctx->ln_bytes = b_all;
+  }
+  char *base = static_cast<char *>(ctx->ln_buf);
+  PredictIO io;
+  memset(&io, 0, sizeof(io));
+  io.v = v;
+  io.tkin = reinterpret_cast<double *>(base);
+  io.cdmol = reinterpret_cast<double *>(base + b_d);
+  io.dens = reinterpret_cast<double *>(base + 2 * b_d);
+  double *surf = reinterpret_cast<double *>(base + 2 * b_d + b_dn);
+  int *status = reinterpret_cast<int *>(base + 2 * b_d + b_dn + b_o);
+  io.surf = surf;
+  io.status = status;
+  io.stride = stride;
+  io.nlines = nlines;
+  for (int k = 0; k < nlines; ++k) io.line[k] = v2 ? k : jup[k] - 1;
+  io.flux = flux;
+  io.counters = reinterpret_cast<unsigned long long *>(counters_dev);
+  const int tpb = 256;
+  for (long long s = 0; s < nls; ++s) {
+    long long lo, hi;
+    cs::local_range(v, s, lo, hi);
+    io.w0 = lo;
+    io.nw = hi - lo;
+    const SolveCfg cfg = make_cfg(ctx, opts, 1.0, set->h[v.src0 + s].tbg, RB_GEOM_LVG);   // model_lvg: LVG, 1 km/s
+    for (long long i0 = 0; i0 < io.nw * v.nsel; i0 += per_call) {
+      io.i0 = i0;
+      io.ni = std::min(per_call, io.nw * v.nsel - i0);
+      const long long m = io.ni * ncomp;
+      const unsigned nbe = (unsigned)((io.ni + tpb - 1) / tpb);
+      if (ncomp == 1)
+        k_predict_expand<1><<<nbe, tpb, 0, ctx->stream>>>(ctx->mol, io);
+      else
+        k_predict_expand<2><<<nbe, tpb, 0, ctx->stream>>>(ctx->mol, io);
+      CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, sizeof(unsigned long long), ctx->stream));   // queue head only
+      SolveIO sio{m, io.tkin, io.dens, io.cdmol, nullptr, nullptr, nullptr, v2 ? nullptr : surf, nullptr, status,
+                  ctx->counters, 0, nullptr, nullptr, nullptr, nullptr};
+      if (v2) {
+        sio.obs_surf = surf;
+        sio.nobs = nlines;
+        for (int k = 0; k < nlines; ++k) sio.obs_line[k] = jup[k] - 1;
+        const Launch L = v2_launch(ctx, m);
+        if (cfg.sched && cfg.cache && m >= RB_SCHED_MIN) {
+          rc = launch_solve_pipeline(ctx, cfg, sio, L);
+          if (rc != RB_OK) return rc;
+        } else {
+          k_lvg_solve_v2<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, sio);
+        }
+      } else {
+        const Launch L = v1_launch(ctx, m);
+        k_lvg_solve_v1<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, sio);
+      }
+      const unsigned nbf = (unsigned)((io.ni * nlines + tpb - 1) / tpb);
+      if (ncomp == 1)
+        k_predict_flux<1><<<nbf, tpb, 0, ctx->stream>>>(io);
+      else
+        k_predict_flux<2><<<nbf, tpb, 0, ctx->stream>>>(io);
+      CUDA_TRY(cudaGetLastError());
+      ctx->launches += 3;
+    }
   }
   return RB_OK;
 }

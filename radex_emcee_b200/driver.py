@@ -23,6 +23,10 @@ The 16/50/84 percentiles (``summary``) and ``theta_med`` are computed on the dev
 (CLI ``--summaries-only``) the chain is never gathered or copied to the host: ``chain`` and ``lnprobability`` of the
 result are ``None``, and so is the pickle's ``(chain, lnprobability)`` slot.  That is the only way to run ensembles whose
 chain does not fit in host memory (``--walkers 1048576``).
+
+With ``predict_jup`` (CLI ``--predict-sled J ...``) the result also gains the posterior-predictive SLED: the 16/50/84
+percentiles of the model flux of each requested line over the chain (``StretchSampler.get_predictive_quantiles``), per
+component with two components -- the model SLEDs the reference's replot draws from the pickled chain.
 """
 from __future__ import annotations
 
@@ -121,6 +125,19 @@ def summaries_from_quantiles(Q, ncomp):
     return out, np.array(Q[1, :ndim])
 
 
+def sled_summaries(Q, jup):
+    """Per plane of get_predictive_quantiles(jup, [16, 50, 84]) of one source ([nplanes, 3, nlines]): J -> (median, +err,
+    -err) of the predicted flux, as percentile_summary gives on the host."""
+    return [{int(J): (m, h - m, m - l) for J, l, m, h in zip(jup, *Qp)} for Qp in Q]
+
+
+def sled_results(sampler, jup):
+    """Per source: the result items of the posterior-predictive SLED, from the device-resident chain."""
+    jup = [int(J) for J in jup]
+    Q = sampler.get_predictive_quantiles(jup, [16, 50, 84])
+    return [dict(sled_jup=np.array(jup), sled_summary=sled_summaries(Qs, jup)) for Qs in Q]
+
+
 def log_autocorr(source, tau):
     logger.info("%s: integrated autocorrelation time (steps) %s", source, np.array2string(np.asarray(tau), precision=1))
 
@@ -200,10 +217,11 @@ def prefit(ncomp, R, Jup, flux, eflux, bounds, p0, T_d=None, opts=None):
 
 def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
                device=0, datapath=None, opts=None, outdir=None, store_chain=True, allow_synthetic=False,
-               chain_to_host=True):
+               chain_to_host=True, predict_jup=None):
     """One pass of the reference's per-source loop.  Returns a dict with every item of the pickle plus
     the percentile summaries, the sampler's acceptance fraction and the integrated autocorrelation time.
-    ``chain_to_host=False``: the chain stays on the device (``chain`` and ``lnprobability`` are None)."""
+    ``chain_to_host=False``: the chain stays on the device (``chain`` and ``lnprobability`` are None).
+    ``predict_jup``: line indices J whose posterior-predictive fluxes the result gains (``sled_jup``, ``sled_summary``)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -253,6 +271,8 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
                   acceptance_fraction_per_walker=sampler.acceptance_fraction,
                   prefit_info=info, solves=int(eng.total_solves.item()) + sampler.total_solves,
                   molfile=R.molpath, molfile_synthetic=R.molfile_is_synthetic)
+    if predict_jup is not None:
+        result.update(sled_results(sampler, predict_jup)[0])
     if outdir is not None:
         os.makedirs(outdir, exist_ok=True)
         if ncomp == 1:     # emcee_radex.py:504-509
@@ -268,13 +288,15 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
 
 
 def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
-                             device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False, chain_to_host=True):
+                             device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False, chain_to_host=True,
+                             predict_jup=None):
     """BASELINE.json configs[3]: every source of the table in ONE ensemble.  The reference fits the sources one after the
     other (emcee_radex.py:389); here the pre-fits run per source (they are a few dozen batched launches each) and the
     walkers of all sources -- each with its own background temperature, bounds, line set and, with two components, dust
     temperature -- step together: ``nwalkers`` per source, partners drawn inside the source's own sub-ensemble, one fused
     lnprob launch per half-step for all of them.  Under torchrun the ensemble is sharded over the ranks (whole sources per
-    rank).  Returns one result dict per source, the same items ``fit_source`` returns (``chain_to_host`` as there)."""
+    rank).  Returns one result dict per source, the same items ``fit_source`` returns (``chain_to_host`` and
+    ``predict_jup`` as there)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -317,6 +339,7 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
     taus = sampler.get_autocorr_time(quiet=True)
     acc = sampler.acceptance_fraction
     chain, lnp = (sampler.get_chain(), sampler.get_log_prob()) if chain_to_host else (None, None)
+    sleds = sled_results(sampler, predict_jup) if predict_jup is not None else None
     results = []
     for k, st in enumerate(setups):
         sl = slice(k * nwalkers, (k + 1) * nwalkers)
@@ -327,6 +350,8 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
         res = dict(st, theta_med=theta_med, chain=c, lnprobability=l, summary=summary, autocorr_time=taus[k],
                    acceptance_fraction=float(np.mean(acc[sl])),
                    acceptance_fraction_per_walker=acc[sl], molfile=R.molpath, molfile_synthetic=R.molfile_is_synthetic)
+        if sleds is not None:
+            res.update(sleds[k])
         if outdir is not None and sampler.rank == 0:
             os.makedirs(outdir, exist_ok=True)
             if ncomp == 1:
@@ -358,6 +383,13 @@ def print_summary(res, ncomp, file=None):
         print("xxx: %s" % key, file=out)
         for c in range(ncomp):
             print("xxx: %s" % (tuple(float(v) for v in res["summary"][c][key]),), file=out)
+    if "sled_summary" in res:
+        names = ["flux"] if ncomp == 1 else ["total flux", "component 1 flux", "component 2 flux"]
+        print("xxx: predicted SLED [Jy km/s]: (median, +err, -err)", file=out)
+        for name, plane in zip(names, res["sled_summary"]):
+            print("xxx: %s" % name, file=out)
+            for J, v in plane.items():
+                print("xxx: J=%d %s" % (J, tuple(float(x) for x in v)), file=out)
 
 
 def main(argv=None):
@@ -380,6 +412,9 @@ def main(argv=None):
                     help="keep the chain on the GPU: percentiles and autocorrelation times are computed there, the "
                          "pickles hold None for (chain, lnprobability); needed for ensembles whose chain does not fit "
                          "in host memory")
+    ap.add_argument("--predict-sled", type=int, nargs="+", default=None, metavar="J",
+                    help="also summarise the posterior-predictive flux of these lines (1-based J, at most 16), per "
+                         "component with two; computed on the GPU, so it works with --summaries-only")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -398,7 +433,7 @@ def main(argv=None):
         for res in fit_sources_concurrently(sources, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                                             n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir,
                                             datapath=args.datapath, allow_synthetic=args.allow_synthetic,
-                                            chain_to_host=not args.summaries_only):
+                                            chain_to_host=not args.summaries_only, predict_jup=args.predict_sled):
             if rank == 0:
                 print_summary(res, args.ncomp)
         if world > 1:
@@ -408,7 +443,8 @@ def main(argv=None):
         logger.info("Processing %s on GPU %d", source, device)
         res = fit_source(source, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                          n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir, datapath=args.datapath,
-                         allow_synthetic=args.allow_synthetic, chain_to_host=not args.summaries_only)
+                         allow_synthetic=args.allow_synthetic, chain_to_host=not args.summaries_only,
+                         predict_jup=args.predict_sled)
         print_summary(res, args.ncomp)
 
 

@@ -29,6 +29,8 @@ Posterior statistics where the chain lives
   ``get_quantiles`` (exact ``np.percentile`` of every source's flattened chain) and ``get_autocorr_time``
   (emcee's integrated autocorrelation time) read the stored chain in place on every rank (csrc/chain_stats.cuh):
   only 256-bin digit histograms and per-lag sums cross ranks (``all_reduce``) and PCIe, never the chain.
+  ``get_predictive_quantiles`` does the same for the model SLED of every sample (csrc/predict_sled.cuh): the predicted
+  line fluxes are solved from the chain in place and ranked where they are computed.
 
 The arithmetic is behind an ``engine`` object so that the host logic (sharding, gather order,
 bookkeeping) can be exercised on CPU by the test-suite's engine (tests/ref_engine.py); the
@@ -277,6 +279,22 @@ class CudaEngine:
         self.launches += 1
         return out
 
+    # ---- posterior-predictive SLEDs (csrc/predict_sled.cuh) ---------------------------------------------------------
+    def predict_sled(self, view, jup, counters=None):
+        """Model fluxes of the lines ``jup`` for every selected sample of ``view``: [nplanes, nsel, nlocal, nlines] on the
+        device; nplanes = 1 (one component) or 3 (total, component 1, component 2).  ``counters``: None, or a device
+        int64[2] that gains (components solved, components out of range)."""
+        self._bind_stream()
+        jj = np.ascontiguousarray(jup, dtype=np.int32)
+        nplanes = 1 if self.model.ncomp == 1 else 3
+        out = torch.empty((nplanes, view.nsel, view.nlocal, jj.size), dtype=torch.float64, device=self.device)
+        vs = view.c_struct()
+        _lib.check(self.L.rb_predict_sled_dev(self.ctx.handle, self.srcset.handle, C.byref(vs), jj.size,
+                                              jj.ctypes.data_as(_lib._ip), C.byref(self.opts), out.data_ptr(),
+                                              counters.data_ptr() if counters is not None else None))
+        self.launches += 1
+        return out
+
     def run_native(self, split, a, step0, nsteps, X, lnp, naccept, counters, thin, chain, lnp_chain):
         """nsteps steps of the whole (single-rank) ensemble inside the library."""
         self._bind_stream()
@@ -307,8 +325,9 @@ def walkers_independent(coords):
 
 class StretchSampler:
     """``EnsembleSampler``-like driver: ``run_mcmc``, ``get_chain``, ``get_log_prob``, ``reset``,
-    ``acceptance_fraction`` (per walker, like emcee), ``get_autocorr_time``, and ``get_quantiles`` (exact
-    percentiles of the stored chain without moving it)."""
+    ``acceptance_fraction`` (per walker, like emcee), ``get_autocorr_time``, ``get_quantiles`` (exact
+    percentiles of the stored chain without moving it), and the posterior-predictive SLEDs ``get_predicted_fluxes`` /
+    ``get_predictive_quantiles``."""
 
     def __init__(self, nwalkers, ndim, engine, a=2.0, seed=0, group=None, randomize_split=True, nsources=1,
                  split_block=None, native=True, time_gather=False):
@@ -540,7 +559,10 @@ class StretchSampler:
         the device), and the interpolation between them is numpy's own arithmetic (numpy/lib/_function_base_impl.py:
         _quantile, _get_indexes, _get_gamma, _lerp)."""
         view = self._chain_view(discard, thin)
-        cols = self._columns(columns)
+        return self._percentiles(view, self._columns(columns), q)
+
+    def _percentiles(self, view, cols, q):
+        """np.percentile(q) of every (source, column) of ``view``: [nsources, len(q), ncol]."""
         qq = np.true_divide(np.asarray(q, dtype=np.float64).reshape(-1), np.float64(100))
         if not (np.all(qq >= 0) and np.all(qq <= 1)):
             raise ValueError("Percentiles must be in the range [0, 100]")
@@ -565,6 +587,39 @@ class StretchSampler:
             np.subtract(b, diff * (1 - t), out=out, where=t >= 0.5)
         out[np.broadcast_to(has_nan[:, None, :], out.shape)] = np.nan
         return out
+
+    # ---- posterior-predictive SLEDs -----------------------------------------------------------------------------------
+    def _predicted(self, jup, discard, thin):
+        """This rank's model fluxes of the lines ``jup`` over the selected samples: [nplanes, nsel, nlocal, nlines]."""
+        jup = np.asarray(jup, dtype=np.int64).reshape(-1)
+        if not 1 <= jup.size <= _lib.RB_MAX_OBS:
+            raise ValueError("between 1 and %d lines per call" % _lib.RB_MAX_OBS)
+        return self.engine.predict_sled(self._chain_view(discard, thin), jup)
+
+    def get_predicted_fluxes(self, jup, discard=0, thin=1, flat=False):
+        """Model SLED of every selected sample, [nplanes, steps, nwalkers, len(jup)] in Jy km/s (flat: [nplanes,
+        steps x nwalkers, len(jup)]), gathered over ranks like ``get_chain``: what ``model_lvg(jup, sample)`` returns
+        for each row of ``get_chain(discard=discard, thin=thin)``, at the background temperature of the walker's source.
+        One component: one plane.  Two: the total, then the cold (theta[0:4]) and the warm (theta[4:8]) component.  A
+        component out of pyradex's range (where model_lvg raises ValueError) gives NaN there and in the total.  For
+        small chains and plots; ``get_predictive_quantiles`` summarises a large chain without moving it."""
+        F = self._predicted(jup, discard, thin)
+        if self.world > 1:
+            F = self._gather(F.permute(2, 0, 1, 3).contiguous()).permute(1, 2, 0, 3)
+        F = F.cpu().numpy()
+        return F.reshape(F.shape[0], -1, F.shape[3]) if flat else F
+
+    def get_predictive_quantiles(self, jup, q, discard=0, thin=1):
+        """Percentiles of the predicted line fluxes per source: [nsources, nplanes, len(q), len(jup)], every value equal
+        to ``np.percentile`` of the source's slice of ``get_predicted_fluxes(jup, discard, thin)`` flattened over steps
+        and walkers (NaN where the slice holds a NaN).  The planes are computed and ranked on each rank's device; only
+        digit histograms cross ranks and PCIe, and the planes are freed on return."""
+        F = self._predicted(jup, discard, thin)
+        cols = [(k, -1) for k in range(F.shape[3])]
+        out = [self._percentiles(ChainView([F[p]], self.nlocal, F.shape[3], self.gid_base, self.split.walkers_per_source,
+                                           0, 1), cols, q) for p in range(F.shape[0])]
+        del F
+        return np.stack(out, axis=1)
 
     def _integrated_time(self, discard, thin, c):
         """emcee's integrated_time per (source, parameter) with the device acf: (tau in thinned steps, window, n_t)."""

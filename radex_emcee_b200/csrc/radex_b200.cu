@@ -1441,10 +1441,16 @@ int upload(rb_ctx *ctx, const std::vector<T> &v, const T **out) {
   return RB_OK;
 }
 
-SolveCfg make_cfg(const rb_ctx *ctx, const rb_opts *o, double deltav_kms, double tbg, int geometry) {
+// the caller's options, or the defaults where it passes none
+rb_opts resolve_opts(const rb_opts *o) {
   rb_opts d;
   rb_default_opts(&d);
   if (o) d = *o;
+  return d;
+}
+
+SolveCfg make_cfg(const rb_ctx *ctx, const rb_opts *o, double deltav_kms, double tbg, int geometry) {
+  const rb_opts d = resolve_opts(o);
   SolveCfg c;
   c.bslab = ctx->bslab;
   c.deltav_cms = deltav_kms * 1.0e5;  // km/s -> cm/s (core.py:447-454)
@@ -1518,18 +1524,90 @@ Launch v2_launch(rb_ctx *ctx, long long n) {
   return L;
 }
 
-int ensure_scratch(rb_ctx *ctx, size_t bytes) {
-  if (bytes <= ctx->scratch_bytes) return RB_OK;
-  if (ctx->scratch) cudaFree(ctx->scratch);
-  ctx->scratch = nullptr;
-  ctx->scratch_bytes = 0;
-  const size_t want = bytes + bytes / 4;
-  CUDA_TRY(cudaMalloc(&ctx->scratch, want));
-  ctx->scratch_bytes = want;
+// An lnprob call of n walkers runs as a pipeline (expand -> scheduled solve of n x ncomp models -> combine) rather
+// than as one fused launch
+bool lnprob_pipelined(const rb_ctx *ctx, const SolveCfg &cfg, const rb_opts *opts, int nsrc, long long n, int ncomp) {
+  return nsrc == 1 && use_v2(ctx, opts) && cfg.sched && cfg.small && cfg.cache && n >= cfg.lnprob_pipe_min &&
+         n * ncomp >= RB_SCHED_MIN;
+}
+
+// Grow-only device buffer p of cap bytes: a request for more replaces it with need + headroom bytes
+int grow(void *&p, size_t &cap, size_t need, size_t headroom = 0) {
+  if (need <= cap) return RB_OK;
+  if (p) cudaFree(p);
+  p = nullptr;
+  cap = 0;
+  CUDA_TRY(cudaMalloc(&p, need + headroom));
+  cap = need + headroom;
   return RB_OK;
 }
 
-inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+int ensure_scratch(rb_ctx *ctx, size_t bytes) { return grow(ctx->scratch, ctx->scratch_bytes, bytes, bytes / 4); }
+
+// Hands out consecutive 256-byte-aligned arrays from base.  A layout is run once with a null base, which only adds up
+// its size, and then with the buffer grown to that size.
+struct Carve {
+  void *base;
+  size_t bytes = 0;
+  template <typename T>
+  T *take(long long count) {
+    T *p = base ? reinterpret_cast<T *>(static_cast<char *>(base) + bytes) : nullptr;
+    bytes += ((size_t)count * sizeof(T) + 255) & ~size_t(255);
+    return p;
+  }
+};
+
+// The model arrays of an expand -> solve -> combine call of m models, from ctx->ln_buf; the brightness holds `stride`
+// lines per model
+int model_arrays(rb_ctx *ctx, long long m, int stride, LnprobPipe *pp) {
+  auto layout = [&](Carve c) {
+    pp->tkin = c.take<double>(m);
+    pp->cdmol = c.take<double>(m);
+    pp->dens = c.take<double>(m * ctx->mol.npart);
+    pp->obs_surf = c.take<double>(m * stride);
+    pp->status = c.take<int>(m);
+    return c.bytes;
+  };
+  const int rc = grow(ctx->ln_buf, ctx->ln_bytes, layout(Carve{nullptr}));
+  if (rc != RB_OK) return rc;
+  layout(Carve{ctx->ln_buf});
+  return RB_OK;
+}
+
+// observed-line mode: only the brightness of lines jup[k] - 1 is written, at obs_surf[model][k]
+void observe_lines(SolveIO &io, double *obs_surf, int nobs, const int32_t *jup) {
+  io.obs_surf = obs_surf;
+  io.nobs = nobs;
+  for (int k = 0; k < nobs; ++k) io.obs_line[k] = jup[k] - 1;
+}
+
+// models [o, o + m) of io
+SolveIO slice(const rb_ctx *ctx, const SolveIO &io, long long o, long long m) {
+  const int np = ctx->mol.npart, nl = ctx->mol.nlev, nn = ctx->mol.nline;
+  SolveIO part = io;
+  part.n = m;
+  part.tkin += o;
+  part.dens += o * np;
+  part.cdmol += o;
+  if (part.xpop) part.xpop += o * nl;
+  if (part.tex) part.tex += o * nn;
+  if (part.tau) part.tau += o * nn;
+  if (part.surf) part.surf += o * nn;
+  if (part.niter) part.niter += o;
+  if (part.status) part.status += o;
+  if (part.obs_surf) part.obs_surf += o * RB_MAX_OBS;
+  return part;
+}
+
+// After the work queued on ctx->stream: the iteration total of the last call (kept in the ctx) and its solves
+int read_counters(rb_ctx *ctx, int64_t *nsolves = nullptr) {
+  unsigned long long cnt[3] = {0, 0, 0};
+  CUDA_TRY(cudaMemcpyAsync(cnt, ctx->counters, sizeof(cnt), cudaMemcpyDeviceToHost, ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  ctx->last_total_iters = (long long)cnt[1];
+  if (nsolves) *nsolves = (int64_t)cnt[2];
+  return RB_OK;
+}
 
 }  // namespace
 
@@ -1685,15 +1763,9 @@ void rb_ctx_destroy(rb_ctx *ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
   for (void *p : ctx->owned) cudaFree(p);
-  if (ctx->scratch) cudaFree(ctx->scratch);
-  if (ctx->counters) cudaFree(ctx->counters);
-  if (ctx->bslab) cudaFree(ctx->bslab);
-  if (ctx->sched_buf) cudaFree(ctx->sched_buf);
-  if (ctx->sched_small) cudaFree(ctx->sched_small);
-  if (ctx->ln_buf) cudaFree(ctx->ln_buf);
-  if (ctx->src_one) cudaFree(ctx->src_one);
-  if (ctx->samp_buf) cudaFree(ctx->samp_buf);
-  if (ctx->cs_buf) cudaFree(ctx->cs_buf);
+  for (void *p : {ctx->scratch, ctx->sched_buf, ctx->ln_buf, ctx->samp_buf, ctx->cs_buf, (void *)ctx->counters,
+                  (void *)ctx->bslab, (void *)ctx->sched_small, (void *)ctx->src_one})
+    if (p) cudaFree(p);
   if (ctx->samp_graph) cudaGraphExecDestroy(ctx->samp_graph);
   if (ctx->ev_samp) cudaEventDestroy(ctx->ev_samp);
   for (cudaEvent_t ev : ctx->chunk_done) cudaEventDestroy(ev);
@@ -1732,56 +1804,38 @@ int rb_ctx_reset_stream(rb_ctx *ctx) {
                                  // launches, 2^17 2 % faster, 2^20 6 % faster)
 #define RB_PIPE_MAX (1LL << 20)   // models per scheduled pass: bounds the parked state + captures at 1 + 7 GB
 
-static int launch_solve_pipeline(rb_ctx *ctx, const SolveCfg &cfg_in, SolveIO io, const Launch &L) {
+static int launch_solve_pipeline(rb_ctx *ctx, const SolveCfg &cfg_in, SolveIO io) {
   if (io.n > RB_PIPE_MAX && cfg_in.small) {   // larger batches: one pass per 2^20 models, totals keep accumulating
-    const int np = ctx->mol.npart, nl = ctx->mol.nlev, nn = ctx->mol.nline;
     for (long long o = 0; o < io.n; o += RB_PIPE_MAX) {
-      SolveIO part = io;
-      part.n = std::min<long long>(RB_PIPE_MAX, io.n - o);
-      part.tkin += o;
-      part.dens += o * np;
-      part.cdmol += o;
-      if (part.xpop) part.xpop += o * nl;
-      if (part.tex) part.tex += o * nn;
-      if (part.tau) part.tau += o * nn;
-      if (part.surf) part.surf += o * nn;
-      if (part.niter) part.niter += o;
-      if (part.status) part.status += o;
-      if (part.obs_surf) part.obs_surf += o * RB_MAX_OBS;
       if (o > 0) CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, sizeof(unsigned long long), ctx->stream));   // queue head
-      const int rc = launch_solve_pipeline(ctx, cfg_in, part, v2_launch(ctx, part.n));
+      const int rc = launch_solve_pipeline(ctx, cfg_in, slice(ctx, io, o, std::min<long long>(RB_PIPE_MAX, io.n - o)));
       if (rc != RB_OK) return rc;
     }
     return RB_OK;
   }
   const long long n = io.n;
+  const Launch L = v2_launch(ctx, n);
   SolveCfg cfg = cfg_in;
   if (cfg.park_max == 0) cfg.park_max = (n >= RB_MID_MIN) ? v2::KP_SMALL_MAX : 4;
   const bool small = cfg.small != 0;   // the parked captures take 4.9 .. 10.5 KB per cacheable model, EXT_AVG x 8 B budgeted
-  const size_t b_state = align256((size_t)n * v2::STATE_STRIDE * sizeof(double)), b_int = align256((size_t)n * sizeof(int));
-  const long long ext_cap = (long long)n * v2::EXT_AVG;
-  const size_t b_off = small ? align256((size_t)n * sizeof(long long)) : 0;
-  const size_t b_ext = small ? align256((size_t)ext_cap * sizeof(double)) : 0;
-  const size_t b_all = b_state + (small ? 3 : 2) * b_int + b_off + b_ext;
-  if (b_all > ctx->sched_bytes) {
-    if (ctx->sched_buf) cudaFree(ctx->sched_buf);
-    ctx->sched_buf = nullptr;
-    ctx->sched_bytes = 0;
-    CUDA_TRY(cudaMalloc(&ctx->sched_buf, b_all));
-    ctx->sched_bytes = b_all;
-  }
+  int *order = nullptr;
+  auto layout = [&](Carve c) {
+    io.state = c.take<double>(n * v2::STATE_STRIDE);
+    io.keys = c.take<int>(n);
+    order = c.take<int>(n);
+    if (small) {
+      io.order_c = c.take<int>(n);
+      io.ext_off = c.take<long long>(n);
+      io.ext_cap = n * v2::EXT_AVG;
+      io.ext = c.take<double>(io.ext_cap);
+    }
+    return c.bytes;
+  };
+  int rc = grow(ctx->sched_buf, ctx->sched_bytes, layout(Carve{nullptr}));
+  if (rc != RB_OK) return rc;
+  layout(Carve{ctx->sched_buf});
   if (!ctx->sched_small) CUDA_TRY(cudaMalloc(&ctx->sched_small, 96 * sizeof(unsigned long long)));
-  char *base = static_cast<char *>(ctx->sched_buf);
-  io.state = reinterpret_cast<double *>(base);
-  io.keys = reinterpret_cast<int *>(base + b_state);
-  int *order = reinterpret_cast<int *>(base + b_state + b_int);
   io.sched_small = ctx->sched_small;
-  if (small) {
-    io.order_c = reinterpret_cast<int *>(base + b_state + 2 * b_int);
-    io.ext_off = reinterpret_cast<long long *>(base + b_state + 3 * b_int);
-    io.ext = reinterpret_cast<double *>(base + b_state + 3 * b_int + b_off);
-    io.ext_cap = ext_cap;
-  }
   CUDA_TRY(cudaMemsetAsync(ctx->sched_small, 0, 96 * sizeof(unsigned long long), ctx->stream));
   io.sched = 1;
   k_lvg_solve_v2<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, io);
@@ -1840,35 +1894,38 @@ static int launch_solve_pipeline(rb_ctx *ctx, const SolveCfg &cfg_in, SolveIO io
   return RB_OK;
 }
 
-// keep_totals: a further chunk of one host call -- only the work-queue head is reset, the iteration total and the
-// cache statistics keep accumulating
-static int solve_batch_dev_impl(rb_ctx *ctx, int64_t n, const double *tkin, const double *dens, const double *cdmol,
-                                double deltav_kms, double tbg, int geometry, const rb_opts *opts, double *xpop,
-                                double *tex, double *tau, double *surf, int32_t *niter, int32_t *status,
-                                bool keep_totals) {
-  int rc = check_common(ctx, deltav_kms, tbg, geometry);
+// The solve of io.n models: k_lvg_solve_v1, one k_lvg_solve_v2 launch, or the scheduled pipeline
+static int launch_solve(rb_ctx *ctx, const SolveCfg &cfg, const rb_opts *opts, const SolveIO &io) {
+  if (!use_v2(ctx, opts)) {
+    const Launch L = v1_launch(ctx, io.n);
+    k_lvg_solve_v1<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, io);
+  } else if (cfg.sched && cfg.cache && cfg.method == RB_GEOM_LVG && io.n >= RB_SCHED_MIN) {
+    return launch_solve_pipeline(ctx, cfg, io);
+  } else {
+    const Launch L = v2_launch(ctx, io.n);
+    k_lvg_solve_v2<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, io);
+  }
+  return RB_OK;
+}
+
+static int check_solve(rb_ctx *ctx, int64_t n, const double *tkin, const double *dens, const double *cdmol,
+                       double deltav_kms, double tbg, int geometry) {
+  const int rc = check_common(ctx, deltav_kms, tbg, geometry);
   if (rc != RB_OK) return rc;
   if (n < 0 || (n > 0 && (!tkin || !dens || !cdmol))) {
     rb_set_error("rb_solve_batch: null input");
     return RB_ERR_ARG;
   }
-  if (n == 0) return RB_OK;
-  CUDA_TRY(cudaSetDevice(ctx->device));
-  const SolveCfg cfg = make_cfg(ctx, opts, deltav_kms, tbg, geometry);
+  return RB_OK;
+}
+
+// keep_totals: a further chunk of one host call -- only the work-queue head is reset, the iteration total and the
+// cache statistics keep accumulating
+static int solve_batch_dev_impl(rb_ctx *ctx, const SolveCfg &cfg, const rb_opts *opts, const SolveIO &io,
+                                bool keep_totals) {
   CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, (keep_totals ? 1 : 8) * sizeof(unsigned long long), ctx->stream));
-  SolveIO io{n, tkin, dens, cdmol, xpop, tex, tau, surf, niter, status, ctx->counters, 0, nullptr, nullptr, nullptr, nullptr};
-  if (use_v2(ctx, opts)) {
-    const Launch L = v2_launch(ctx, n);
-    if (cfg.sched && cfg.cache && geometry == RB_GEOM_LVG && n >= RB_SCHED_MIN) {
-      rc = launch_solve_pipeline(ctx, cfg, io, L);
-      if (rc != RB_OK) return rc;
-    } else {
-      k_lvg_solve_v2<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, io);
-    }
-  } else {
-    const Launch L = v1_launch(ctx, n);
-    k_lvg_solve_v1<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, io);
-  }
+  const int rc = launch_solve(ctx, cfg, opts, io);
+  if (rc != RB_OK) return rc;
   CUDA_TRY(cudaGetLastError());
   ctx->launches += 1;
   return RB_OK;
@@ -1877,8 +1934,11 @@ static int solve_batch_dev_impl(rb_ctx *ctx, int64_t n, const double *tkin, cons
 int rb_solve_batch_dev(rb_ctx *ctx, int64_t n, const double *tkin, const double *dens, const double *cdmol,
                        double deltav_kms, double tbg, int geometry, const rb_opts *opts, double *xpop,
                        double *tex, double *tau, double *surf, int32_t *niter, int32_t *status) {
-  return solve_batch_dev_impl(ctx, n, tkin, dens, cdmol, deltav_kms, tbg, geometry, opts, xpop, tex, tau, surf, niter,
-                              status, false);
+  const int rc = check_solve(ctx, n, tkin, dens, cdmol, deltav_kms, tbg, geometry);
+  if (rc != RB_OK || n == 0) return rc;
+  CUDA_TRY(cudaSetDevice(ctx->device));
+  const SolveIO io{n, tkin, dens, cdmol, xpop, tex, tau, surf, niter, status, ctx->counters};
+  return solve_batch_dev_impl(ctx, make_cfg(ctx, opts, deltav_kms, tbg, geometry), opts, io, false);
 }
 
 // Host-pointer entry.  Batches of more than 2 RB_HOST_CHUNK models are solved chunk by chunk, the results of one
@@ -1895,33 +1955,27 @@ int rb_solve_batch_dev(rb_ctx *ctx, int64_t n, const double *tkin, const double 
 int rb_solve_batch(rb_ctx *ctx, int64_t n, const double *tkin, const double *dens, const double *cdmol,
                    double deltav_kms, double tbg, int geometry, const rb_opts *opts, double *xpop, double *tex,
                    double *tau, double *surf, int32_t *niter, int32_t *status) {
-  int rc = check_common(ctx, deltav_kms, tbg, geometry);
-  if (rc != RB_OK) return rc;
-  if (n < 0 || (n > 0 && (!tkin || !dens || !cdmol))) {
-    rb_set_error("rb_solve_batch: null input");
-    return RB_ERR_ARG;
-  }
-  if (n == 0) return RB_OK;
+  int rc = check_solve(ctx, n, tkin, dens, cdmol, deltav_kms, tbg, geometry);
+  if (rc != RB_OK || n == 0) return rc;
   CUDA_TRY(cudaSetDevice(ctx->device));
   const int nl = ctx->mol.nlev, nn = ctx->mol.nline, np = ctx->mol.npart;
-  const size_t b_t = align256(n * sizeof(double)), b_d = align256((size_t)n * np * sizeof(double));
-  const size_t b_x = xpop ? align256((size_t)n * nl * sizeof(double)) : 0;
-  const size_t b_l = align256((size_t)n * nn * sizeof(double));
-  const size_t b_i = align256(n * sizeof(int32_t));
-  const size_t total = 2 * b_t + b_d + b_x + (tex ? b_l : 0) + (tau ? b_l : 0) + (surf ? b_l : 0) + 2 * b_i;
-  rc = ensure_scratch(ctx, total);
+  double *d_t, *d_c, *d_d, *d_x, *d_tex, *d_tau, *d_s;
+  int32_t *d_it, *d_st;
+  auto layout = [&](Carve c) {
+    d_t = c.take<double>(n);
+    d_c = c.take<double>(n);
+    d_d = c.take<double>(n * np);
+    d_x = xpop ? c.take<double>(n * nl) : nullptr;
+    d_tex = tex ? c.take<double>(n * nn) : nullptr;
+    d_tau = tau ? c.take<double>(n * nn) : nullptr;
+    d_s = surf ? c.take<double>(n * nn) : nullptr;
+    d_it = c.take<int32_t>(n);
+    d_st = c.take<int32_t>(n);
+    return c.bytes;
+  };
+  rc = ensure_scratch(ctx, layout(Carve{nullptr}));
   if (rc != RB_OK) return rc;
-  char *p = static_cast<char *>(ctx->scratch);
-  double *d_t = (double *)p; p += b_t;
-  double *d_c = (double *)p; p += b_t;
-  double *d_d = (double *)p; p += b_d;
-  double *d_x = nullptr, *d_tex = nullptr, *d_tau = nullptr, *d_s = nullptr;
-  if (xpop) { d_x = (double *)p; p += b_x; }
-  if (tex) { d_tex = (double *)p; p += b_l; }
-  if (tau) { d_tau = (double *)p; p += b_l; }
-  if (surf) { d_s = (double *)p; p += b_l; }
-  int32_t *d_it = (int32_t *)p; p += b_i;
-  int32_t *d_st = (int32_t *)p; p += b_i;
+  layout(Carve{ctx->scratch});
   cudaStream_t s = ctx->stream;
   CUDA_TRY(cudaMemcpyAsync(d_t, tkin, n * sizeof(double), cudaMemcpyHostToDevice, s));
   CUDA_TRY(cudaMemcpyAsync(d_c, cdmol, n * sizeof(double), cudaMemcpyHostToDevice, s));
@@ -1949,14 +2003,10 @@ int rb_solve_batch(rb_ctx *ctx, int64_t n, const double *tkin, const double *den
     CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
     ctx->chunk_done.push_back(ev);
   }
-  auto solve_chunk = [&](int64_t k) -> int {
-    const int64_t o = c_off[k], m = c_len[k];
-    if (nchunk == 1)
-      return solve_batch_dev_impl(ctx, n, d_t, d_d, d_c, deltav_kms, tbg, geometry, opts, d_x, d_tex, d_tau, d_s, d_it,
-                                  d_st, false);
-    return solve_batch_dev_impl(ctx, m, d_t + o, d_d + o * np, d_c + o, deltav_kms, tbg, geometry, opts,
-                                d_x ? d_x + o * nl : nullptr, d_tex ? d_tex + o * nn : nullptr,
-                                d_tau ? d_tau + o * nn : nullptr, d_s ? d_s + o * nn : nullptr, d_it + o, d_st + o, k > 0);
+  const SolveCfg cfg = make_cfg(ctx, opts, deltav_kms, tbg, geometry);
+  const SolveIO io{n, d_t, d_d, d_c, d_x, d_tex, d_tau, d_s, d_it, d_st, ctx->counters};
+  auto solve_chunk = [&](int64_t k) {
+    return solve_batch_dev_impl(ctx, cfg, opts, slice(ctx, io, c_off[k], c_len[k]), k > 0);
   };
   rc = solve_chunk(0);
   if (rc != RB_OK) return rc;
@@ -1981,11 +2031,7 @@ int rb_solve_batch(rb_ctx *ctx, int64_t n, const double *tkin, const double *den
     if (status) CUDA_TRY(cudaMemcpyAsync(status + o, d_st + o, m * sizeof(int32_t), cudaMemcpyDeviceToHost, cs));
   }
   if (nchunk > 1) CUDA_TRY(cudaStreamSynchronize(ctx->copy_stream));
-  unsigned long long cnt[3] = {0, 0, 0};
-  CUDA_TRY(cudaMemcpyAsync(cnt, ctx->counters, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  ctx->last_total_iters = (long long)cnt[1];
-  return RB_OK;
+  return read_counters(ctx);
 }
 
 struct rb_srcset {
@@ -2013,9 +2059,7 @@ static int check_source(const rb_ctx *ctx, const rb_source &S) {
   return RB_OK;
 }
 
-// lnprob of n walkers against the device table d_srcs (row src_id[i], or row 0); h0 = host copy of row 0.
-static int lnprob_core(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const rb_source *d_srcs, int nsrc,
-                       const rb_source &h0, const int *src_id, const rb_opts *opts, double *lnp) {
+static int check_lnprob(const rb_ctx *ctx, int64_t n, const double *P, const double *lnp) {
   if (!ctx) {
     rb_set_error("null context");
     return RB_ERR_ARG;
@@ -2024,6 +2068,14 @@ static int lnprob_core(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const
     rb_set_error("rb_lnprob: null argument");
     return RB_ERR_ARG;
   }
+  return RB_OK;
+}
+
+// lnprob of n walkers against the device table d_srcs (row src_id[i], or row 0); h0 = host copy of row 0.
+static int lnprob_core(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const rb_source *d_srcs, int nsrc,
+                       const rb_source &h0, const int *src_id, const rb_opts *opts, double *lnp) {
+  int rc = check_lnprob(ctx, n, P, lnp);
+  if (rc != RB_OK) return rc;
   if (!ctx->ln_partners_ok) {
     // the drivers set {'oH2', 'pH2'} (emcee_radex.py:122-124), which pyradex folds into H2 when the file has that
     // partner (core.py:551-556); a file with neither has all-zero colliders there (ValueError)
@@ -2042,39 +2094,20 @@ static int lnprob_core(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const
   io.srcs = d_srcs;
   io.src_id = (nsrc > 1) ? src_id : nullptr;
   io.counters = ctx->counters;
-  if (nsrc == 1 && use_v2(ctx, opts) && cfg.sched && cfg.small && cfg.cache && n >= cfg.lnprob_pipe_min &&
-      n * ncomp >= RB_SCHED_MIN) {
+  if (lnprob_pipelined(ctx, cfg, opts, nsrc, n, ncomp)) {
     // large ensembles: expand -> scheduled solve of all n x ncomp models (half-warp engine) -> combine
     const long long m = n * ncomp;
-    const int np = ctx->mol.npart;
-    const size_t b_d = align256((size_t)m * sizeof(double)), b_dn = align256((size_t)m * np * sizeof(double));
-    const size_t b_o = align256((size_t)m * RB_MAX_OBS * sizeof(double)), b_s = align256((size_t)m * sizeof(int));
-    const size_t b_all = 2 * b_d + b_dn + b_o + b_s;
-    if (b_all > ctx->ln_bytes) {
-      if (ctx->ln_buf) cudaFree(ctx->ln_buf);
-      ctx->ln_buf = nullptr;
-      ctx->ln_bytes = 0;
-      CUDA_TRY(cudaMalloc(&ctx->ln_buf, b_all));
-      ctx->ln_bytes = b_all;
-    }
-    char *base = static_cast<char *>(ctx->ln_buf);
     LnprobPipe pp;
-    pp.tkin = reinterpret_cast<double *>(base);
-    pp.cdmol = reinterpret_cast<double *>(base + b_d);
-    pp.dens = reinterpret_cast<double *>(base + 2 * b_d);
-    pp.obs_surf = reinterpret_cast<double *>(base + 2 * b_d + b_dn);
-    pp.status = reinterpret_cast<int *>(base + 2 * b_d + b_dn + b_o);
+    rc = model_arrays(ctx, m, RB_MAX_OBS, &pp);
+    if (rc != RB_OK) return rc;
     const int tpb = 256;
-    SolveIO sio{m, pp.tkin, pp.dens, pp.cdmol, nullptr, nullptr, nullptr, nullptr, nullptr, pp.status, ctx->counters,
-                0, nullptr, nullptr, nullptr, nullptr};
-    sio.obs_surf = pp.obs_surf;
-    sio.nobs = h0.obs.nobs;
-    for (int i = 0; i < h0.obs.nobs; ++i) sio.obs_line[i] = h0.obs.jup[i] - 1;
+    SolveIO sio{m, pp.tkin, pp.dens, pp.cdmol, nullptr, nullptr, nullptr, nullptr, nullptr, pp.status, ctx->counters};
+    observe_lines(sio, pp.obs_surf, h0.obs.nobs, h0.obs.jup);
     if (ncomp == 1)
       k_lnprob_expand<1><<<(unsigned)((n + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(ctx->mol, io, pp);
     else
       k_lnprob_expand<2><<<(unsigned)((n + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(ctx->mol, io, pp);
-    int rc = launch_solve_pipeline(ctx, cfg, sio, v2_launch(ctx, m));
+    rc = launch_solve(ctx, cfg, opts, sio);
     if (rc != RB_OK) return rc;
     const unsigned nbc = (unsigned)((n * 32 + tpb - 1) / tpb);
     if (ncomp == 1)
@@ -2132,35 +2165,27 @@ static int lnprob_dev(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const 
 
 static int lnprob_host(rb_ctx *ctx, int ncomp, int64_t n, const double *P, const rb_obs *obs, const double *bounds,
                        int has_td, double t_d, double tbg, const rb_opts *opts, double *lnp, int64_t *nsolves) {
-  if (!ctx) {
-    rb_set_error("null context");
-    return RB_ERR_ARG;
-  }
-  if (n < 0 || (n > 0 && (!P || !lnp))) {
-    rb_set_error("rb_lnprob: null argument");
-    return RB_ERR_ARG;
-  }
+  int rc = check_lnprob(ctx, n, P, lnp);
+  if (rc != RB_OK) return rc;
   if (n == 0) {
     if (nsolves) *nsolves = 0;
     return RB_OK;
   }
   CUDA_TRY(cudaSetDevice(ctx->device));
-  const size_t b_p = align256((size_t)n * 4 * ncomp * sizeof(double)), b_l = align256(n * sizeof(double));
-  int rc = ensure_scratch(ctx, b_p + b_l);
+  double *d_p, *d_l;
+  auto layout = [&](Carve c) {
+    d_p = c.take<double>(n * 4 * ncomp);
+    d_l = c.take<double>(n);
+    return c.bytes;
+  };
+  rc = ensure_scratch(ctx, layout(Carve{nullptr}));
   if (rc != RB_OK) return rc;
-  double *d_p = (double *)ctx->scratch;
-  double *d_l = (double *)((char *)ctx->scratch + b_p);
-  cudaStream_t s = ctx->stream;
-  CUDA_TRY(cudaMemcpyAsync(d_p, P, (size_t)n * 4 * ncomp * sizeof(double), cudaMemcpyHostToDevice, s));
+  layout(Carve{ctx->scratch});
+  CUDA_TRY(cudaMemcpyAsync(d_p, P, (size_t)n * 4 * ncomp * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
   rc = lnprob_dev(ctx, ncomp, n, d_p, obs, bounds, has_td, t_d, tbg, opts, d_l);
   if (rc != RB_OK) return rc;
-  CUDA_TRY(cudaMemcpyAsync(lnp, d_l, n * sizeof(double), cudaMemcpyDeviceToHost, s));
-  unsigned long long cnt[3] = {0, 0, 0};
-  CUDA_TRY(cudaMemcpyAsync(cnt, ctx->counters, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  ctx->last_total_iters = (long long)cnt[1];
-  if (nsolves) *nsolves = (int64_t)cnt[2];
-  return RB_OK;
+  CUDA_TRY(cudaMemcpyAsync(lnp, d_l, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+  return read_counters(ctx, nsolves);
 }
 
 int rb_lnprob1(rb_ctx *ctx, int64_t n, const double *P, const rb_obs *obs, const double *bounds, double tbg,
@@ -2301,66 +2326,56 @@ static int make_split(const rb_split *sp, int64_t gid_base, int64_t nlocal, int3
   return RB_OK;
 }
 
-int rb_stretch_pack_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
-                        int64_t nlocal, int32_t ndim, const double *X, double *Chalf) {
-  st2::SplitDev sp;
-  if (!ctx || !X || !Chalf || (half != 0 && half != 1)) {
-    rb_set_error("rb_stretch_pack_dev: bad argument");
+// The three entry points below: argument checks (args_ok: the entry point's own arguments), the split, the device, then
+// launch(sp, nhalf, blocks) with blocks of 128 threads over the nhalf walkers of the half
+extern "C++" {   // a template
+template <typename F>
+static int stretch2_launch(const char *who, bool args_ok, rb_ctx *ctx, const rb_split *split, int32_t half,
+                           int64_t gid_base, int64_t nlocal, int32_t ndim, F launch) {
+  if (!ctx || !args_ok || (half != 0 && half != 1)) {
+    rb_set_error(std::string(who) + ": bad argument");
     return RB_ERR_ARG;
   }
-  int rc = make_split(split, gid_base, nlocal, ndim, &sp);
+  st2::SplitDev sp;
+  const int rc = make_split(split, gid_base, nlocal, ndim, &sp);
   if (rc != RB_OK) return rc;
   const long long nhalf = nlocal / 2;
   if (nhalf == 0) return RB_OK;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  const int tpb = 128;
-  st2::k_pack<<<(unsigned)((nhalf + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, Chalf);
+  launch(sp, nhalf, (unsigned)((nhalf + 127) / 128));
   CUDA_TRY(cudaGetLastError());
   ctx->launches += 1;
   return RB_OK;
+}
+}
+
+int rb_stretch_pack_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
+                        int64_t nlocal, int32_t ndim, const double *X, double *Chalf) {
+  return stretch2_launch("rb_stretch_pack_dev", X && Chalf, ctx, split, half, gid_base, nlocal, ndim,
+                         [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
+    st2::k_pack<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, Chalf);
+  });
 }
 
 int rb_stretch_propose2_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
                             int64_t nlocal, int32_t ndim, const double *X, const double *Call, double a, double *Q,
                             double *logfac, int32_t *src_id) {
-  st2::SplitDev sp;
-  if (!ctx || !X || !Call || !Q || !logfac || !(a > 1.0) || (half != 0 && half != 1)) {
-    rb_set_error("rb_stretch_propose2_dev: bad argument");
-    return RB_ERR_ARG;
-  }
-  int rc = make_split(split, gid_base, nlocal, ndim, &sp);
-  if (rc != RB_OK) return rc;
-  const long long nhalf = nlocal / 2;
-  if (nhalf == 0) return RB_OK;
-  CUDA_TRY(cudaSetDevice(ctx->device));
-  const int tpb = 128;
-  st2::k_propose2<<<(unsigned)((nhalf + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X,
-                                                                                 Call, a, split->seed, Q, logfac, src_id);
-  CUDA_TRY(cudaGetLastError());
-  ctx->launches += 1;
-  return RB_OK;
+  return stretch2_launch("rb_stretch_propose2_dev", X && Call && Q && logfac && a > 1.0, ctx, split, half, gid_base,
+                         nlocal, ndim, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
+    st2::k_propose2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, Call, a, split->seed,
+                                                 Q, logfac, src_id);
+  });
 }
 
 int rb_stretch_accept2_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
                            int64_t nlocal, int32_t ndim, double *X, double *lnp, const double *Q, const double *lnp_new,
                            const double *logfac, int64_t *naccept, int64_t *nan_count) {
-  st2::SplitDev sp;
-  if (!ctx || !X || !lnp || !Q || !lnp_new || !logfac || (half != 0 && half != 1)) {
-    rb_set_error("rb_stretch_accept2_dev: bad argument");
-    return RB_ERR_ARG;
-  }
-  int rc = make_split(split, gid_base, nlocal, ndim, &sp);
-  if (rc != RB_OK) return rc;
-  const long long nhalf = nlocal / 2;
-  if (nhalf == 0) return RB_OK;
-  CUDA_TRY(cudaSetDevice(ctx->device));
-  const int tpb = 128;
-  st2::k_accept2<<<(unsigned)((nhalf + tpb - 1) / tpb), tpb, 0, ctx->stream>>>(
-      sp, nullptr, step, half, gid_base, nhalf, ndim, X, lnp, Q, lnp_new, logfac, split->seed,
-      reinterpret_cast<long long *>(naccept), reinterpret_cast<unsigned long long *>(nan_count), nullptr, nullptr);
-  CUDA_TRY(cudaGetLastError());
-  ctx->launches += 1;
-  return RB_OK;
+  return stretch2_launch("rb_stretch_accept2_dev", X && lnp && Q && lnp_new && logfac, ctx, split, half, gid_base,
+                         nlocal, ndim, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
+    st2::k_accept2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, lnp, Q, lnp_new, logfac,
+                                                split->seed, reinterpret_cast<long long *>(naccept),
+                                                reinterpret_cast<unsigned long long *>(nan_count), nullptr, nullptr);
+  });
 }
 
 // One stretch-move step (both half-steps) on ctx->stream; the step index is *d_step + 0 (device-resident, so that the
@@ -2469,47 +2484,44 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
   if (nsteps == 0) return RB_OK;
   CUDA_TRY(cudaSetDevice(ctx->device));
   const long long nhalf = N / 2;
-  const size_t b_c = align256((size_t)nhalf * ndim * sizeof(double)), b_v = align256((size_t)nhalf * sizeof(double));
-  const size_t b_i = align256((size_t)nhalf * sizeof(int));
   // speculative second half-step while the three candidates of every slot can run side by side (one warp each; measured
   // on B200, walker-steps/s with / without: 100 walkers 2.57e5 / 1.35e5, 800: 1.28e6 / 9.4e5, 1600: 1.74e6 / 1.51e6,
   // 3200: 2.22e6 / 2.38e6; two components, 800 walkers: 3.97e5 / 2.54e5), unless rb_opts.spec_half says otherwise
-  rb_opts od;
-  rb_default_opts(&od);
-  if (opts) od = *opts;
+  const rb_opts od = resolve_opts(opts);
   const bool spec_fits = od.spec_half > 0 || (od.spec_half == 0 && 3 * nhalf <= (long long)RB_SPEC_WARPS_PER_SM * ctx->sm_count);
-  const size_t b_spec = spec_fits ? (5 * b_c + 6 * b_v + 5 * b_i) : 0;
-  const size_t b_all = 2 * b_c + 2 * b_v + b_i + 256 + b_spec;
-  if (b_all > ctx->samp_bytes) {
-    if (ctx->samp_graph) {
-      cudaGraphExecDestroy(ctx->samp_graph);
-      ctx->samp_graph = nullptr;
-    }
-    if (ctx->samp_buf) cudaFree(ctx->samp_buf);
-    ctx->samp_buf = nullptr;
-    ctx->samp_bytes = 0;
-    CUDA_TRY(cudaMalloc(&ctx->samp_buf, b_all));
-    ctx->samp_bytes = b_all;
-  }
-  char *base = static_cast<char *>(ctx->samp_buf);
-  double *Cbuf = reinterpret_cast<double *>(base), *Q = reinterpret_cast<double *>(base + b_c);
-  double *logfac = reinterpret_cast<double *>(base + 2 * b_c), *lnp_new = reinterpret_cast<double *>(base + 2 * b_c + b_v);
-  int *src_id = reinterpret_cast<int *>(base + 2 * b_c + 2 * b_v);
-  unsigned long long *d_step = reinterpret_cast<unsigned long long *>(base + 2 * b_c + 2 * b_v + b_i);
+  double *Cbuf, *Q, *logfac, *lnp_new;
+  int *src_id;
+  unsigned long long *d_step;
   SpecBufs sb{};
-  if (spec_fits) {
-    char *q = base + 2 * b_c + 2 * b_v + b_i + 256;
-    sb.C1 = reinterpret_cast<double *>(q); q += b_c;
-    sb.Cold = reinterpret_cast<double *>(q); q += b_c;
-    sb.Q3 = reinterpret_cast<double *>(q); q += 3 * b_c;   // three blocks of nhalf x ndim, contiguous: b_c is padded, so
-    sb.L3 = reinterpret_cast<double *>(q); q += 3 * b_v;   // the blocks are addressed by nhalf * ndim, not by b_c
-    sb.logfac0 = reinterpret_cast<double *>(q); q += b_v;
-    sb.logfac1 = reinterpret_cast<double *>(q); q += b_v;
-    sb.Lsel = reinterpret_cast<double *>(q); q += b_v;
-    sb.jpart = reinterpret_cast<int *>(q); q += b_i;
-    sb.acc0 = reinterpret_cast<int *>(q); q += b_i;
-    sb.src3 = reinterpret_cast<int *>(q); q += 3 * b_i;   // addressed by nhalf (b_i is padded)
+  auto layout = [&](Carve c) {
+    Cbuf = c.take<double>(nhalf * ndim);
+    Q = c.take<double>(nhalf * ndim);
+    logfac = c.take<double>(nhalf);
+    lnp_new = c.take<double>(nhalf);
+    src_id = c.take<int>(nhalf);
+    d_step = c.take<unsigned long long>(1);
+    if (spec_fits) {
+      sb.C1 = c.take<double>(nhalf * ndim);
+      sb.Cold = c.take<double>(nhalf * ndim);
+      sb.Q3 = c.take<double>(3 * nhalf * ndim);
+      sb.L3 = c.take<double>(3 * nhalf);
+      sb.logfac0 = c.take<double>(nhalf);
+      sb.logfac1 = c.take<double>(nhalf);
+      sb.Lsel = c.take<double>(nhalf);
+      sb.jpart = c.take<int>(nhalf);
+      sb.acc0 = c.take<int>(nhalf);
+      sb.src3 = c.take<int>(3 * nhalf);
+    }
+    return c.bytes;
+  };
+  const size_t need = layout(Carve{nullptr});
+  if (need > ctx->samp_bytes && ctx->samp_graph) {   // the captured step holds pointers into the old buffer
+    cudaGraphExecDestroy(ctx->samp_graph);
+    ctx->samp_graph = nullptr;
   }
+  rc = grow(ctx->samp_buf, ctx->samp_bytes, need);
+  if (rc != RB_OK) return rc;
+  layout(Carve{ctx->samp_buf});
   cudaStream_t s = ctx->stream;
   const unsigned long long step0_ = step0;
   CUDA_TRY(cudaMemcpyAsync(d_step, &step0_, sizeof(step0_), cudaMemcpyHostToDevice, s));
@@ -2534,12 +2546,9 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
   // A half-ensemble that fits one fused lnprob launch is latency-bound (config 1: 50 models per half-step): its step is
   // captured once and replayed.  The key holds every argument the captured launches depend on.
   const SolveCfg cfg = make_cfg(ctx, opts, 1.0, set->h[0].tbg, RB_GEOM_LVG);
-  const bool fused = !(set->nsrc == 1 && use_v2(ctx, opts) && cfg.sched && cfg.small && cfg.cache &&
-                       nhalf >= cfg.lnprob_pipe_min && nhalf * set->ncomp >= RB_SCHED_MIN);
+  const bool fused = !lnprob_pipelined(ctx, cfg, opts, set->nsrc, nhalf, set->ncomp);
   // (forced speculation on a large ensemble: the 1.5 N candidates must still be one fused launch, not the pipeline)
-  spec = fused && spec_fits &&
-         !(set->nsrc == 1 && use_v2(ctx, opts) && cfg.sched && cfg.small && cfg.cache && 3 * nhalf >= cfg.lnprob_pipe_min &&
-           3 * nhalf * set->ncomp >= RB_SCHED_MIN);
+  spec = fused && spec_fits && !lnprob_pipelined(ctx, cfg, opts, set->nsrc, 3 * nhalf, set->ncomp);
   int64_t k = 0;
   if (fused && nsteps >= 3) {
     struct Key {
@@ -2550,9 +2559,7 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
     } key;
     memset(&key, 0, sizeof(key));
     key.set = set; key.X = X; key.lnp = lnp; key.naccept = naccept; key.counters = counters; key.buf = ctx->samp_buf;
-    key.stream = s; key.split = *split; key.a = a;
-    rb_default_opts(&key.opts);
-    if (opts) key.opts = *opts;
+    key.stream = s; key.split = *split; key.opts = od; key.a = a;
     const unsigned char *kb = reinterpret_cast<const unsigned char *>(&key);
     if (!ctx->samp_graph || ctx->samp_key.size() != sizeof(key) || memcmp(ctx->samp_key.data(), kb, sizeof(key)) != 0) {
       if (ctx->samp_graph) {
@@ -2794,13 +2801,7 @@ int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const
     nb += (nls - 2) * ngW + (h2 - l2 + cs::ACF_GROUP - 1) / cs::ACF_GROUP;
   }
   const size_t need = (size_t)nb * std::min<long long>(nl_all, cs::ACF_LAGS) * v.ndim * sizeof(double);
-  if (need > ctx->cs_bytes) {
-    if (ctx->cs_buf) cudaFree(ctx->cs_buf);
-    ctx->cs_buf = nullptr;
-    ctx->cs_bytes = 0;
-    CUDA_TRY(cudaMalloc(&ctx->cs_buf, need));
-    ctx->cs_bytes = need;
-  }
+  if ((rc = grow(ctx->cs_buf, ctx->cs_bytes, need)) != RB_OK) return rc;
   double *partial = static_cast<double *>(ctx->cs_buf);
   const size_t smem = (size_t)v.ndim * (2 * cs::ACF_TT + cs::ACF_LAGS + 2 * cs::ACF_R) * sizeof(double);
   CUDA_TRY(cudaFuncSetAttribute(cs::k_acf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -2851,10 +2852,10 @@ int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *
   CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, 8 * sizeof(unsigned long long), ctx->stream));
   const long long nls = local_sources(v);
   if (nls == 0 || v.nsel == 0) return RB_OK;
-  const int ncomp = set->ncomp, np = ctx->mol.npart, nn = ctx->mol.nline;
+  const int ncomp = set->ncomp;
   const bool v2 = use_v2(ctx, opts);
   // v2: observed-line mode, line k of model m at obs_surf[m][k]; v1: every line, at surf[m][J - 1]
-  const int stride = v2 ? RB_MAX_OBS : nn;
+  const int stride = v2 ? RB_MAX_OBS : ctx->mol.nline;
   long long total = 0;
   for (long long s = 0; s < nls; ++s) {
     long long lo, hi;
@@ -2862,33 +2863,24 @@ int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *
     total = std::max(total, (hi - lo) * v.nsel);
   }
   const long long per_call = std::max<long long>(1, RB_PREDICT_MAX / ncomp);
-  const long long mmax = std::min(total, per_call) * ncomp;
-  const size_t b_d = align256((size_t)mmax * sizeof(double)), b_dn = align256((size_t)mmax * np * sizeof(double));
-  const size_t b_o = align256((size_t)mmax * stride * sizeof(double)), b_s = align256((size_t)mmax * sizeof(int));
-  const size_t b_all = 2 * b_d + b_dn + b_o + b_s;
-  if (b_all > ctx->ln_bytes) {
-    if (ctx->ln_buf) cudaFree(ctx->ln_buf);
-    ctx->ln_buf = nullptr;
-    ctx->ln_bytes = 0;
-    CUDA_TRY(cudaMalloc(&ctx->ln_buf, b_all));
-    ctx->ln_bytes = b_all;
-  }
-  char *base = static_cast<char *>(ctx->ln_buf);
+  LnprobPipe pp;
+  if ((rc = model_arrays(ctx, std::min(total, per_call) * ncomp, stride, &pp)) != RB_OK) return rc;
   PredictIO io;
   memset(&io, 0, sizeof(io));
   io.v = v;
-  io.tkin = reinterpret_cast<double *>(base);
-  io.cdmol = reinterpret_cast<double *>(base + b_d);
-  io.dens = reinterpret_cast<double *>(base + 2 * b_d);
-  double *surf = reinterpret_cast<double *>(base + 2 * b_d + b_dn);
-  int *status = reinterpret_cast<int *>(base + 2 * b_d + b_dn + b_o);
-  io.surf = surf;
-  io.status = status;
+  io.tkin = pp.tkin;
+  io.cdmol = pp.cdmol;
+  io.dens = pp.dens;
+  io.surf = pp.obs_surf;
+  io.status = pp.status;
   io.stride = stride;
   io.nlines = nlines;
   for (int k = 0; k < nlines; ++k) io.line[k] = v2 ? k : jup[k] - 1;
   io.flux = flux;
   io.counters = reinterpret_cast<unsigned long long *>(counters_dev);
+  SolveIO sio{0, pp.tkin, pp.dens, pp.cdmol, nullptr, nullptr, nullptr, v2 ? nullptr : pp.obs_surf, nullptr, pp.status,
+              ctx->counters};
+  if (v2) observe_lines(sio, pp.obs_surf, nlines, jup);
   const int tpb = 256;
   for (long long s = 0; s < nls; ++s) {
     long long lo, hi;
@@ -2899,30 +2891,14 @@ int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *
     for (long long i0 = 0; i0 < io.nw * v.nsel; i0 += per_call) {
       io.i0 = i0;
       io.ni = std::min(per_call, io.nw * v.nsel - i0);
-      const long long m = io.ni * ncomp;
       const unsigned nbe = (unsigned)((io.ni + tpb - 1) / tpb);
       if (ncomp == 1)
         k_predict_expand<1><<<nbe, tpb, 0, ctx->stream>>>(ctx->mol, io);
       else
         k_predict_expand<2><<<nbe, tpb, 0, ctx->stream>>>(ctx->mol, io);
       CUDA_TRY(cudaMemsetAsync(ctx->counters, 0, sizeof(unsigned long long), ctx->stream));   // queue head only
-      SolveIO sio{m, io.tkin, io.dens, io.cdmol, nullptr, nullptr, nullptr, v2 ? nullptr : surf, nullptr, status,
-                  ctx->counters, 0, nullptr, nullptr, nullptr, nullptr};
-      if (v2) {
-        sio.obs_surf = surf;
-        sio.nobs = nlines;
-        for (int k = 0; k < nlines; ++k) sio.obs_line[k] = jup[k] - 1;
-        const Launch L = v2_launch(ctx, m);
-        if (cfg.sched && cfg.cache && m >= RB_SCHED_MIN) {
-          rc = launch_solve_pipeline(ctx, cfg, sio, L);
-          if (rc != RB_OK) return rc;
-        } else {
-          k_lvg_solve_v2<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, sio);
-        }
-      } else {
-        const Launch L = v1_launch(ctx, m);
-        k_lvg_solve_v1<<<L.blocks, L.warps_per_block * 32, L.smem, ctx->stream>>>(ctx->mol, cfg, sio);
-      }
+      sio.n = io.ni * ncomp;
+      if ((rc = launch_solve(ctx, cfg, opts, sio)) != RB_OK) return rc;
       const unsigned nbf = (unsigned)((io.ni * nlines + tpb - 1) / tpb);
       if (ncomp == 1)
         k_predict_flux<1><<<nbf, tpb, 0, ctx->stream>>>(io);
@@ -2938,10 +2914,8 @@ int rb_predict_sled_dev(rb_ctx *ctx, const rb_srcset *set, const rb_chain_view *
 int rb_ctx_counters(rb_ctx *ctx, int64_t *total_iters_last, int64_t *launches_total) {
   if (!ctx) return RB_ERR_ARG;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  unsigned long long cnt[3] = {0, 0, 0};
-  CUDA_TRY(cudaMemcpyAsync(cnt, ctx->counters, sizeof(cnt), cudaMemcpyDeviceToHost, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  ctx->last_total_iters = (long long)cnt[1];
+  const int rc = read_counters(ctx);
+  if (rc != RB_OK) return rc;
   if (total_iters_last) *total_iters_last = ctx->last_total_iters;
   if (launches_total) *launches_total = ctx->launches;
   return RB_OK;

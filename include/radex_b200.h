@@ -261,6 +261,39 @@ int rb_chain_moments_dev(rb_ctx *ctx, const rb_chain_view *view, double *mean, d
 int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *mean, const double *c0,
                      int64_t k0, int64_t k1, double *rho_sum);
 
+/* ---- corner-plot marginals, covariance and the sample nearest a target, of the device-resident chain: replaces the
+ * replot's `corner` over the pickled chain and the host search of nearest_sample_to_vector (er1:242-266), without
+ * moving the chain.  The view, columns, sources, pointers and errors are as in rb_chain_hist_dev.
+ *   marginals: bin k of a value x for the edges e[0..nbins] of its (source, column) is (number of edges <= x) - 1, and
+ *            x == e[nbins] is in bin nbins - 1 (np.searchsorted(e, x, 'right') - 1: np.histogram / np.histogram2d with
+ *            range=); NaN, +-inf and values outside [e[0], e[nbins]] are not counted.  One read of the chain counts every
+ *            column and as many pairs as fit shared memory (all 45 pairs of 10 columns at 20 bins).
+ *   sums   : s1 = sum (x - c), s2 = sum (x - c)(x - c)^T over each source's selected samples on this rank, c = center of
+ *            the source.  Fixed summation order (per-block partials, then the blocks in order): a repeated call on the same
+ *            rank layout gives the same bits.  Covariance: sums with c = 0 summed over ranks give the mean m = s1 / n;
+ *            sums with c = m summed over ranks give cov = (s2 - s1 s1^T / n) / (n - 1).
+ *   nearest: per selected sample w = L^-1 (x - t) by forward substitution (L = chol of the source, lower triangle), d2 =
+ *            sum_r w_r^2 in r order; per source the minimum d2, NaN before every number (np.argmin), ties to the lowest
+ *            index j W + (gid - s W): the row of the sample in get_chain(discard, thin)[:, s W:(s + 1) W].reshape(-1,
+ *            ndim); x is that sample.  Across ranks: the minimum d2 (NaN first), then the lowest index. */
+#define RB_CHAIN_MAX_BINS 100
+/* edges: DEVICE [nsrc][ncol][nbins+1], finite, strictly increasing (the caller's precondition).
+   counts1: DEVICE [nsrc][ncol][nbins].
+   counts2: DEVICE [nsrc][npair][nbins][nbins] or NULL.
+   Pairs are (a, b) with a < b, in the order (0,1), (0,2), ..., (0,n-1), (1,2), ...; npair = ncol (ncol - 1) / 2.
+   counts2[s][p][ka][kb] counts the samples with column a in bin ka AND column b in bin kb.
+   Counts are ADDED (the caller zeroes them), like rb_chain_hist_dev.  col_i, col_j are HOST arrays. */
+int rb_chain_marginals_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, int32_t ncol, const int32_t *col_i,
+                           const int32_t *col_j, int32_t nbins, const double *edges, uint64_t *counts1, uint64_t *counts2);
+/* center: DEVICE [nsrc][ndim].  s1: [nsrc][ndim], s2: [nsrc][ndim][ndim].
+   Both are written, not added; sources with no walkers on this rank get 0. */
+int rb_chain_sums_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *center, double *s1, double *s2);
+/* target: DEVICE [nsrc][ndim].  chol: DEVICE [nsrc][ndim][ndim], lower triangle read.
+   Outputs: d2 [nsrc], index [nsrc], x [nsrc][ndim].
+   A source with no walkers on this rank gets index -1 and d2 = +inf (and x = 0). */
+int rb_chain_nearest_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *target, const double *chol,
+                         double *d2, int64_t *index, double *x);
+
 /* ---- posterior-predictive SLEDs of the device-resident chain: replaces the host replot's model_lvg over the pickled
  * chain (er1:120-130, er2:122-147), one Radex call per sample, without moving the chain.  DEVICE pointers except jup,
  * asynchronous on the ctx stream; rb_ctx_counters / rb_ctx_cache_stats report the call like any solve call.

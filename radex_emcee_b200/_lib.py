@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(HERE, "libradex_b200.so")
 
 RB_MAX_OBS = 16
 RB_MAX_CHUNKS, RB_CHAIN_MAX_DIM, RB_CHAIN_MAX_COLS, RB_CHAIN_MAX_HIST = 64, 16, 32, 128
+RB_CHAIN_MAX_BINS = 100
 STOP_PYRADEX, STOP_RADEX = 0, 1
 GEOM = {"sphere": 1, "lvg": 2, "slab": 3}
 ST_T_RANGE, ST_N_RANGE, ST_MAXITER, ST_NONFINITE = 1, 2, 4, 8
@@ -101,7 +102,11 @@ SIGNATURES = {
                                     _vp, _vp, _vp]),
     "rb_chain_moments_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), _vp, _vp]),
     "rb_chain_acf_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, _vp, _vp, C.c_int64, C.c_int64, _vp]),
-    "rb_predict_sled_dev": (C.c_int, [_vp, _vp, C.POINTER(rb_chain_view), C.c_int32, _ip, C.POINTER(rb_opts), _vp,
+    "rb_chain_marginals_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, C.c_int32, _ip, _ip, C.c_int32, _vp,
+                                         _vp, _vp]),
+    "rb_chain_sums_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, _vp, _vp, _vp]),
+    "rb_chain_nearest_dev": (C.c_int, [_vp, C.POINTER(rb_chain_view), C.c_int32, _vp, _vp, _vp, _vp, _vp]),
+    "rb_predict_sled_dev":(C.c_int, [_vp, _vp, C.POINTER(rb_chain_view), C.c_int32, _ip, C.POINTER(rb_opts), _vp,
                                       _vp]),
 }
 

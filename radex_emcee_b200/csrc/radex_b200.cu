@@ -1406,6 +1406,7 @@ __global__ void k_stretch_accept(long long ns, int ndim, double *S, double *lnp_
 
 #include "stretch.cuh"
 #include "chain_stats.cuh"
+#include "chain_marginals.cuh"
 #include "predict_sled.cuh"
 
 // ------------------------------------------------------------------------------------------------
@@ -2817,6 +2818,141 @@ int rb_chain_acf_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const
     CUDA_TRY(cudaGetLastError());
     ctx->launches += 2;
   }
+  return RB_OK;
+}
+
+// ---- corner-plot marginals, covariance sums, nearest sample (chain_marginals.cuh) ----------------------------------
+// blocks per local source: enough to fill the GPU, at most one per `per` items of the largest local source
+static long long blocks_per_source(const rb_ctx *ctx, const cs::View &v, long long nls, long long per) {
+  const long long items = std::min<long long>(v.W, v.nlocal) * v.nsel;
+  long long bx = std::max<long long>(1, (long long)ctx->sm_count * 4 / nls);
+  return std::max<long long>(1, std::min<long long>(bx, (items + per - 1) / per));
+}
+
+int rb_chain_marginals_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, int32_t ncol, const int32_t *col_i,
+                           const int32_t *col_j, int32_t nbins, const double *edges, uint64_t *counts1,
+                           uint64_t *counts2) {
+  static const char *who = "rb_chain_marginals_dev";
+  cs::View v;
+  int rc = chain_view(who, view, nsrc, &v);
+  if (rc != RB_OK) return rc;
+  cs::Cols cols;
+  std::string e;
+  if (ncol < 1 || ncol > RB_CHAIN_MAX_COLS || !col_i || !col_j) e = "ncol must be in 1..RB_CHAIN_MAX_COLS";
+  else if (nbins < 1 || nbins > RB_CHAIN_MAX_BINS) e = "nbins must be in 1..RB_CHAIN_MAX_BINS";
+  else if (!edges || !counts1) e = "null edges or counts";
+  for (int c = 0; e.empty() && c < ncol; ++c) {
+    if (col_i[c] < 0 || col_i[c] >= v.ndim || col_j[c] < -1 || col_j[c] >= v.ndim) e = "column outside [0, ndim)";
+    cols.i[c] = col_i[c];
+    cols.j[c] = col_j[c];
+  }
+  cols.n = ncol;
+  if (!e.empty()) {
+    rb_set_error(std::string(who) + ": " + e);
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long nls = local_sources(v);
+  if (nls == 0 || v.nsel == 0) return RB_OK;
+  // shared memory: edges, staged rows, 1-D counters, column bins; then 4 nbins^2 bytes of counters + 2 per pair
+  const int nb = nbins, npair = counts2 ? ncol * (ncol - 1) / 2 : 0;
+  const size_t fixed = (size_t)ncol * (nb + 1) * 8 + (size_t)cs::MARG_THREADS * (v.ndim | 1) * 8 + (size_t)ncol * nb * 4 +
+                       (size_t)ncol * cs::MARG_THREADS;
+  const size_t per_pair = (size_t)nb * nb * 4 + 2;
+  const long long fit = ((long long)ctx->smem_optin - (long long)fixed) / (long long)per_pair;
+  if (npair > 0 && fit < 1) {
+    rb_set_error(std::string(who) + ": one pair's counters do not fit shared memory");
+    return RB_ERR_LIMIT;
+  }
+  // pair groups of equal size, as few as fit: each group is one read of the chain
+  const int ngroups = npair > 0 ? (int)((npair + fit - 1) / fit) : 1;
+  const int per_group = npair > 0 ? (npair + ngroups - 1) / ngroups : 0;
+  CUDA_TRY(cudaFuncSetAttribute(cs::k_marg, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)(fixed + per_group * per_pair)));
+  // at most 2^31 items per block so that the 32-bit shared counters cannot wrap
+  const long long items = std::min<long long>(v.W, v.nlocal) * v.nsel;
+  long long bx = blocks_per_source(ctx, v, nls, cs::MARG_THREADS);
+  bx = std::max<long long>(bx, (items >> 31) + 1);
+  if (nls > 65535 || bx > 0x7fffffffLL) {
+    rb_set_error(std::string(who) + ": too many sources on this rank");
+    return RB_ERR_ARG;
+  }
+  for (int g = 0; g < ngroups; ++g) {
+    const int p0 = g * per_group, npg = std::min(per_group, npair - p0);
+    const size_t smem = fixed - (g ? (size_t)ncol * nb * 4 : 0) + (size_t)npg * per_pair;
+    cs::k_marg<<<dim3((unsigned)bx, (unsigned)nls), cs::MARG_THREADS, smem, ctx->stream>>>(
+        v, cols, nb, p0, npg, g == 0, edges, reinterpret_cast<unsigned long long *>(counts1),
+        reinterpret_cast<unsigned long long *>(counts2));
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches += 1;
+  }
+  return RB_OK;
+}
+
+int rb_chain_sums_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *center, double *s1,
+                      double *s2) {
+  static const char *who = "rb_chain_sums_dev";
+  cs::View v;
+  int rc = chain_view(who, view, nsrc, &v);
+  if (rc != RB_OK) return rc;
+  if (nsrc < 1 || !center || !s1 || !s2) {
+    rb_set_error(std::string(who) + ": bad argument (nsrc >= 1, non-null center, s1, s2)");
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long nls = local_sources(v);
+  const int nent = v.ndim + v.ndim * (v.ndim + 1) / 2;
+  const long long bx = (nls > 0 && v.nsel > 0) ? blocks_per_source(ctx, v, nls, cs::SUMS_THREADS) : 0;
+  if (nls > 65535) {
+    rb_set_error(std::string(who) + ": too many sources on this rank");
+    return RB_ERR_ARG;
+  }
+  if ((rc = grow(ctx->cs_buf, ctx->cs_bytes, std::max<size_t>(8, (size_t)nls * bx * nent * sizeof(double)))) != RB_OK)
+    return rc;
+  double *partial = static_cast<double *>(ctx->cs_buf);
+  if (bx > 0) {
+    cs::k_sums<<<dim3((unsigned)bx, (unsigned)nls), cs::SUMS_THREADS, 0, ctx->stream>>>(v, center, partial);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches += 1;
+  }
+  const long long nout = (long long)nsrc * nent;
+  cs::k_sums_reduce<<<(unsigned)((nout + 255) / 256), 256, 0, ctx->stream>>>(v, nsrc, bx > 0 ? nls : 0, (int)bx,
+                                                                             partial, s1, s2);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches += 1;
+  return RB_OK;
+}
+
+int rb_chain_nearest_dev(rb_ctx *ctx, const rb_chain_view *view, int32_t nsrc, const double *target, const double *chol,
+                         double *d2, int64_t *index, double *x) {
+  static const char *who = "rb_chain_nearest_dev";
+  cs::View v;
+  int rc = chain_view(who, view, nsrc, &v);
+  if (rc != RB_OK) return rc;
+  if (nsrc < 1 || !target || !chol || !d2 || !index || !x) {
+    rb_set_error(std::string(who) + ": bad argument (nsrc >= 1, non-null target, chol, d2, index, x)");
+    return RB_ERR_ARG;
+  }
+  if ((rc = chain_device(who, ctx)) != RB_OK) return rc;
+  const long long nls = local_sources(v);
+  const long long bx = (nls > 0 && v.nsel > 0) ? blocks_per_source(ctx, v, nls, cs::NEAR_THREADS) : 0;
+  if (nls > 65535) {
+    rb_set_error(std::string(who) + ": too many sources on this rank");
+    return RB_ERR_ARG;
+  }
+  const size_t nblk = (size_t)nls * bx;
+  if ((rc = grow(ctx->cs_buf, ctx->cs_bytes, std::max<size_t>(16, nblk * 16))) != RB_OK) return rc;
+  double *pd2 = static_cast<double *>(ctx->cs_buf);
+  long long *pidx = reinterpret_cast<long long *>(pd2 + nblk);
+  if (bx > 0) {
+    cs::k_near<<<dim3((unsigned)bx, (unsigned)nls), cs::NEAR_THREADS, 0, ctx->stream>>>(v, target, chol, pd2, pidx);
+    CUDA_TRY(cudaGetLastError());
+    ctx->launches += 1;
+  }
+  cs::k_near_reduce<<<(unsigned)((nsrc + 255) / 256), 256, 0, ctx->stream>>>(
+      v, nsrc, bx > 0 ? nls : 0, (int)bx, pd2, pidx, d2, reinterpret_cast<long long *>(index), x);
+  CUDA_TRY(cudaGetLastError());
+  ctx->launches += 1;
   return RB_OK;
 }
 

@@ -27,6 +27,11 @@ chain does not fit in host memory (``--walkers 1048576``).
 With ``predict_jup`` (CLI ``--predict-sled J ...``) the result also gains the posterior-predictive SLED: the 16/50/84
 percentiles of the model flux of each requested line over the chain (``StretchSampler.get_predictive_quantiles``), per
 component with two components -- the model SLEDs the reference's replot draws from the pickled chain.
+
+With ``corner_bins`` (CLI ``--corner-bins B``) the result also gains ``corner``: the counts the replot's corner plots are
+drawn from (B-bin marginals of every summary column and of every pair, ``StretchSampler.get_histograms``), the covariance
+and the Mahalanobis-nearest sample to ``theta_med`` -- all computed on the device, so they work with ``--summaries-only``;
+with ``outdir`` they are also written to ``<source>_corner.npz`` (``<source>_corner_2comp.npz`` with two components).
 """
 from __future__ import annotations
 
@@ -138,6 +143,26 @@ def sled_results(sampler, jup):
     return [dict(sled_jup=np.array(jup), sled_summary=sled_summaries(Qs, jup)) for Qs in Q]
 
 
+def corner_results(sampler, ncomp, theta_med, bins):
+    """Per source: the ``corner`` result item from the device-resident chain -- B-bin marginals of the summary columns
+    and of their pairs, the covariance and the sample nearest ``theta_med`` ([nsources, ndim]) in the Mahalanobis
+    metric of nearest_sample_to_vector."""
+    cols = summary_columns(ncomp)
+    edges, h1, h2, _pairs = sampler.get_histograms(bins, columns=cols)
+    cov = sampler.get_covariance()
+    x, idx, d2 = sampler.get_nearest_sample(theta_med, metric="mahalanobis")
+    return [dict(columns=cols, edges=edges[s], hist1d=h1[s], hist2d=h2[s], covariance=cov[s], theta_nearest=x[s],
+                 theta_nearest_index=int(idx[s]), theta_nearest_d2=float(d2[s])) for s in range(len(edges))]
+
+
+def write_corner(outdir, source, ncomp, corner):
+    """<source>_corner.npz (<source>_corner_2comp.npz): the corner item, columns as (i, j) rows (j = -1: x[i] alone)."""
+    name = os.path.join(outdir, "%s_corner%s.npz" % (source, "" if ncomp == 1 else "_2comp"))
+    cols = np.array([(c, -1) if isinstance(c, int) else c for c in corner["columns"]], dtype=np.int64)
+    np.savez(name, **dict(corner, columns=cols))
+    return name
+
+
 def log_autocorr(source, tau):
     logger.info("%s: integrated autocorrelation time (steps) %s", source, np.array2string(np.asarray(tau), precision=1))
 
@@ -217,11 +242,12 @@ def prefit(ncomp, R, Jup, flux, eflux, bounds, p0, T_d=None, opts=None):
 
 def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
                device=0, datapath=None, opts=None, outdir=None, store_chain=True, allow_synthetic=False,
-               chain_to_host=True, predict_jup=None):
+               chain_to_host=True, predict_jup=None, corner_bins=None):
     """One pass of the reference's per-source loop.  Returns a dict with every item of the pickle plus
     the percentile summaries, the sampler's acceptance fraction and the integrated autocorrelation time.
     ``chain_to_host=False``: the chain stays on the device (``chain`` and ``lnprobability`` are None).
-    ``predict_jup``: line indices J whose posterior-predictive fluxes the result gains (``sled_jup``, ``sled_summary``)."""
+    ``predict_jup``: line indices J whose posterior-predictive fluxes the result gains (``sled_jup``, ``sled_summary``).
+    ``corner_bins``: bins of the ``corner`` item the result gains (marginals, covariance, nearest sample)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -273,8 +299,12 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
                   molfile=R.molpath, molfile_synthetic=R.molfile_is_synthetic)
     if predict_jup is not None:
         result.update(sled_results(sampler, predict_jup)[0])
+    if corner_bins is not None:
+        result["corner"] = corner_results(sampler, ncomp, theta_med[None], corner_bins)[0]
     if outdir is not None:
         os.makedirs(outdir, exist_ok=True)
+        if corner_bins is not None:
+            result["corner_npz"] = write_corner(outdir, source, ncomp, result["corner"])
         if ncomp == 1:     # emcee_radex.py:504-509
             name = os.path.join(outdir, "%s_bounds.pickle" % source)
             payload = (source, z, bounds, (Jup, flux, eflux), (popt, pcov), pmin, theta_med, (chain, lnprobability))
@@ -289,14 +319,14 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
 
 def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
                              device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False, chain_to_host=True,
-                             predict_jup=None):
+                             predict_jup=None, corner_bins=None):
     """BASELINE.json configs[3]: every source of the table in ONE ensemble.  The reference fits the sources one after the
     other (emcee_radex.py:389); here the pre-fits run per source (they are a few dozen batched launches each) and the
     walkers of all sources -- each with its own background temperature, bounds, line set and, with two components, dust
     temperature -- step together: ``nwalkers`` per source, partners drawn inside the source's own sub-ensemble, one fused
     lnprob launch per half-step for all of them.  Under torchrun the ensemble is sharded over the ranks (whole sources per
-    rank).  Returns one result dict per source, the same items ``fit_source`` returns (``chain_to_host`` and
-    ``predict_jup`` as there)."""
+    rank).  Returns one result dict per source, the same items ``fit_source`` returns (``chain_to_host``, ``predict_jup``
+    and ``corner_bins`` as there)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -340,6 +370,10 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
     acc = sampler.acceptance_fraction
     chain, lnp = (sampler.get_chain(), sampler.get_log_prob()) if chain_to_host else (None, None)
     sleds = sled_results(sampler, predict_jup) if predict_jup is not None else None
+    corners = None
+    if corner_bins is not None:
+        meds = np.array([summaries_from_quantiles(Q[k], ncomp)[1] for k in range(len(setups))])
+        corners = corner_results(sampler, ncomp, meds, corner_bins)
     results = []
     for k, st in enumerate(setups):
         sl = slice(k * nwalkers, (k + 1) * nwalkers)
@@ -352,8 +386,12 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
                    acceptance_fraction_per_walker=acc[sl], molfile=R.molpath, molfile_synthetic=R.molfile_is_synthetic)
         if sleds is not None:
             res.update(sleds[k])
+        if corners is not None:
+            res["corner"] = corners[k]
         if outdir is not None and sampler.rank == 0:
             os.makedirs(outdir, exist_ok=True)
+            if corners is not None:
+                res["corner_npz"] = write_corner(outdir, st["source"], ncomp, corners[k])
             if ncomp == 1:
                 name = os.path.join(outdir, "%s_bounds.pickle" % st["source"])
                 payload = (st["source"], st["z"], st["bounds"], st["data"], (st["popt"], st["pcov"]), st["pmin"],
@@ -390,6 +428,8 @@ def print_summary(res, ncomp, file=None):
             print("xxx: %s" % name, file=out)
             for J, v in plane.items():
                 print("xxx: J=%d %s" % (J, tuple(float(x) for x in v)), file=out)
+    if "corner" in res:
+        print("xxx: sample nearest the median (Mahalanobis): %s" % res["corner"]["theta_nearest"], file=out)
 
 
 def main(argv=None):
@@ -415,6 +455,10 @@ def main(argv=None):
     ap.add_argument("--predict-sled", type=int, nargs="+", default=None, metavar="J",
                     help="also summarise the posterior-predictive flux of these lines (1-based J, at most 16), per "
                          "component with two; computed on the GPU, so it works with --summaries-only")
+    ap.add_argument("--corner-bins", type=int, default=None, metavar="B",
+                    help="also compute the corner-plot counts (B-bin marginals of the summary columns and their pairs), "
+                         "the covariance and the sample nearest the median, on the GPU (works with --summaries-only); "
+                         "written to <source>_corner.npz")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO)
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -433,7 +477,8 @@ def main(argv=None):
         for res in fit_sources_concurrently(sources, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                                             n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir,
                                             datapath=args.datapath, allow_synthetic=args.allow_synthetic,
-                                            chain_to_host=not args.summaries_only, predict_jup=args.predict_sled):
+                                            chain_to_host=not args.summaries_only, predict_jup=args.predict_sled,
+                                            corner_bins=args.corner_bins):
             if rank == 0:
                 print_summary(res, args.ncomp)
         if world > 1:
@@ -444,7 +489,7 @@ def main(argv=None):
         res = fit_source(source, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                          n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir, datapath=args.datapath,
                          allow_synthetic=args.allow_synthetic, chain_to_host=not args.summaries_only,
-                         predict_jup=args.predict_sled)
+                         predict_jup=args.predict_sled, corner_bins=args.corner_bins)
         print_summary(res, args.ncomp)
 
 

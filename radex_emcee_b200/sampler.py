@@ -30,7 +30,9 @@ Posterior statistics where the chain lives
   (emcee's integrated autocorrelation time) read the stored chain in place on every rank (csrc/chain_stats.cuh):
   only 256-bin digit histograms and per-lag sums cross ranks (``all_reduce``) and PCIe, never the chain.
   ``get_predictive_quantiles`` does the same for the model SLED of every sample (csrc/predict_sled.cuh): the predicted
-  line fluxes are solved from the chain in place and ranked where they are computed.
+  line fluxes are solved from the chain in place and ranked where they are computed.  ``get_histograms``,
+  ``get_covariance`` and ``get_nearest_sample`` (csrc/chain_marginals.cuh) give the counts a corner plot is drawn from, the
+  covariance and the sample nearest a target; only counts, sums and one row per source cross ranks.
 
 The arithmetic is behind an ``engine`` object so that the host logic (sharding, gather order,
 bookkeeping) can be exercised on CPU by the test-suite's engine (tests/ref_engine.py); the
@@ -39,6 +41,7 @@ package itself only ships the CUDA engine -- there is no CPU fallback in the pro
 from __future__ import annotations
 
 import ctypes as C
+import itertools
 import logging
 
 import numpy as np
@@ -279,6 +282,49 @@ class CudaEngine:
         self.launches += 1
         return out
 
+    # ---- corner-plot marginals, sums, nearest sample (csrc/chain_marginals.cuh) --------------------------------------
+    def chain_marginals(self, view, nsrc, cols, edges, pairs=True):
+        """Counts of one rank: hist1d [nsrc, ncol, B] and hist2d [nsrc, npair, B, B] (int64, None without pairs) for
+        the edges [nsrc, ncol, B + 1]."""
+        self._bind_stream()
+        ncol, B = len(cols), edges.shape[2] - 1
+        ci = (C.c_int32 * ncol)(*[i for i, _ in cols])
+        cj = (C.c_int32 * ncol)(*[j for _, j in cols])
+        e = torch.from_numpy(np.ascontiguousarray(edges, dtype=np.float64)).to(self.device)
+        h1 = torch.zeros((nsrc, ncol, B), dtype=torch.int64, device=self.device)
+        h2 = torch.zeros((nsrc, ncol * (ncol - 1) // 2, B, B), dtype=torch.int64, device=self.device) if pairs else None
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_marginals_dev(self.ctx.handle, C.byref(vs), nsrc, ncol, ci, cj, B, e.data_ptr(),
+                                                 h1.data_ptr(), h2.data_ptr() if h2 is not None else None))
+        self.launches += 1
+        return h1, h2
+
+    def chain_sums(self, view, nsrc, center):
+        """s1 [nsrc, ndim] and s2 [nsrc, ndim, ndim] of this rank's samples, centred on center [nsrc, ndim]."""
+        self._bind_stream()
+        c = torch.as_tensor(np.ascontiguousarray(center, dtype=np.float64)).to(self.device)
+        s1 = torch.empty((nsrc, view.ndim), dtype=torch.float64, device=self.device)
+        s2 = torch.empty((nsrc, view.ndim, view.ndim), dtype=torch.float64, device=self.device)
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_sums_dev(self.ctx.handle, C.byref(vs), nsrc, c.data_ptr(), s1.data_ptr(),
+                                            s2.data_ptr()))
+        self.launches += 1
+        return s1, s2
+
+    def chain_nearest(self, view, nsrc, target, chol):
+        """This rank's nearest sample per source: d2 [nsrc], index [nsrc] (int64, -1: none here), x [nsrc, ndim]."""
+        self._bind_stream()
+        t = torch.as_tensor(np.ascontiguousarray(target, dtype=np.float64)).to(self.device)
+        L = torch.as_tensor(np.ascontiguousarray(chol, dtype=np.float64)).to(self.device)
+        d2 = torch.empty(nsrc, dtype=torch.float64, device=self.device)
+        idx = torch.empty(nsrc, dtype=torch.int64, device=self.device)
+        x = torch.empty((nsrc, view.ndim), dtype=torch.float64, device=self.device)
+        vs = view.c_struct()
+        _lib.check(self.L.rb_chain_nearest_dev(self.ctx.handle, C.byref(vs), nsrc, t.data_ptr(), L.data_ptr(),
+                                               d2.data_ptr(), idx.data_ptr(), x.data_ptr()))
+        self.launches += 1
+        return d2, idx, x
+
     # ---- posterior-predictive SLEDs (csrc/predict_sled.cuh) ---------------------------------------------------------
     def predict_sled(self, view, jup, counters=None):
         """Model fluxes of the lines ``jup`` for every selected sample of ``view``: [nplanes, nsel, nlocal, nlines] on the
@@ -326,8 +372,9 @@ def walkers_independent(coords):
 class StretchSampler:
     """``EnsembleSampler``-like driver: ``run_mcmc``, ``get_chain``, ``get_log_prob``, ``reset``,
     ``acceptance_fraction`` (per walker, like emcee), ``get_autocorr_time``, ``get_quantiles`` (exact
-    percentiles of the stored chain without moving it), and the posterior-predictive SLEDs ``get_predicted_fluxes`` /
-    ``get_predictive_quantiles``."""
+    percentiles of the stored chain without moving it), the posterior-predictive SLEDs ``get_predicted_fluxes`` /
+    ``get_predictive_quantiles``, and the corner-plot counts, covariance and nearest sample ``get_histograms`` /
+    ``get_covariance`` / ``get_nearest_sample``."""
 
     def __init__(self, nwalkers, ndim, engine, a=2.0, seed=0, group=None, randomize_split=True, nsources=1,
                  split_block=None, native=True, time_gather=False):
@@ -587,6 +634,120 @@ class StretchSampler:
             np.subtract(b, diff * (1 - t), out=out, where=t >= 0.5)
         out[np.broadcast_to(has_nan[:, None, :], out.shape)] = np.nan
         return out
+
+    # ---- corner-plot marginals, covariance, nearest sample ------------------------------------------------------------
+    def _bin_edges(self, view, cols, bins, lohi):
+        """[nsources, ncol, bins + 1] edges as np.histogram / np.histogram2d make them for ``range=lohi`` (None: the exact
+        min and max of each (source, column), found by the radix select; numpy's errors and its widening of lo == hi)."""
+        S, ncol = self.nsources, len(cols)
+        if lohi is None:
+            r = self._percentiles(view, cols, [0, 100]).transpose(0, 2, 1)          # [S, ncol, 2]
+            bad = np.argwhere(~np.isfinite(r).all(axis=2))
+            if bad.size:
+                s, c = bad[0]
+                raise ValueError("autodetected range of [%s, %s] is not finite (source %d, column %d)"
+                                 % (r[s, c, 0], r[s, c, 1], s, c))
+        else:
+            r = np.asarray(lohi, dtype=np.float64)
+            if r.shape == (ncol, 2):
+                r = np.broadcast_to(r, (S, ncol, 2))
+            if r.shape != (S, ncol, 2):
+                raise ValueError("range must be ncol (lo, hi) pairs or [nsources][ncol][2]")
+            if not np.isfinite(r).all():
+                raise ValueError("supplied range is not finite")
+            if (r[..., 0] > r[..., 1]).any():
+                raise ValueError("max must be larger than min in range parameter.")
+        edges = np.empty((S, ncol, bins + 1))
+        for s in range(S):
+            for c in range(ncol):
+                lo, hi = r[s, c]
+                if lo == hi:
+                    lo, hi = lo - 0.5, hi + 0.5
+                edges[s, c] = np.linspace(lo, hi, bins + 1)
+        if np.any(edges[..., :-1] >= edges[..., 1:]):
+            raise ValueError("Too many bins for data range. Cannot create %d finite-sized bins." % bins)
+        return edges
+
+    def get_histograms(self, bins=20, discard=0, thin=1, columns=None, range=None):
+        """The counts a corner plot is drawn from, per source: (edges [nsources, ncol, bins + 1], hist1d int64 [nsources,
+        ncol, bins], hist2d int64 [nsources, npair, bins, bins], pairs).  ``pairs`` lists the column pairs (a, b), a < b, in
+        the order (0, 1), (0, 2), ..., (1, 2), ...; hist2d[s, p] is ``np.histogram2d(col_a, col_b, bins, range=...)`` of
+        source s's slice of ``get_chain(flat=True, discard=discard, thin=thin)`` and hist1d[s, c] is ``np.histogram``.
+        ``columns`` as in ``get_quantiles``.  ``range``: None (each (source, column) from its exact min to its max, as
+        numpy and ``corner`` do; a NaN or infinite value raises ValueError), ncol (lo, hi) pairs for every source, or
+        [nsources][ncol][2].  The chain is read in place; only the counts cross ranks (``all_reduce``) and PCIe."""
+        bins = int(bins)
+        if not 1 <= bins <= _lib.RB_CHAIN_MAX_BINS:
+            raise ValueError("bins must be in 1..%d" % _lib.RB_CHAIN_MAX_BINS)
+        view = self._chain_view(discard, thin)
+        cols = self._columns(columns)
+        ncol = len(cols)
+        edges = self._bin_edges(view, cols, bins, range)
+        h1, h2 = self.engine.chain_marginals(view, self.nsources, cols, edges, pairs=ncol > 1)
+        h1 = self._allreduce(h1).cpu().numpy()
+        h2 = (self._allreduce(h2).cpu().numpy() if h2 is not None
+              else np.zeros((self.nsources, 0, bins, bins), dtype=np.int64))
+        pairs = list(itertools.combinations([k for k, _ in enumerate(cols)], 2))
+        return edges, h1, h2, pairs
+
+    def get_covariance(self, discard=0, thin=1):
+        """Covariance of the parameters per source, [nsources, ndim, ndim]: ``np.cov`` of the source's slice of
+        ``get_chain(flat=True, discard=discard, thin=thin)`` (rowvar=False) to rounding.  Two reads of the chain: the sums
+        with centre 0 give the mean, the sums centred on the mean give cov = (s2 - s1 s1^T / n) / (n - 1).  NaN propagates."""
+        view = self._chain_view(discard, thin)
+        n = view.nsel * self.split.walkers_per_source
+        if n == 0:
+            raise ValueError("no stored samples are selected")
+        S = self.nsources
+        s1, _ = self.engine.chain_sums(view, S, np.zeros((S, self.ndim)))
+        mean = self._allreduce(s1).cpu().numpy() / n
+        s1, s2 = self.engine.chain_sums(view, S, mean)
+        s1, s2 = self._allreduce(s1).cpu().numpy(), self._allreduce(s2).cpu().numpy()
+        with np.errstate(invalid="ignore", divide="ignore"):
+            return (s2 - s1[:, :, None] * s1[:, None, :] / n) / (n - 1)
+
+    def get_nearest_sample(self, target, discard=0, thin=1, metric="mahalanobis", eps=1e-9):
+        """The selected sample of each source closest to ``target`` ([ndim] for every source, or [nsources, ndim]):
+        (samples [nsources, ndim], index [nsources], d2 [nsources]), as ``driver.nearest_sample_to_vector`` gives on the
+        source's slice of ``get_chain(flat=True, discard=discard, thin=thin)`` (index is the row there).  d2 = |L^-1 (x -
+        target)|^2 with L = cholesky(cov + eps I) ('mahalanobis'), diag of the standard deviations, eps where one is 0
+        ('z'), or I ('euclidean').  A NaN distance is nearest (np.argmin); ties go to the lowest index."""
+        S, nd = self.nsources, self.ndim
+        t = np.asarray(target, dtype=np.float64)
+        if t.shape == (nd,):
+            t = np.broadcast_to(t, (S, nd))
+        if t.shape != (S, nd):
+            raise ValueError("target must have shape (%d,) or (%d, %d)" % (nd, S, nd))
+        if metric == "mahalanobis":
+            L = np.linalg.cholesky(self.get_covariance(discard, thin) + eps * np.eye(nd))
+        elif metric == "z":
+            sd = np.sqrt(np.diagonal(self.get_covariance(discard, thin), axis1=1, axis2=2))
+            L = np.eye(nd) * np.where(sd > 0, sd, eps)[:, None, :]
+        elif metric == "euclidean":
+            L = np.broadcast_to(np.eye(nd), (S, nd, nd))
+        else:
+            raise ValueError("metric must be 'mahalanobis', 'z' or 'euclidean'")
+        view = self._chain_view(discard, thin)
+        if view.nsel == 0:
+            raise ValueError("no stored samples are selected")
+        d2, idx, x = self.engine.chain_nearest(view, S, t, L)
+        if self.world > 1:
+            # minimum d2 (NaN first: key -1; d2 >= 0, so its bits order as int64), then the lowest index, then its row
+            none = torch.iinfo(torch.int64).max
+            key = torch.where(torch.isnan(d2), torch.full_like(idx, -1), d2.view(torch.int64))
+            kmin = self._allreduce_op(key.clone(), self.dist.ReduceOp.MIN)
+            cand = torch.where((key == kmin) & (idx >= 0), idx, torch.full_like(idx, none))
+            imin = self._allreduce_op(cand.clone(), self.dist.ReduceOp.MIN)
+            mine = (idx == imin) & (idx >= 0)
+            bits = self._allreduce(torch.where(mine[:, None], x.view(torch.int64), torch.zeros_like(x, dtype=torch.int64)))
+            d2 = torch.where(kmin == -1, torch.full_like(d2, float("nan")), kmin.view(torch.float64))
+            idx = torch.where(imin == none, torch.full_like(idx, -1), imin)
+            x = bits.view(torch.float64)
+        return x.cpu().numpy(), idx.cpu().numpy(), d2.cpu().numpy()
+
+    def _allreduce_op(self, t, op):
+        self.dist.all_reduce(t, op=op, group=self.group)
+        return t
 
     # ---- posterior-predictive SLEDs -----------------------------------------------------------------------------------
     def _predicted(self, jup, discard, thin):

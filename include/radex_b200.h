@@ -218,6 +218,54 @@ int rb_stretch_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split,
                        int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
                        int64_t *counters, int32_t thin, double *chain, double *lnp_chain);
 
+/* ---- moves and move mixtures: emcee's EnsembleSampler(moves=...) for StretchMove(a) and DEMove(sigma, gamma0).
+ *   rb_move        : one move of the list; weights >= 0 are normalised over the list (emcee's [(move, weight), ...]).
+ *                    gamma0 = 0 means 2.38 / sqrt(2 ndim).
+ *   schedule       : every step applies ONE move of the list to the whole ensemble, drawn from one Philox call keyed by
+ *                    (seed ^ 'MOVESCHD', step) against the cumulative normalised weights (last bound 1): the same on
+ *                    every rank and for any rank count.  rb_move_schedule writes the move index of steps step0 ..
+ *                    step0 + nsteps - 1 to out[nsteps] (host memory, no device needed); a one-move list gives 0.
+ *   DE split       : the split of rb_split generalised to k = 3 groups: in block b, group g holds
+ *                    n_g = block / 3 + (g < block % 3) slots; slot t of group g is walker b*block + pi(off_g + t),
+ *                    off_g = sum_{h<g} n_h, with the same keyed bijection pi of (seed, step, b) (randomize = 1), or
+ *                    b*block + g + 3t (randomize = 0).  For k = 2 this is the red/blue split above.  Every group's
+ *                    complement within its source must hold >= 2 walkers, and block >= 3 (RB_ERR_ARG otherwise).
+ *   DE step        : groups g = 0, 1, 2 in turn: propose (rb_de_propose_dev), lnprob of the group, accept
+ *                    (rb_group_accept_dev); partners are read from the positions as they stand after the earlier groups.
+ *   rb_de_propose_dev   : Q[k] = s + gamma (c_j2 - c_j1) for the local slots k of group g (nslots = nlocal / block * n_g,
+ *                    in slot order), (j1, j2) uniform over the ordered pairs of distinct walkers of the complement of
+ *                    group g within the walker's source, gamma = gamma0 (1 + sigma n), n ~ N(0, 1).  Xall[nwalkers, ndim]
+ *                    is the whole ensemble in global walker order (one rank: X; several: the all-gather of X).
+ *                    src_id[nslots] may be NULL.
+ *   rb_group_accept_dev : accept test of the local slots of group g of ngroups, as rb_stretch_accept2_dev (logfac NULL:
+ *                    0); kind selects the random stream: RB_MOVE_STRETCH with ngroups = 2 (it IS rb_stretch_accept2_dev)
+ *                    or RB_MOVE_DE with ngroups = 3 (and the DE split rules); any other pair is RB_ERR_ARG.
+ *   rb_moves_run_dev    : rb_stretch_run_dev for a move list (arguments as there); one captured CUDA graph per entry of
+ *                    the list, the host launches the scheduled move's graph step after step without a device sync.
+ *                    rb_stretch_run_dev(a) is rb_moves_run_dev with the single move {RB_MOVE_STRETCH, a}.
+ * DE random numbers: Philox4x32-10 keyed by seed ^ 'DEmvmove', counter (global id, 4 step + group, draw); the split
+ * of a step stays keyed by (seed, step, block) whatever the move.                                                   */
+enum rb_move_kind { RB_MOVE_STRETCH = 0, RB_MOVE_DE = 1 };
+#define RB_MAX_MOVES 8
+typedef struct rb_move {
+  int32_t kind;      /* rb_move_kind                                    */
+  int32_t reserved;
+  double a;          /* RB_MOVE_STRETCH: scale, > 1 (emcee: 2)          */
+  double gamma0;     /* RB_MOVE_DE: 0 = 2.38 / sqrt(2 ndim)             */
+  double sigma;      /* RB_MOVE_DE: >= 0 (emcee: 1e-5)                  */
+  double weight;     /* >= 0, normalised over the list                  */
+} rb_move;
+int rb_move_schedule(uint64_t seed, uint64_t step0, int64_t nsteps, const double *weights, int32_t nmoves, int32_t *out);
+int rb_moves_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, const rb_move *moves, int32_t nmoves,
+                     uint64_t step0, int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
+                     int64_t *counters, int32_t thin, double *chain, double *lnp_chain);
+int rb_de_propose_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t group, int64_t gid_base, int64_t nlocal,
+                      int32_t ndim, const double *X, const double *Xall, double gamma0, double sigma, double *Q,
+                      int32_t *src_id);
+int rb_group_accept_dev(rb_ctx *ctx, const rb_split *split, int32_t kind, uint64_t step, int32_t group, int32_t ngroups,
+                        int64_t gid_base, int64_t nlocal, int32_t ndim, double *X, double *lnp, const double *Q,
+                        const double *lnp_new, const double *logfac, int64_t *naccept, int64_t *nan_count);
+
 /* ---- posterior statistics of the device-resident chain: replaces np.percentile over the flattened chain
  * (er1:511-531) and emcee's get_autocorr_time / integrated_time, without moving the chain.  DEVICE pointers,
  * asynchronous on the ctx stream.  Argument errors give RB_ERR_ARG, a machine without a CUDA device RB_ERR_CUDA.

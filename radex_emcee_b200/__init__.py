@@ -3,7 +3,8 @@
 Public surface (mirrors the reference's):
   Radex                       pyradex.Radex-compatible batched solver      (radex.py)
   emcee_radex, emcee_radex_2comp   lnprob/lnprior/lnlike/model_lvg, vectorised  (emcee_radex*.py)
-  StretchSampler              device-resident stretch-move ensemble sampler (sampler.py)
+  StretchSampler              device-resident ensemble sampler (sampler.py)
+  StretchMove, DEMove         its moves, alone or mixed (emcee's moves=)   (moves.py)
   read_data, get_source       flux table readers                           (data.py)
 The CUDA library (libradex_b200.so) must be built; there is no CPU fallback.
 """

@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(HERE, "libradex_b200.so")
 RB_MAX_OBS = 16
 RB_MAX_CHUNKS, RB_CHAIN_MAX_DIM, RB_CHAIN_MAX_COLS, RB_CHAIN_MAX_HIST = 64, 16, 32, 128
 RB_CHAIN_MAX_BINS = 100
+RB_MOVE_STRETCH, RB_MOVE_DE, RB_MAX_MOVES = 0, 1, 8
 STOP_PYRADEX, STOP_RADEX = 0, 1
 GEOM = {"sphere": 1, "lvg": 2, "slab": 3}
 ST_T_RANGE, ST_N_RANGE, ST_MAXITER, ST_NONFINITE = 1, 2, 4, 8
@@ -41,6 +42,11 @@ class rb_source(C.Structure):
 class rb_split(C.Structure):
     _fields_ = [("nwalkers", C.c_int64), ("walkers_per_source", C.c_int64), ("block", C.c_int64),
                 ("randomize", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64)]
+
+
+class rb_move(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("reserved", C.c_int32), ("a", C.c_double), ("gamma0", C.c_double),
+                ("sigma", C.c_double), ("weight", C.c_double)]
 
 
 class rb_chain_view(C.Structure):
@@ -95,6 +101,13 @@ SIGNATURES = {
                                          C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rb_stretch_run_dev": (C.c_int, [_vp, _vp, C.POINTER(rb_split), C.c_double, C.c_uint64, C.c_int64,
                                      C.POINTER(rb_opts), _vp, _vp, _vp, _vp, C.c_int32, _vp, _vp]),
+    "rb_move_schedule": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, _dp, C.c_int32, _ip]),
+    "rb_moves_run_dev": (C.c_int, [_vp, _vp, C.POINTER(rb_split), C.POINTER(rb_move), C.c_int32, C.c_uint64, C.c_int64,
+                                   C.POINTER(rb_opts), _vp, _vp, _vp, _vp, C.c_int32, _vp, _vp]),
+    "rb_de_propose_dev": (C.c_int, [_vp, C.POINTER(rb_split), C.c_uint64, C.c_int32, C.c_int64, C.c_int64, C.c_int32,
+                                    _vp, _vp, C.c_double, C.c_double, _vp, _vp]),
+    "rb_group_accept_dev": (C.c_int, [_vp, C.POINTER(rb_split), C.c_int32, C.c_uint64, C.c_int32, C.c_int32, C.c_int64,
+                                      C.c_int64, C.c_int32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rb_ctx_counters": (C.c_int, [_vp, _lp, _lp]),
     "rb_ctx_cache_stats": (C.c_int, [_vp, _lp]),
     "rb_fp64_peak": (C.c_int, [_vp, _dp]),
@@ -282,3 +295,12 @@ class Context:
         it, ln = C.c_int64(), C.c_int64()
         check(load().rb_ctx_counters(self.handle, C.byref(it), C.byref(ln)))
         return it.value, ln.value
+
+
+def move_schedule(seed, step0, nsteps, weights):
+    """Index of the move of every step step0 .. step0 + nsteps - 1 (rb_move_schedule; host only, no device needed)."""
+    w = np.ascontiguousarray(weights, dtype=np.float64)
+    out = np.empty(int(nsteps), dtype=np.int32)
+    check(load().rb_move_schedule(int(seed) & 0xFFFFFFFFFFFFFFFF, int(step0), int(nsteps), w.ctypes.data_as(_dp), w.size,
+                                  out.ctypes.data_as(_ip)))
+    return out

@@ -103,8 +103,8 @@ struct rb_ctx {
   void *samp_buf = nullptr;               // rb_stretch_run_dev: complementary half, proposals, their lnprob, step counter (grow-only)
   size_t samp_bytes = 0;
   cudaEvent_t ev_samp = nullptr;
-  cudaGraphExec_t samp_graph = nullptr;   // one stretch-move step, captured for the arguments in samp_key
-  std::vector<unsigned char> samp_key;
+  cudaGraphExec_t samp_graph[RB_MAX_MOVES] = {};   // one step of move m of the list, captured for the arguments in samp_key[m]
+  std::vector<unsigned char> samp_key[RB_MAX_MOVES];
   void *cs_buf = nullptr;                 // rb_chain_acf_dev: per-block partial sums (grow-only)
   size_t cs_bytes = 0;
   long long launches = 0;
@@ -1339,11 +1339,20 @@ __global__ void k_lnprob_combine(LnprobIO io, LnprobPipe pp) {
 // ------------------------------------------------------------------------------------------------
 // stretch move (emcee StretchMove / RedBlueMove; SURVEY.md 3.5) with Philox4x32-10
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+// host and device: the move schedule (rb_move_schedule) is drawn on the host from the same generator
+__host__ __device__ __forceinline__ uint32_t mulhi32(uint32_t a, uint32_t b) {
+#ifdef __CUDA_ARCH__
+  return __umulhi(a, b);
+#else
+  return (uint32_t)(((uint64_t)a * b) >> 32);
+#endif
+}
+
+__host__ __device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+    const uint32_t hi0 = mulhi32(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+    const uint32_t hi1 = mulhi32(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
     const uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
     c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
     k0 += 0x9E3779B9u;
@@ -1351,7 +1360,7 @@ __device__ __forceinline__ void philox4x32_10(uint32_t c[4], uint32_t k0, uint32
   }
 }
 
-__device__ __forceinline__ double u01(uint32_t hi, uint32_t lo) {  // 53-bit uniform in [0,1)
+__host__ __device__ __forceinline__ double u01(uint32_t hi, uint32_t lo) {  // 53-bit uniform in [0,1)
   const unsigned long long v = ((unsigned long long)hi << 32) | lo;
   return (double)(v >> 11) * 1.1102230246251565e-16;
 }
@@ -1767,7 +1776,8 @@ void rb_ctx_destroy(rb_ctx *ctx) {
   for (void *p : {ctx->scratch, ctx->sched_buf, ctx->ln_buf, ctx->samp_buf, ctx->cs_buf, (void *)ctx->counters,
                   (void *)ctx->bslab, (void *)ctx->sched_small, (void *)ctx->src_one})
     if (p) cudaFree(p);
-  if (ctx->samp_graph) cudaGraphExecDestroy(ctx->samp_graph);
+  for (cudaGraphExec_t g : ctx->samp_graph)
+    if (g) cudaGraphExecDestroy(g);
   if (ctx->ev_samp) cudaEventDestroy(ctx->ev_samp);
   for (cudaEvent_t ev : ctx->chunk_done) cudaEventDestroy(ev);
   for (int j = 0; j < 6; ++j) {
@@ -2327,23 +2337,42 @@ static int make_split(const rb_split *sp, int64_t gid_base, int64_t nlocal, int3
   return RB_OK;
 }
 
-// The three entry points below: argument checks (args_ok: the entry point's own arguments), the split, the device, then
-// launch(sp, nhalf, blocks) with blocks of 128 threads over the nhalf walkers of the half
-extern "C++" {   // a template
+// every group of the DE split has slots in every block and a complement of >= 2 walkers within its source (two distinct
+// partners)
+static int check_de_split(const char *who, const rb_split *split) {
+  if (split->block < 3) {
+    rb_set_error(std::string(who) + ": the 3-group split needs blocks of >= 3 walkers");
+    return RB_ERR_ARG;
+  }
+  for (int g = 0; g < 3; ++g)
+    if (split->walkers_per_source - (split->walkers_per_source / split->block) * st2::group_size((int)split->block, 3, g) < 2) {
+      rb_set_error(std::string(who) + ": a group of the 3-group split leaves fewer than 2 walkers of its source to draw from");
+      return RB_ERR_ARG;
+    }
+  return RB_OK;
+}
+
+static double de_gamma0(double gamma0, int ndim) { return gamma0 == 0.0 ? 2.38 / std::sqrt(2.0 * ndim) : gamma0; }
+
+// The entry points below: argument checks (args_ok: the entry point's own arguments), the split, the device, then
+// launch(sp, nslots, blocks) with blocks of 128 threads over the local slots of group g of ngroups (the stretch move: half g
+// of 2)
+extern "C++" {
 template <typename F>
-static int stretch2_launch(const char *who, bool args_ok, rb_ctx *ctx, const rb_split *split, int32_t half,
-                           int64_t gid_base, int64_t nlocal, int32_t ndim, F launch) {
-  if (!ctx || !args_ok || (half != 0 && half != 1)) {
+static int group_launch(const char *who, bool args_ok, rb_ctx *ctx, const rb_split *split, int32_t group, int32_t ngroups,
+                        int64_t gid_base, int64_t nlocal, int32_t ndim, bool de, F launch) {
+  if (!ctx || !args_ok || ngroups < 2 || group < 0 || group >= ngroups) {
     rb_set_error(std::string(who) + ": bad argument");
     return RB_ERR_ARG;
   }
   st2::SplitDev sp;
-  const int rc = make_split(split, gid_base, nlocal, ndim, &sp);
+  int rc = make_split(split, gid_base, nlocal, ndim, &sp);
   if (rc != RB_OK) return rc;
-  const long long nhalf = nlocal / 2;
-  if (nhalf == 0) return RB_OK;
+  if (de && (rc = check_de_split(who, split)) != RB_OK) return rc;
+  const long long nslots = nlocal / sp.B * st2::group_size(sp.B, ngroups, group);
+  if (nslots == 0) return RB_OK;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  launch(sp, nhalf, (unsigned)((nhalf + 127) / 128));
+  launch(sp, nslots, (unsigned)((nslots + 127) / 128));
   CUDA_TRY(cudaGetLastError());
   ctx->launches += 1;
   return RB_OK;
@@ -2352,17 +2381,17 @@ static int stretch2_launch(const char *who, bool args_ok, rb_ctx *ctx, const rb_
 
 int rb_stretch_pack_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
                         int64_t nlocal, int32_t ndim, const double *X, double *Chalf) {
-  return stretch2_launch("rb_stretch_pack_dev", X && Chalf, ctx, split, half, gid_base, nlocal, ndim,
+  return group_launch("rb_stretch_pack_dev", X && Chalf, ctx, split, half, 2, gid_base, nlocal, ndim, false,
                          [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
-    st2::k_pack<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, Chalf);
+    st2::k_pack<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, 2, gid_base, nhalf, ndim, X, Chalf);
   });
 }
 
 int rb_stretch_propose2_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
                             int64_t nlocal, int32_t ndim, const double *X, const double *Call, double a, double *Q,
                             double *logfac, int32_t *src_id) {
-  return stretch2_launch("rb_stretch_propose2_dev", X && Call && Q && logfac && a > 1.0, ctx, split, half, gid_base,
-                         nlocal, ndim, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
+  return group_launch("rb_stretch_propose2_dev", X && Call && Q && logfac && a > 1.0, ctx, split, half, 2, gid_base,
+                         nlocal, ndim, false, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
     st2::k_propose2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, Call, a, split->seed,
                                                  Q, logfac, src_id);
   });
@@ -2371,9 +2400,9 @@ int rb_stretch_propose2_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, i
 int rb_stretch_accept2_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t half, int64_t gid_base,
                            int64_t nlocal, int32_t ndim, double *X, double *lnp, const double *Q, const double *lnp_new,
                            const double *logfac, int64_t *naccept, int64_t *nan_count) {
-  return stretch2_launch("rb_stretch_accept2_dev", X && lnp && Q && lnp_new && logfac, ctx, split, half, gid_base,
-                         nlocal, ndim, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
-    st2::k_accept2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, gid_base, nhalf, ndim, X, lnp, Q, lnp_new, logfac,
+  return group_launch("rb_stretch_accept2_dev", X && lnp && Q && lnp_new && logfac, ctx, split, half, 2, gid_base,
+                         nlocal, ndim, false, [&](const st2::SplitDev &sp, long long nhalf, unsigned nb) {
+    st2::k_accept2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, half, 2, 0, gid_base, nhalf, ndim, X, lnp, Q, lnp_new, logfac,
                                                 split->seed, reinterpret_cast<long long *>(naccept),
                                                 reinterpret_cast<unsigned long long *>(nan_count), nullptr, nullptr);
   });
@@ -2390,11 +2419,11 @@ static int stretch_one_step(rb_ctx *ctx, const rb_srcset *set, const st2::SplitD
   const unsigned nb = (unsigned)((nhalf + tpb - 1) / tpb);
   cudaStream_t s = ctx->stream;
   for (int half = 0; half < 2; ++half) {
-    st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1 - half, 0, nhalf, ndim, X, Cbuf);
+    st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1 - half, 2, 0, nhalf, ndim, X, Cbuf);
     st2::k_propose2<<<nb, tpb, 0, s>>>(sp, d_step, 0, half, 0, nhalf, ndim, X, Cbuf, a, split->seed, Q, logfac, src_id);
     int rc = lnprob_core(ctx, set->ncomp, nhalf, Q, set->d, set->nsrc, set->h[0], src_id, opts, lnp_new);
     if (rc != RB_OK) return rc;
-    st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, half, 0, nhalf, ndim, X, lnp, Q, lnp_new, logfac, split->seed, naccept,
+    st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, half, 2, 0, 0, nhalf, ndim, X, lnp, Q, lnp_new, logfac, split->seed, naccept,
                                       counters, ctx->counters + 2, counters ? counters + 1 : nullptr);
     ctx->launches += 3;
   }
@@ -2419,18 +2448,18 @@ static int stretch_one_step_spec(rb_ctx *ctx, const rb_srcset *set, const st2::S
   const unsigned nb = (unsigned)((nhalf + tpb - 1) / tpb);
   cudaStream_t s = ctx->stream;
   double *Q0 = b.Q3, *Qa = b.Q3 + nhalf * ndim, *Qb = b.Q3 + 2 * nhalf * ndim;
-  st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1, 0, nhalf, ndim, X, b.C1);
+  st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1, 2, 0, nhalf, ndim, X, b.C1);
   int *src3 = (set->nsrc > 1) ? b.src3 : nullptr;
   st2::k_propose2<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, 0, nhalf, ndim, X, b.C1, a, split->seed, Q0, b.logfac0, src3);
-  st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, 0, nhalf, ndim, X, b.Cold);
+  st2::k_pack<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, 2, 0, nhalf, ndim, X, b.Cold);
   st2::k_propose_spec<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, nhalf, ndim, X, b.Cold, Q0, a, split->seed, Qa, Qb, b.logfac1, b.jpart,
                                          src3 ? src3 + nhalf : nullptr, src3 ? src3 + 2 * nhalf : nullptr);
   int rc = lnprob_core(ctx, set->ncomp, 3 * nhalf, b.Q3, set->d, set->nsrc, set->h[0], src3, opts, b.L3);
   if (rc != RB_OK) return rc;
-  st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, 0, nhalf, ndim, X, lnp, Q0, b.L3, b.logfac0, split->seed, naccept, counters,
+  st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, 0, 2, 0, 0, nhalf, ndim, X, lnp, Q0, b.L3, b.logfac0, split->seed, naccept, counters,
                                     ctx->counters + 2, counters ? counters + 1 : nullptr, b.acc0);
   st2::k_select_spec<<<nb, tpb, 0, s>>>(nhalf, ndim, b.acc0, b.jpart, Qa, Qb, b.L3 + nhalf, b.L3 + 2 * nhalf, b.C1, b.Lsel);
-  st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1, 0, nhalf, ndim, X, lnp, b.C1, b.Lsel, b.logfac1, split->seed, naccept,
+  st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, 1, 2, 0, 0, nhalf, ndim, X, lnp, b.C1, b.Lsel, b.logfac1, split->seed, naccept,
                                     counters, nullptr, nullptr);
   st2::k_step_inc<<<1, 1, 0, s>>>(d_step);
   ctx->launches += 9;
@@ -2438,39 +2467,154 @@ static int stretch_one_step_spec(rb_ctx *ctx, const rb_srcset *set, const st2::S
   return RB_OK;
 }
 
-static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, double a, uint64_t step0,
-                            int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
-                            int64_t *counters, int32_t thin, double *chain, double *lnp_chain);
+// ---- moves: differential evolution, the k-group accept, the move schedule --------------------------------------------
+int rb_de_propose_dev(rb_ctx *ctx, const rb_split *split, uint64_t step, int32_t group, int64_t gid_base, int64_t nlocal,
+                      int32_t ndim, const double *X, const double *Xall, double gamma0, double sigma, double *Q,
+                      int32_t *src_id) {
+  const bool ok = X && Xall && Q && std::isfinite(gamma0) && gamma0 >= 0.0 && std::isfinite(sigma) && sigma >= 0.0;
+  const double g0 = de_gamma0(gamma0, ndim);
+  return group_launch("rb_de_propose_dev", ok, ctx, split, group, 3, gid_base, nlocal, ndim, true,
+                      [&](const st2::SplitDev &sp, long long nslots, unsigned nb) {
+    st2::k_de_propose<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, group, gid_base, nslots, ndim, X, Xall, g0, sigma,
+                                                   split->seed, Q, src_id);
+  });
+}
 
-int rb_stretch_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, double a, uint64_t step0,
-                       int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
-                       int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
-  if (!ctx) {
-    rb_set_error("rb_stretch_run_dev: bad argument");
+int rb_group_accept_dev(rb_ctx *ctx, const rb_split *split, int32_t kind, uint64_t step, int32_t group, int32_t ngroups,
+                        int64_t gid_base, int64_t nlocal, int32_t ndim, double *X, double *lnp, const double *Q,
+                        const double *lnp_new, const double *logfac, int64_t *naccept, int64_t *nan_count) {
+  // the random streams have room for two groups per step (stretch: counter 2 step + group) and three (DE: 4 step + group)
+  const bool ok = X && lnp && Q && lnp_new &&
+                  ((kind == RB_MOVE_STRETCH && ngroups == 2) || (kind == RB_MOVE_DE && ngroups == 3));
+  return group_launch("rb_group_accept_dev", ok, ctx, split, group, ngroups, gid_base, nlocal, ndim, kind == RB_MOVE_DE,
+                      [&](const st2::SplitDev &sp, long long nslots, unsigned nb) {
+    st2::k_accept2<<<nb, 128, 0, ctx->stream>>>(sp, nullptr, step, group, ngroups, kind == RB_MOVE_DE ? 1 : 0, gid_base, nslots,
+                                                ndim, X, lnp, Q, lnp_new, logfac, split->seed,
+                                                reinterpret_cast<long long *>(naccept),
+                                                reinterpret_cast<unsigned long long *>(nan_count), nullptr, nullptr);
+  });
+}
+
+int rb_move_schedule(uint64_t seed, uint64_t step0, int64_t nsteps, const double *weights, int32_t nmoves, int32_t *out) {
+  if (nsteps < 0 || nmoves < 1 || nmoves > RB_MAX_MOVES || !weights || (nsteps > 0 && !out)) {
+    rb_set_error("rb_move_schedule: bad argument");
     return RB_ERR_ARG;
   }
-  // CUDA's legacy default stream (what PyTorch's default stream is) cannot be captured: the loop then runs on the
-  // ctx's own stream, ordered after the work already queued on the caller's stream and before what it queues next
+  double tot = 0.0;
+  for (int m = 0; m < nmoves; ++m) {
+    if (!(weights[m] >= 0.0) || !std::isfinite(weights[m])) {
+      rb_set_error("rb_move_schedule: move weights must be finite and >= 0");
+      return RB_ERR_ARG;
+    }
+    tot += weights[m];
+  }
+  if (!(tot > 0.0) || !std::isfinite(tot)) {
+    rb_set_error("rb_move_schedule: the move weights must have a positive, finite sum");
+    return RB_ERR_ARG;
+  }
+  double cum[RB_MAX_MOVES], acc = 0.0;
+  for (int m = 0; m < nmoves; ++m) {
+    acc += weights[m];
+    cum[m] = acc / tot;
+  }
+  cum[nmoves - 1] = 1.0;
+  const uint32_t k0 = (uint32_t)seed ^ 0x4D4F5645u, k1 = (uint32_t)(seed >> 32) ^ 0x53434844u;   // 'MOVE', 'SCHD'
+  for (int64_t k = 0; k < nsteps; ++k) {
+    const uint64_t step = step0 + (uint64_t)k;
+    uint32_t c[4] = {(uint32_t)step, (uint32_t)(step >> 32), 0u, 0u};
+    philox4x32_10(c, k0, k1);
+    const double u = u01(c[0], c[1]);
+    int m = 0;
+    while (m < nmoves - 1 && !(u < cum[m])) ++m;
+    out[k] = m;
+  }
+  return RB_OK;
+}
+
+// One DE step (three sub-steps) on ctx->stream; step index *d_step, as stretch_one_step
+static int de_one_step(rb_ctx *ctx, const rb_srcset *set, const st2::SplitDev &sp, const rb_split *split, double gamma0,
+                       double sigma, const rb_opts *opts, long long N, int ndim, double *X, double *lnp, long long *naccept,
+                       unsigned long long *counters, double *Q, double *lnp_new, int *src_id, unsigned long long *d_step) {
+  const int tpb = 128;
+  cudaStream_t s = ctx->stream;
+  for (int g = 0; g < 3; ++g) {
+    const long long ns = N / sp.B * st2::group_size(sp.B, 3, g);
+    if (ns == 0) continue;
+    const unsigned nb = (unsigned)((ns + tpb - 1) / tpb);
+    st2::k_de_propose<<<nb, tpb, 0, s>>>(sp, d_step, 0, g, 0, ns, ndim, X, X, gamma0, sigma, split->seed, Q, src_id);
+    int rc = lnprob_core(ctx, set->ncomp, ns, Q, set->d, set->nsrc, set->h[0], src_id, opts, lnp_new);
+    if (rc != RB_OK) return rc;
+    st2::k_accept2<<<nb, tpb, 0, s>>>(sp, d_step, 0, g, 3, 1, 0, ns, ndim, X, lnp, Q, lnp_new, nullptr, split->seed, naccept,
+                                      counters, ctx->counters + 2, counters ? counters + 1 : nullptr);
+    ctx->launches += 2;
+  }
+  st2::k_step_inc<<<1, 1, 0, s>>>(d_step);
+  ctx->launches += 1;
+  CUDA_TRY(cudaGetLastError());
+  return RB_OK;
+}
+
+static int moves_run_impl(const char *who, rb_ctx *ctx, const rb_srcset *set, const rb_split *split, const rb_move *moves,
+                          int32_t nmoves, uint64_t step0, int64_t nsteps, const rb_opts *opts, double *X, double *lnp,
+                          int64_t *naccept, int64_t *counters, int32_t thin, double *chain, double *lnp_chain);
+
+// CUDA's legacy default stream (what PyTorch's default stream is) cannot be captured: the loop then runs on the ctx's own
+// stream, ordered after the work already queued on the caller's stream and before what it queues next
+static int moves_run(const char *who, rb_ctx *ctx, const rb_srcset *set, const rb_split *split, const rb_move *moves,
+                     int32_t nmoves, uint64_t step0, int64_t nsteps, const rb_opts *opts, double *X, double *lnp,
+                     int64_t *naccept, int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
+  if (!ctx) {
+    rb_set_error(std::string(who) + ": bad argument");
+    return RB_ERR_ARG;
+  }
   cudaStream_t caller = ctx->stream;
   if (caller != nullptr && caller != cudaStreamLegacy)
-    return stretch_run_impl(ctx, set, split, a, step0, nsteps, opts, X, lnp, naccept, counters, thin, chain, lnp_chain);
+    return moves_run_impl(who, ctx, set, split, moves, nmoves, step0, nsteps, opts, X, lnp, naccept, counters, thin, chain,
+                          lnp_chain);
   CUDA_TRY(cudaSetDevice(ctx->device));
   if (!ctx->ev_samp) CUDA_TRY(cudaEventCreateWithFlags(&ctx->ev_samp, cudaEventDisableTiming));
   CUDA_TRY(cudaEventRecord(ctx->ev_samp, caller));
   CUDA_TRY(cudaStreamWaitEvent(ctx->own_stream, ctx->ev_samp, 0));
   ctx->stream = ctx->own_stream;
-  const int rc = stretch_run_impl(ctx, set, split, a, step0, nsteps, opts, X, lnp, naccept, counters, thin, chain, lnp_chain);
+  const int rc = moves_run_impl(who, ctx, set, split, moves, nmoves, step0, nsteps, opts, X, lnp, naccept, counters, thin,
+                                chain, lnp_chain);
   ctx->stream = caller;
   CUDA_TRY(cudaEventRecord(ctx->ev_samp, ctx->own_stream));
   CUDA_TRY(cudaStreamWaitEvent(caller, ctx->ev_samp, 0));
   return rc;
 }
 
-static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, double a, uint64_t step0,
-                            int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
-                            int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
-  if (!ctx || !set || set->ctx != ctx || !split || !X || !lnp || nsteps < 0 || !(a > 1.0) || thin < 1) {
-    rb_set_error("rb_stretch_run_dev: bad argument");
+int rb_stretch_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, double a, uint64_t step0,
+                       int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
+                       int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
+  const rb_move stretch = {RB_MOVE_STRETCH, 0, a, 0.0, 0.0, 1.0};
+  return moves_run("rb_stretch_run_dev", ctx, set, split, &stretch, 1, step0, nsteps, opts, X, lnp, naccept, counters, thin,
+                   chain, lnp_chain);
+}
+
+int rb_moves_run_dev(rb_ctx *ctx, const rb_srcset *set, const rb_split *split, const rb_move *moves, int32_t nmoves,
+                     uint64_t step0, int64_t nsteps, const rb_opts *opts, double *X, double *lnp, int64_t *naccept,
+                     int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
+  return moves_run("rb_moves_run_dev", ctx, set, split, moves, nmoves, step0, nsteps, opts, X, lnp, naccept, counters, thin,
+                   chain, lnp_chain);
+}
+
+static int moves_run_impl(const char *who, rb_ctx *ctx, const rb_srcset *set, const rb_split *split, const rb_move *moves,
+                          int32_t nmoves, uint64_t step0, int64_t nsteps, const rb_opts *opts, double *X, double *lnp,
+                          int64_t *naccept, int64_t *counters, int32_t thin, double *chain, double *lnp_chain) {
+  bool ok = ctx && set && set->ctx == ctx && split && X && lnp && nsteps >= 0 && thin >= 1 && moves && nmoves >= 1 &&
+            nmoves <= RB_MAX_MOVES;
+  bool has_de = false;
+  for (int m = 0; ok && m < nmoves; ++m) {
+    const rb_move &mv = moves[m];
+    if (mv.kind == RB_MOVE_STRETCH) ok = mv.a > 1.0;
+    else if (mv.kind == RB_MOVE_DE)
+      ok = std::isfinite(mv.gamma0) && mv.gamma0 >= 0.0 && std::isfinite(mv.sigma) && mv.sigma >= 0.0;
+    else ok = false;
+    has_de |= mv.kind == RB_MOVE_DE;
+  }
+  if (!ok) {
+    rb_set_error(std::string(who) + ": bad argument");
     return RB_ERR_ARG;
   }
   const long long N = split->nwalkers;
@@ -2479,12 +2623,18 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
   int rc = make_split(split, 0, N, ndim, &sp);
   if (rc != RB_OK) return rc;
   if (N / split->walkers_per_source != set->nsrc) {
-    rb_set_error("rb_stretch_run_dev: nwalkers / walkers_per_source must equal the number of sources");
+    rb_set_error(std::string(who) + ": nwalkers / walkers_per_source must equal the number of sources");
     return RB_ERR_ARG;
   }
+  if (has_de && (rc = check_de_split(who, split)) != RB_OK) return rc;
+  double weights[RB_MAX_MOVES];
+  for (int m = 0; m < nmoves; ++m) weights[m] = moves[m].weight;
+  std::vector<int32_t> sched((size_t)nsteps);
+  rc = rb_move_schedule(split->seed, step0, nsteps, weights, nmoves, sched.data());
+  if (rc != RB_OK) return rc;
   if (nsteps == 0) return RB_OK;
   CUDA_TRY(cudaSetDevice(ctx->device));
-  const long long nhalf = N / 2;
+  const long long nhalf = N / 2;   // also >= every group of the 3-group split
   // speculative second half-step while the three candidates of every slot can run side by side (one warp each; measured
   // on B200, walker-steps/s with / without: 100 walkers 2.57e5 / 1.35e5, 800: 1.28e6 / 9.4e5, 1600: 1.74e6 / 1.51e6,
   // 3200: 2.22e6 / 2.38e6; two components, 800 walkers: 3.97e5 / 2.54e5), unless rb_opts.spec_half says otherwise
@@ -2516,10 +2666,12 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
     return c.bytes;
   };
   const size_t need = layout(Carve{nullptr});
-  if (need > ctx->samp_bytes && ctx->samp_graph) {   // the captured step holds pointers into the old buffer
-    cudaGraphExecDestroy(ctx->samp_graph);
-    ctx->samp_graph = nullptr;
-  }
+  if (need > ctx->samp_bytes)   // the captured steps hold pointers into the old buffer
+    for (cudaGraphExec_t &g : ctx->samp_graph)
+      if (g) {
+        cudaGraphExecDestroy(g);
+        g = nullptr;
+      }
   rc = grow(ctx->samp_buf, ctx->samp_bytes, need);
   if (rc != RB_OK) return rc;
   layout(Carve{ctx->samp_buf});
@@ -2529,11 +2681,16 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
   CUDA_TRY(cudaStreamSynchronize(s));   // step0_ lives on this stack frame
   unsigned long long *cnt = reinterpret_cast<unsigned long long *>(counters);
   long long *nacc = reinterpret_cast<long long *>(naccept);
+  int *srcp = (set->nsrc > 1) ? src_id : nullptr;
   bool spec = false;   // decided below, once it is known that the half-ensemble runs as one fused launch
-  auto step_once = [&]() {
-    if (spec) return stretch_one_step_spec(ctx, set, sp, split, a, opts, N, ndim, X, lnp, nacc, cnt, sb, d_step);
-    return stretch_one_step(ctx, set, sp, split, a, opts, N, ndim, X, lnp, nacc, cnt, Cbuf, Q, logfac, lnp_new,
-                            (set->nsrc > 1) ? src_id : nullptr, d_step);
+  auto step_once = [&](int m) {
+    const rb_move &mv = moves[m];
+    if (mv.kind == RB_MOVE_DE)
+      return de_one_step(ctx, set, sp, split, de_gamma0(mv.gamma0, ndim), mv.sigma, opts, N, ndim, X, lnp, nacc, cnt, Q,
+                         lnp_new, srcp, d_step);
+    if (spec) return stretch_one_step_spec(ctx, set, sp, split, mv.a, opts, N, ndim, X, lnp, nacc, cnt, sb, d_step);
+    return stretch_one_step(ctx, set, sp, split, mv.a, opts, N, ndim, X, lnp, nacc, cnt, Cbuf, Q, logfac, lnp_new, srcp,
+                            d_step);
   };
   auto store = [&](int64_t k) -> int {   // state after step k (0-based) -> chain slot
     if ((k + 1) % thin) return RB_OK;
@@ -2544,65 +2701,92 @@ static int stretch_run_impl(rb_ctx *ctx, const rb_srcset *set, const rb_split *s
       CUDA_TRY(cudaMemcpyAsync(lnp_chain + (size_t)slot * N, lnp, (size_t)N * sizeof(double), cudaMemcpyDeviceToDevice, s));
     return RB_OK;
   };
-  // A half-ensemble that fits one fused lnprob launch is latency-bound (config 1: 50 models per half-step): its step is
-  // captured once and replayed.  The key holds every argument the captured launches depend on.
+  // A half-ensemble that fits one fused lnprob launch is latency-bound (config 1: 50 models per half-step): the step of
+  // every move of the list is captured once and replayed.  The key holds every argument the captured launches depend on.
   const SolveCfg cfg = make_cfg(ctx, opts, 1.0, set->h[0].tbg, RB_GEOM_LVG);
   const bool fused = !lnprob_pipelined(ctx, cfg, opts, set->nsrc, nhalf, set->ncomp);
   // (forced speculation on a large ensemble: the 1.5 N candidates must still be one fused launch, not the pipeline)
   spec = fused && spec_fits && !lnprob_pipelined(ctx, cfg, opts, set->nsrc, 3 * nhalf, set->ncomp);
-  int64_t k = 0;
-  if (fused && nsteps >= 3) {
-    struct Key {
-      const void *set, *X, *lnp, *naccept, *counters, *buf, *stream;
-      rb_split split;
-      rb_opts opts;
-      double a;
-    } key;
-    memset(&key, 0, sizeof(key));
-    key.set = set; key.X = X; key.lnp = lnp; key.naccept = naccept; key.counters = counters; key.buf = ctx->samp_buf;
-    key.stream = s; key.split = *split; key.opts = od; key.a = a;
-    const unsigned char *kb = reinterpret_cast<const unsigned char *>(&key);
-    if (!ctx->samp_graph || ctx->samp_key.size() != sizeof(key) || memcmp(ctx->samp_key.data(), kb, sizeof(key)) != 0) {
-      if (ctx->samp_graph) {
-        cudaGraphExecDestroy(ctx->samp_graph);
-        ctx->samp_graph = nullptr;
-      }
-      rc = step_once();   // un-captured first step: every lazy allocation happens here
+  if (!(fused && nsteps >= 3)) {
+    for (int64_t k = 0; k < nsteps; ++k) {
+      rc = step_once(sched[k]);
       if (rc != RB_OK) return rc;
-      rc = store(k++);
-      if (rc != RB_OK) return rc;
-      cudaGraph_t g = nullptr;
-      const long long launches_before = ctx->launches;
-      CUDA_TRY(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      rc = step_once();
-      cudaError_t ce = cudaStreamEndCapture(s, &g);
-      ctx->launches = launches_before;   // nothing ran
-      if (rc != RB_OK || ce != cudaSuccess || !g) {
-        if (g) cudaGraphDestroy(g);
-        if (rc == RB_OK) rb_set_error(std::string("rb_stretch_run_dev: graph capture failed: ") + cudaGetErrorString(ce));
-        return rc != RB_OK ? rc : RB_ERR_CUDA;
-      }
-      ce = cudaGraphInstantiate(&ctx->samp_graph, g, 0);
-      cudaGraphDestroy(g);
-      if (ce != cudaSuccess) {
-        ctx->samp_graph = nullptr;
-        rb_set_error(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
-        return RB_ERR_CUDA;
-      }
-      ctx->samp_key.assign(kb, kb + sizeof(key));
-    }
-    const long long per_step = 2 * 4 + 1;   // pack, propose2, lnprob, accept2 per half-step + the step counter (speculative: 9 as well)
-    for (; k < nsteps; ++k) {
-      CUDA_TRY(cudaGraphLaunch(ctx->samp_graph, s));
-      ctx->launches += per_step;
       rc = store(k);
       if (rc != RB_OK) return rc;
     }
     return RB_OK;
   }
-  for (; k < nsteps; ++k) {
-    rc = step_once();
-    if (rc != RB_OK) return rc;
+  struct Key {
+    const void *set, *X, *lnp, *naccept, *counters, *buf, *stream;
+    rb_split split;
+    rb_opts opts;
+    rb_move move;
+  };
+  std::vector<Key> keys((size_t)nmoves);
+  int ready[RB_MAX_MOVES] = {}, ran[RB_MAX_MOVES] = {};   // graph m matches its key / ran un-captured in this call
+  long long per_step[RB_MAX_MOVES];
+  for (int m = 0; m < nmoves; ++m) {
+    Key &key = keys[m];
+    memset(&key, 0, sizeof(key));
+    key.set = set; key.X = X; key.lnp = lnp; key.naccept = naccept; key.counters = counters; key.buf = ctx->samp_buf;
+    key.stream = s; key.split = *split; key.opts = od;
+    key.move.kind = moves[m].kind;
+    if (moves[m].kind == RB_MOVE_DE) {
+      key.move.gamma0 = moves[m].gamma0;
+      key.move.sigma = moves[m].sigma;
+    } else {
+      key.move.a = moves[m].a;
+    }
+    const unsigned char *kb = reinterpret_cast<const unsigned char *>(&key);
+    ready[m] = ctx->samp_graph[m] && ctx->samp_key[m].size() == sizeof(key) &&
+               memcmp(ctx->samp_key[m].data(), kb, sizeof(key)) == 0;
+    // pack, propose2, lnprob, accept2 per half-step + the step counter (speculative: 9 as well); DE: propose, lnprob,
+    // accept per non-empty group + the step counter
+    per_step[m] = 9;
+    if (moves[m].kind == RB_MOVE_DE) {
+      per_step[m] = 1;
+      for (int g = 0; g < 3; ++g) per_step[m] += st2::group_size(sp.B, 3, g) ? 3 : 0;
+    }
+  }
+  for (int64_t k = 0; k < nsteps; ++k) {
+    const int m = sched[k];
+    if (!ready[m]) {
+      if (!ran[m]) {   // un-captured first step of the move: every lazy allocation happens here
+        if (ctx->samp_graph[m]) {
+          cudaGraphExecDestroy(ctx->samp_graph[m]);
+          ctx->samp_graph[m] = nullptr;
+        }
+        ran[m] = 1;
+        rc = step_once(m);
+        if (rc != RB_OK) return rc;
+        rc = store(k);
+        if (rc != RB_OK) return rc;
+        continue;
+      }
+      cudaGraph_t g = nullptr;
+      const long long launches_before = ctx->launches;
+      CUDA_TRY(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+      rc = step_once(m);
+      cudaError_t ce = cudaStreamEndCapture(s, &g);
+      ctx->launches = launches_before;   // nothing ran
+      if (rc != RB_OK || ce != cudaSuccess || !g) {
+        if (g) cudaGraphDestroy(g);
+        if (rc == RB_OK) rb_set_error(std::string(who) + ": graph capture failed: " + cudaGetErrorString(ce));
+        return rc != RB_OK ? rc : RB_ERR_CUDA;
+      }
+      ce = cudaGraphInstantiate(&ctx->samp_graph[m], g, 0);
+      cudaGraphDestroy(g);
+      if (ce != cudaSuccess) {
+        ctx->samp_graph[m] = nullptr;
+        rb_set_error(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
+        return RB_ERR_CUDA;
+      }
+      const unsigned char *kb = reinterpret_cast<const unsigned char *>(&keys[m]);
+      ctx->samp_key[m].assign(kb, kb + sizeof(Key));
+      ready[m] = 1;
+    }
+    CUDA_TRY(cudaGraphLaunch(ctx->samp_graph[m], s));
+    ctx->launches += per_step[m];
     rc = store(k);
     if (rc != RB_OK) return rc;
   }

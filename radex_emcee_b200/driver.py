@@ -48,6 +48,7 @@ from . import _lib
 from . import emcee_radex as _er1
 from . import emcee_radex_2comp as _er2
 from .data import get_source, read_data
+from .moves import parse_moves
 
 logger = logging.getLogger("radex_emcee_b200.driver")
 
@@ -242,12 +243,13 @@ def prefit(ncomp, R, Jup, flux, eflux, bounds, p0, T_d=None, opts=None):
 
 def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
                device=0, datapath=None, opts=None, outdir=None, store_chain=True, allow_synthetic=False,
-               chain_to_host=True, predict_jup=None, corner_bins=None):
+               chain_to_host=True, predict_jup=None, corner_bins=None, moves=None):
     """One pass of the reference's per-source loop.  Returns a dict with every item of the pickle plus
     the percentile summaries, the sampler's acceptance fraction and the integrated autocorrelation time.
     ``chain_to_host=False``: the chain stays on the device (``chain`` and ``lnprobability`` are None).
     ``predict_jup``: line indices J whose posterior-predictive fluxes the result gains (``sled_jup``, ``sled_summary``).
-    ``corner_bins``: bins of the ``corner`` item the result gains (marginals, covariance, nearest sample)."""
+    ``corner_bins``: bins of the ``corner`` item the result gains (marginals, covariance, nearest sample).
+    ``moves``: the sampler's moves as ``StretchSampler(moves=...)`` takes them (None: the stretch move)."""
     from .radex import Radex
     from .sampler import CudaEngine, SLEDModel, StretchSampler
 
@@ -278,7 +280,7 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
     rng = np.random.RandomState(seed)                       # the reference draws from numpy's global state
     pos = np.array([popt + 1e-3 * rng.randn(ndim) for _ in range(nwalkers)])
     eng = CudaEngine(R._ctx, SLEDModel(ncomp, Jup, flux, eflux, bounds, tbg, T_d=T_d, opts=opts))
-    sampler = StretchSampler(nwalkers, ndim, eng, seed=seed)
+    sampler = StretchSampler(nwalkers, ndim, eng, seed=seed, moves=moves)
     logger.info("burning samples")
     sampler.run_mcmc(pos, n_iter_burn, store=False)
     sampler.reset()
@@ -319,7 +321,7 @@ def fit_source(source, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_wal
 
 def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=100, n_iter_walk=None, seed=20170914,
                              device=0, datapath=None, opts=None, outdir=None, allow_synthetic=False, chain_to_host=True,
-                             predict_jup=None, corner_bins=None):
+                             predict_jup=None, corner_bins=None, moves=None):
     """BASELINE.json configs[3]: every source of the table in ONE ensemble.  The reference fits the sources one after the
     other (emcee_radex.py:389); here the pre-fits run per source (they are a few dozen batched launches each) and the
     walkers of all sources -- each with its own background temperature, bounds, line set and, with two components, dust
@@ -359,7 +361,7 @@ def fit_sources_concurrently(sources, data, ncomp=1, nwalkers=None, n_iter_burn=
         setups.append(dict(source=source, z=z, bounds=bounds, T_d=T_d, data=(Jup, flux, eflux), popt=popt, pcov=pcov,
                            pmin=pmin, prefit_info=info))
     eng = CudaEngine(R._ctx, models)
-    sampler = StretchSampler(nwalkers * len(sources), ndim, eng, seed=seed, nsources=len(sources))
+    sampler = StretchSampler(nwalkers * len(sources), ndim, eng, seed=seed, nsources=len(sources), moves=moves)
     logger.info("burning samples (%d sources x %d walkers in one ensemble)", len(sources), nwalkers)
     sampler.run_mcmc(np.vstack(starts), n_iter_burn, store=False)
     sampler.reset()
@@ -455,6 +457,9 @@ def main(argv=None):
     ap.add_argument("--predict-sled", type=int, nargs="+", default=None, metavar="J",
                     help="also summarise the posterior-predictive flux of these lines (1-based J, at most 16), per "
                          "component with two; computed on the GPU, so it works with --summaries-only")
+    ap.add_argument("--moves", nargs="+", default=None, metavar="MOVE[:WEIGHT]",
+                    help="sampler moves, e.g. de:0.8 stretch:0.2 (emcee's DEMove / StretchMove mixture; default: the "
+                         "stretch move)")
     ap.add_argument("--corner-bins", type=int, default=None, metavar="B",
                     help="also compute the corner-plot counts (B-bin marginals of the summary columns and their pairs), "
                          "the covariance and the sample nearest the median, on the GPU (works with --summaries-only); "
@@ -468,6 +473,7 @@ def main(argv=None):
     outdir = args.out or ("./single" if args.ncomp == 1 else "./double")
     data = read_data(datafile)
     sources = [s for s in data if args.sources is None or s in args.sources]
+    moves = None if args.moves is None else parse_moves(args.moves)
     if args.concurrent:
         if world > 1:
             import torch
@@ -478,7 +484,7 @@ def main(argv=None):
                                             n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir,
                                             datapath=args.datapath, allow_synthetic=args.allow_synthetic,
                                             chain_to_host=not args.summaries_only, predict_jup=args.predict_sled,
-                                            corner_bins=args.corner_bins):
+                                            corner_bins=args.corner_bins, moves=moves):
             if rank == 0:
                 print_summary(res, args.ncomp)
         if world > 1:
@@ -489,7 +495,7 @@ def main(argv=None):
         res = fit_source(source, data, ncomp=args.ncomp, nwalkers=args.walkers, n_iter_burn=args.burn,
                          n_iter_walk=args.steps, seed=args.seed, device=device, outdir=outdir, datapath=args.datapath,
                          allow_synthetic=args.allow_synthetic, chain_to_host=not args.summaries_only,
-                         predict_jup=args.predict_sled, corner_bins=args.corner_bins)
+                         predict_jup=args.predict_sled, corner_bins=args.corner_bins, moves=moves)
         print_summary(res, args.ncomp)
 
 

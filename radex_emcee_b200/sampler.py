@@ -1,4 +1,4 @@
-"""Device-resident affine-invariant ensemble sampler (stretch move).
+"""Device-resident affine-invariant ensemble sampler (stretch move, differential-evolution move, mixtures of them).
 
 Replaces ``emcee.EnsembleSampler`` + its default ``StretchMove(a=2)`` for the drivers' call
 sites (emcee/emcee_radex.py:483-499, emcee/emcee_radex_2comp.py:557-574; SURVEY.md 3.5): walkers,
@@ -25,6 +25,14 @@ Sharding
   independent of G.  On one GPU the whole loop runs inside the library (``rb_stretch_run_dev``; small
   ensembles replay a CUDA graph of one step) -- same kernels, same chain.
 
+Moves
+  ``moves=`` takes emcee's forms: one move, a list, or a list of (move, weight) of ``StretchMove`` and ``DEMove``
+  (moves.py).  Every step applies one move, drawn from the normalised weights by ``rb_move_schedule`` (keyed by
+  (seed, step): the same on every rank).  A DE step moves three groups in turn (the split generalised to three groups
+  per block); each group's partners are read from the whole ensemble, so with several ranks every DE sub-step is one
+  ``all_gather_into_tensor`` of X.  On one GPU the whole loop runs in the library (``rb_moves_run_dev``).
+  ``moves=None`` is ``[StretchMove(a)]`` on the code path of the stretch move alone.
+
 Posterior statistics where the chain lives
   ``get_quantiles`` (exact ``np.percentile`` of every source's flattened chain) and ``get_autocorr_time``
   (emcee's integrated autocorrelation time) read the stored chain in place on every rank (csrc/chain_stats.cuh):
@@ -48,6 +56,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .moves import DEMove, StretchMove, normalize_moves  # noqa: F401  (StretchMove: re-exported)
 
 logger = logging.getLogger("radex_emcee_b200.sampler")
 
@@ -353,6 +362,47 @@ class CudaEngine:
                                              lnp_chain.data_ptr() if lnp_chain is not None else None))
         self.launches += self.ctx.counters()[1] - l0
 
+    # ---- moves (moves.py): differential evolution, the k-group accept, a move list in the library -------------------
+    def de_propose(self, split, step, group, gid_base, X, Xall, gamma0, sigma):
+        """Proposals Q [nslots, ndim] of the local slots of DE group ``group`` and their source rows."""
+        self._bind_stream()
+        nlocal, ndim = X.shape
+        ns = nlocal // split.block * group_size(split.block, 3, group)
+        Q = torch.empty((ns, ndim), dtype=torch.float64, device=self.device)
+        src_id = torch.empty(ns, dtype=torch.int32, device=self.device)
+        sp = split.c_struct()
+        _lib.check(self.L.rb_de_propose_dev(self.ctx.handle, C.byref(sp), step, group, gid_base, nlocal, ndim, X.data_ptr(),
+                                            Xall.data_ptr(), gamma0, sigma, Q.data_ptr(), src_id.data_ptr()))
+        self.launches += 1
+        return Q, src_id
+
+    def group_accept(self, split, kind, step, group, ngroups, gid_base, X, lnp, Q, lnp_new, logfac, naccept, counters):
+        self._bind_stream()
+        nlocal, ndim = X.shape
+        sp = split.c_struct()
+        _lib.check(self.L.rb_group_accept_dev(self.ctx.handle, C.byref(sp), kind, step, group, ngroups, gid_base, nlocal,
+                                              ndim, X.data_ptr(), lnp.data_ptr(), Q.data_ptr(), lnp_new.data_ptr(),
+                                              logfac.data_ptr() if logfac is not None else None, naccept.data_ptr(),
+                                              counters.data_ptr()))
+        self.launches += 1
+
+    def run_moves(self, split, moves, step0, nsteps, X, lnp, naccept, counters, thin, chain, lnp_chain):
+        """nsteps steps of the move list [(move, weight)] of the whole (single-rank) ensemble inside the library."""
+        self._bind_stream()
+        sp = split.c_struct()
+        arr = (_lib.rb_move * len(moves))(*[m.c_struct(w) for m, w in moves])
+        _, l0 = self.ctx.counters()
+        _lib.check(self.L.rb_moves_run_dev(self.ctx.handle, self.srcset.handle, C.byref(sp), arr, len(moves), step0, nsteps,
+                                           C.byref(self.opts), X.data_ptr(), lnp.data_ptr(), naccept.data_ptr(),
+                                           counters.data_ptr(), thin, chain.data_ptr() if chain is not None else None,
+                                           lnp_chain.data_ptr() if lnp_chain is not None else None))
+        self.launches += self.ctx.counters()[1] - l0
+
+
+def group_size(block, ngroups, g):
+    """Slots of group g in a split block of the k-group split (st2::group_size)."""
+    return block // ngroups + (1 if g < block % ngroups else 0)
+
 
 def walkers_independent(coords):
     """emcee's check of an initial ensemble (ensemble.py, ``walkers_independent``): finite, no degenerate
@@ -377,7 +427,7 @@ class StretchSampler:
     ``get_covariance`` / ``get_nearest_sample``."""
 
     def __init__(self, nwalkers, ndim, engine, a=2.0, seed=0, group=None, randomize_split=True, nsources=1,
-                 split_block=None, native=True, time_gather=False):
+                 split_block=None, native=True, time_gather=False, moves=None):
         self.dist = torch.distributed if (torch.distributed.is_available() and torch.distributed.is_initialized()) else None
         self.group = group
         self.world = self.dist.get_world_size(group) if self.dist else 1
@@ -397,11 +447,32 @@ class StretchSampler:
         self.nlocal = self.nwalkers // self.world          # walkers owned by this rank: global ids gid_base ...
         self.gid_base = self.rank * self.nlocal
         W = self.nwalkers // nsources
-        block = int(split_block) if split_block else default_split_block(W, randomize_split)
+        # moves=None: the stretch move alone, on its own code path; otherwise a list of (move, weight)
+        self.moves = None if moves is None else normalize_moves(moves)
+        has_de = self.moves is not None and any(isinstance(m, DEMove) for m, _ in self.moves)
+        if split_block:
+            block = int(split_block)
+        elif has_de and not randomize_split:
+            # groups g + 3t of a block that is a multiple of 3: walker id mod 3, as emcee labels them, whatever the block;
+            # 6 when it divides the sub-ensemble and every rank's share (then the chain does not depend on the rank count),
+            # else one block per sub-ensemble, which needs whole sub-ensembles per rank
+            if W % 6 == 0 and self.nlocal % 6 == 0:
+                block = 6
+            elif self.nlocal % W == 0:
+                block = W
+            else:
+                raise ValueError("DEMove with randomize_split=False: no split block fits %d walkers per source and %d "
+                                 "walkers per rank (6 divides neither, or not both, and a rank holds part of a "
+                                 "source); pass split_block" % (W, self.nlocal))
+        else:
+            block = default_split_block(W, randomize_split)
         self.split = SplitSpec(self.nwalkers, W, block, randomize_split, self.seed)
         if self.nlocal % block:
             raise ValueError("every rank must own whole split blocks: nwalkers/world_size = %d is not a multiple of "
                              "split_block = %d (pass split_block, or randomize_split=False)" % (self.nlocal, block))
+        if has_de and (block < 3 or any(W - W // block * group_size(block, 3, g) < 2 for g in range(3))):
+            raise ValueError("DEMove: the 3-group split needs split_block >= 3 and leaves every group at least 2 walkers "
+                             "of its source to draw partners from (split_block = %d)" % block)
         self.native = bool(native) and self.world == 1 and hasattr(engine, "run_native")
         self.time_gather = bool(time_gather)
         self._gather_events = []
@@ -460,13 +531,30 @@ class StretchSampler:
             raise ValueError("Probability function returned NaN")
 
     # ---- the move -------------------------------------------------------------------------------
-    def _half_step(self, half):
+    def _half_step(self, half, a=None):
         eng, sp = self.engine, self.split
         Call = self._gather(eng.pack(sp, self.step, 1 - half, self.gid_base, self.X))
-        Q, logfac, src_id = eng.propose2(sp, self.step, half, self.gid_base, self.X, Call, self.a)
+        Q, logfac, src_id = eng.propose2(sp, self.step, half, self.gid_base, self.X, Call, self.a if a is None else a)
         lnp_new = eng.lnprob(Q, src_id if self.nsources > 1 else None)
         eng.accept2(sp, self.step, half, self.gid_base, self.X, self.lnp, Q, lnp_new, logfac, self.naccept,
                     self.counters)
+
+    def _de_substep(self, g, mv):
+        """Group g of a DE step: all-gather of X (the partners come from the whole ensemble), propose, lnprob, accept."""
+        eng, sp = self.engine, self.split
+        Xall = self._gather(self.X)
+        Q, src_id = eng.de_propose(sp, self.step, g, self.gid_base, self.X, Xall, mv.gamma0_for(self.ndim), mv.sigma)
+        lnp_new = eng.lnprob(Q, src_id if self.nsources > 1 else None)
+        eng.group_accept(sp, _lib.RB_MOVE_DE, self.step, g, 3, self.gid_base, self.X, self.lnp, Q, lnp_new, None,
+                         self.naccept, self.counters)
+
+    def _move_step(self, mv):
+        if isinstance(mv, DEMove):
+            for g in range(3):
+                self._de_substep(g, mv)
+        else:
+            self._half_step(0, mv.a)
+            self._half_step(1, mv.a)
 
     def run_mcmc(self, p0, nsteps, store=True, thin=1):
         if p0 is not None:
@@ -484,8 +572,12 @@ class StretchSampler:
             else:
                 chain = lchain = None
             if not store or aligned:
-                self.engine.run_native(self.split, self.a, self.step, nsteps, self.X, self.lnp, self.naccept,
-                                       self.counters, thin, chain, lchain)
+                if self.moves is None:
+                    self.engine.run_native(self.split, self.a, self.step, nsteps, self.X, self.lnp, self.naccept,
+                                           self.counters, thin, chain, lchain)
+                else:
+                    self.engine.run_moves(self.split, self.moves, self.step, nsteps, self.X, self.lnp, self.naccept,
+                                          self.counters, thin, chain, lchain)
                 self.step += nsteps
                 self.nsteps_done += nsteps
                 if chain is not None:
@@ -498,10 +590,15 @@ class StretchSampler:
         chain = torch.empty((nstore, self.nlocal, self.ndim), dtype=torch.float64, device=self.device)
         lchain = torch.empty((nstore, self.nlocal), dtype=torch.float64, device=self.device)
         k = 0
+        sched = (None if self.moves is None else
+                 _lib.move_schedule(self.seed, self.step, nsteps, [w for _, w in self.moves]))
         try:
-            for _ in range(nsteps):
-                self._half_step(0)
-                self._half_step(1)
+            for n in range(nsteps):
+                if sched is None:
+                    self._half_step(0)
+                    self._half_step(1)
+                else:
+                    self._move_step(self.moves[sched[n]][0])
                 self.step += 1
                 self.nsteps_done += 1
                 if store and (self.nsteps_done % thin == 0):
